@@ -3,11 +3,13 @@
 
     python bench.py --gpus 1 --steps 20 --warmup 3                  # our arm (CUDA, through the public API)
     python bench.py --impl reference --gpus 1 --steps 3 --warmup 1  # reference arm: the CPU oracle port
+    python bench.py --steps 5 --dump-outputs /tmp/cirim_out         # also write the last step's outputs (.npy)
 
 A "step" = one pass of the hot path (CIRIM.forward: 5 cascades x 8 time steps, ConvGRU, SENSE) over one batch of
 `--batch` (default 16) synthetic 15-coil 320x320 slices per GPU, followed by the gather of the reconstructions.  One process
 per GPU (torchrun for N > 1), slices sharded across ranks, no data-path collective, weak scaling.
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  Inputs and weights are seeded, so two runs with the same arguments see the same data and
+their --dump-outputs files can be compared array for array (e.g. two builds of the library).
 """
 import argparse
 import json
@@ -28,6 +30,10 @@ HW8 = H * W * 8
 DC_BYTES_PER_SLICE = 2 * CHW8 + HW8 + 2 * HW8
 # algorithmic FLOPs of the conv stack per time step per slice (2*MACs), SURVEY 8(d): 19.163 GFLOP
 CONV_FLOPS_PER_STEP = 2 * H * W * (4 * 64 * 25 + 2 * (64 * 192 * 2) + 64 * 64 * 9 + 64 * 2 * 9)
+# --dump-outputs: complex values kept per intermediate estimate, and at most this many of the final reconstruction (the
+# whole volume below that); 40 x 2^16 + 2^22 complex float32 values = 52 MiB at most
+DUMP_ESTIMATE_SAMPLES = 1 << 16
+DUMP_RECON_MAX = 1 << 22
 
 
 def load_peaks():
@@ -136,6 +142,34 @@ def cpu_reference_step(sd, cfg, b):
     return out[-1][-1]
 
 
+def _seeded_sample(n, k):
+    """The same k of n flat positions every run (all n when n <= k), in increasing order."""
+    import torch
+
+    return torch.randperm(n, generator=torch.Generator().manual_seed(0))[:k].sort().values
+
+
+def dump_outputs(path, cascades, volume=None):
+    """Write what CIRIM.forward returned in the last timed step as float32 .npy files, complex values as [..., 2] (real,
+    imaginary):
+      reconstruction.npy    the final estimate cascades[-1][-1] (with N > 1 GPUs the gathered volume), [slices, H, W, 2];
+                            above DUMP_RECON_MAX values, a fixed seeded sample of its flat positions, [DUMP_RECON_MAX, 2]
+      estimates_sample.npy  every cascade's estimate after every time step at one fixed seeded sample of flat positions,
+                            [num_cascades, time_steps, DUMP_ESTIMATE_SAMPLES, 2] (all of them would be 40 volumes); with
+                            N > 1 GPUs these are rank 0's slices only, so they cover other slices than a 1-GPU dump"""
+    import numpy as np
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    rec = torch.view_as_real(cascades[-1][-1] if volume is None else volume)
+    if rec.numel() // 2 > DUMP_RECON_MAX:
+        rec = rec.reshape(-1, 2)[_seeded_sample(rec.numel() // 2, DUMP_RECON_MAX).to(rec.device)]
+    np.save(os.path.join(path, "reconstruction.npy"), rec.float().cpu().numpy())
+    idx = _seeded_sample(cascades[0][0].numel(), DUMP_ESTIMATE_SAMPLES).to(rec.device)
+    est = torch.stack([torch.stack([torch.view_as_real(e.reshape(-1))[idx] for e in c]) for c in cascades])
+    np.save(os.path.join(path, "estimates_sample.npy"), est.float().cpu().numpy())
+
+
 def run_reference(args):
     import torch
     from mridc_b200 import synth
@@ -153,19 +187,15 @@ def run_reference(args):
     for _ in range(args.warmup):
         cpu_reference_step(sd, cfg, b)
     t0 = time.perf_counter()
-    done = 0
     for _ in range(args.steps):
         cpu_reference_step(sd, cfg, b)
-        done += 1
-        if time.perf_counter() - t0 > 240 and done < args.steps:
-            break  # bounded sample: keep the whole run within a few minutes
     dt = time.perf_counter() - t0
-    val = done / dt
+    val = args.steps / dt
     sample = "%d step(s) of 1 slice each (full CIRIM 5x8 GRU, 15x320x320), %d warm-up, torch-CPU %d threads" % (
-        done, args.warmup, cores)
+        args.steps, args.warmup, cores)
     line = {
         "impl": "reference", "metric": "cirim_320x320x15coil_slices_per_sec", "value": val, "unit": "slices/s",
-        "n_gpus": args.gpus, "steps": done, "warmup": args.warmup, "ms_per_step": 1e3 * dt / done,
+        "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt / args.steps,
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         # the repo arm's own config (the metric is per slice; a CPU step is a bounded sample of that workload: one slice)
         "config": workload_config(args.batch, args.gpus),
@@ -328,9 +358,12 @@ def run_ours(args):
     n_global = B * world
 
     pending = []
+    kept = {}
 
-    def step_resident():
+    def step_resident(keep=False):
         out = next(model(d["y"], d["sensitivity_maps"], d["mask"], None, d["target"]))
+        if keep:
+            kept["out"] = out  # every estimate of this step, for --dump-outputs
         rec = out[-1][-1]
         if world == 1:
             return rec
@@ -390,9 +423,9 @@ def run_ours(args):
     _lib.reset_launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(args.steps):
-        step_resident()
-    drain()
+    for i in range(args.steps):
+        step_resident(keep=args.dump_outputs is not None and rank == 0 and i == args.steps - 1)
+    gathered = drain()
     e1.record()
     barrier_sync()
     launches = _lib.launch_count()
@@ -401,6 +434,8 @@ def run_ours(args):
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_total = ms.item()
     clocks = sampler.stop() if sampler else None
+    if kept:
+        dump_outputs(args.dump_outputs, kept.pop("out"), gathered)
 
     # ---- end-to-end timing: host buffers, H2D + compute + D2H of the reconstruction every step ------
     out_host = torch.empty((B, H, W), dtype=torch.complex64).pin_memory()
@@ -574,7 +609,13 @@ def main():
     ap.add_argument("--batch", type=int, default=16, help="slices per GPU per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary measurements (latency, E2EVN, brain)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm (--impl ours)")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -184,28 +184,35 @@ def test_host_logic_cascadenet_and_recurrentvarnet(golden, cpu_ops):
     assert rel_l2(k1n, g["rvn_k1n"]) < 1e-6 and rel_l2(h1n, g["rvn_h1n"]) < 1e-6
 
 
-def test_initialisers_follow_the_reference_rng_order():
-    """Same seed => the reference's random-init weights (module construction order and initialisers): checked against
-    the live reference when it is present."""
-    from oracle import ref_import
-
-    if not ref_import.available():
-        pytest.skip("reference tree not present")
+def test_initialisers_follow_the_reference_rng_order(golden):
+    """Same seed => the reference's random-init weights (module construction order and initialisers), against the weights
+    the reference modules drew for tests/golden (stored with '.' in the keys replaced by '_'): RecurrentInit followed by a
+    RecurrentVarNetBlock from one seed, the NormUnet of a qVarNetBlock and the JRSCIRIM blocks."""
     import mridc_b200 as mb
+    from oracle.make_golden import JRS_CASES, JRS_RIM
 
-    R = ref_import.Ref()
-    torch.manual_seed(11)
-    a = R.recurrentvarnet.RecurrentVarNetBlock(2, 8, 3, True, "ortho", SD, 1).state_dict()
-    torch.manual_seed(11)
-    b = mb.RecurrentVarNetBlock(2, 8, 3, True, "ortho", SD, 1).state_dict()
-    assert list(a) == list(b)
-    for k in a:
-        assert torch.equal(a[k], b[k]), k
-    torch.manual_seed(12)
-    a = R.recurrentvarnet.RecurrentInit(2, 8, (8, 8, 16), (1, 2, 4), depth=3, multiscale_depth=2).state_dict()
-    torch.manual_seed(12)
-    b = mb.RecurrentInit(2, 8, (8, 8, 16), (1, 2, 4), depth=3, multiscale_depth=2).state_dict()
-    assert list(a) == list(b) and all(torch.equal(a[k], b[k]) for k in a)
+    def check(g, prefix, module, skip=()):
+        keys = [k[len(prefix):] for k in g if k.startswith(prefix)]
+        sd = module.state_dict()
+        assert keys == [k.replace(".", "_") for k in sd], prefix
+        for k, v in sd.items():
+            if k not in skip:
+                assert torch.equal(T(g[prefix + k.replace(".", "_")]), v), prefix + k
+
+    g = golden("consumers")
+    torch.manual_seed(6)
+    init = mb.RecurrentInit(2, 8, (8, 8), (1, 2), depth=2, multiscale_depth=2)
+    blk = mb.RecurrentVarNetBlock(2, 8, 2, True, "ortho", SD, 1)
+    check(g, "rvn_init_", init)
+    check(g, "rvn_blk_", blk, skip=("learning_rate",))  # set to 0.9 after construction
+    torch.manual_seed(7)
+    unet = mb.NormUnet(chans=4, num_pools=2, in_chans=8, out_chans=8, padding_size=3)
+    check(g, "qvn_w_", mb.qVarNetBlock(unet, True, "ortho", SD, 2, False), skip=("dc_weight",))
+    g = golden("jrscirim")
+    for idx, (name, sp, in_ch, mag, slices) in enumerate(JRS_CASES):
+        torch.manual_seed(40 + idx)
+        check(g, "jrs%d_w_" % idx, mb.JRSCIRIMBlock(dict(JRS_RIM), dict(sp), in_ch, mag, True, "ortho", SD, 2, 2, slices,
+                                                   "SENSE", True))
 
 
 def test_oracle_jrscirim_golden(golden):

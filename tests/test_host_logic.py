@@ -4,11 +4,21 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import ref_import
-
 RIM_HP = dict(conv_filters=[16, 16, 2], conv_kernels=[5, 3, 3], conv_dilations=[1, 2, 1],
               conv_bias=[True, True, False], recurrent_filters=[16, 16, 0], recurrent_kernels=[1, 1, 0],
               recurrent_dilations=[1, 1, 0], recurrent_bias=[True, True, False])
+LAYERS = ["GRU", "IndRNN", "MGU"]  # layer codes of the golden configs
+
+
+def assert_reference_init(g, prefix, sd, skip=()):
+    """`sd`, the state_dict of a module built right after torch.manual_seed(s), against the weights the reference module
+    got from the same seed (stored under `prefix` by oracle/make_golden.py): same keys in the same order, same values bit
+    for bit.  `skip` names parameters the generator overwrote after construction."""
+    keys = [k[len(prefix):] for k in g if k.startswith(prefix)]
+    assert keys == list(sd), prefix
+    for k in keys:
+        if k not in skip:
+            assert torch.equal(torch.from_numpy(g[prefix + k]), sd[k]), prefix + k
 
 
 def test_masks_bit_exact_vs_reference_golden(golden):
@@ -70,26 +80,35 @@ def test_state_dict_keys_match_reference_layout(golden):
     assert sum(p.numel() for p in vn.parameters()) == 89267
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
-def test_initialisers_reproduce_reference_weights():
-    """Same seed -> same random-init weights as the reference modules (same init calls in the same order)."""
+def test_initialisers_reproduce_reference_weights(golden):
+    """Same seed -> same random-init weights as the reference modules (same init calls in the same order): every RIMBlock
+    (GRU / IndRNN / MGU, 2-D and 3-D), NormUnet and VarNetBlock whose reference weights are stored in tests/golden."""
     import mridc_b200 as mb
+    from oracle.make_golden import RIM_HP as GOLDEN_RIM_HP
 
-    R = ref_import.Ref()
-    for layer in ("GRU", "MGU", "IndRNN"):
-        kw = dict(recurrent_layer=layer, depth=2, time_steps=8, conv_dim=2, no_dc=True, **RIM_HP)
-        torch.manual_seed(1)
-        a = R.rim_block.RIMBlock(**kw).state_dict()
-        torch.manual_seed(1)
-        b = mb.RIMBlock(**kw).state_dict()
-        assert sorted(a) == sorted(b)
-        for k in a:
-            assert torch.equal(a[k], b[k]), (layer, k)
-    torch.manual_seed(2)
-    a = R.unet_block.NormUnet(chans=6, num_pools=3, padding_size=11).state_dict()
-    torch.manual_seed(2)
-    b = mb.NormUnet(chans=6, num_pools=3, padding_size=11).state_dict()
-    assert sorted(a) == sorted(b) and all(torch.equal(a[k], b[k]) for k in a)
+    g = golden("rim")
+    for i in range(int(g["nrim"])):
+        layer, rk, no_dc = (int(v) for v in g["rim%d_cfg" % i][:3])
+        torch.manual_seed(1 + i)
+        blk = mb.RIMBlock(**dict(GOLDEN_RIM_HP, recurrent_layer=LAYERS[layer], recurrent_kernels=[rk, rk, 0],
+                                 no_dc=bool(no_dc)))
+        assert_reference_init(g, "rim%d_w_" % i, blk.state_dict())
+    g = golden("rim3d")
+    for i in range(int(g["nrim"])):
+        layer, steps = int(g["rim%d_cfg" % i][0]), int(g["rim%d_cfg" % i][3])
+        torch.manual_seed(40 + i)
+        blk = mb.RIMBlock(**dict(GOLDEN_RIM_HP, recurrent_layer=LAYERS[layer], no_dc=True, time_steps=steps, conv_dim=3,
+                                 dimensionality=3))
+        assert_reference_init(g, "rim%d_w_" % i, blk.state_dict())
+    g = golden("unet_vn")
+    for i in range(int(g["nunet"])):
+        chans, pools, padsz = (int(v) for v in g["unet%d_cfg" % i])
+        torch.manual_seed(5 + i)
+        assert_reference_init(g, "unet%d_w_" % i, mb.NormUnet(chans=chans, num_pools=pools, padding_size=padsz).state_dict())
+    for j in range(int(g["nvn"])):
+        torch.manual_seed(40 + j)
+        vb = mb.VarNetBlock(mb.NormUnet(chans=4, num_pools=2, padding_size=11), no_dc=bool(g["vn%d_cfg" % j][2]))
+        assert_reference_init(g, "vn%d_w_" % j, vb.state_dict(), skip=("dc_weight",))  # set to 0.7 after construction
 
 
 def test_error_behaviour_matches_reference_texts():
@@ -180,55 +199,52 @@ def test_qcirim_ctor_errors():
         mb.RescaleByMax.reverse(torch.zeros(1, 4, 4, 4), torch.ones(4))
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
-def test_qrim_initialisers_reproduce_reference_weights():
+def test_qrim_initialisers_reproduce_reference_weights(golden):
+    """qRIMBlock (GRU / IndRNN / MGU) and the cascades of qCIRIM against the reference weights stored in tests/golden."""
     import mridc_b200 as mb
+    from oracle.make_golden import QRIM_HP, oqnets_cfg
 
-    R = ref_import.Ref()
-    kw = dict(conv_filters=[8, 8, 4], conv_kernels=[5, 3, 3], conv_dilations=[1, 2, 1], conv_bias=[True, True, False],
-              recurrent_filters=[8, 8, 0], recurrent_kernels=[1, 1, 0], recurrent_dilations=[1, 1, 0],
-              recurrent_bias=[True, True, False], depth=2, time_steps=8, conv_dim=2, no_dc=True, coil_dim=2)
-    for layer in ("GRU", "MGU", "IndRNN"):
-        torch.manual_seed(3)
-        a = R.qrim_block.qRIMBlock(recurrent_layer=layer, **kw).state_dict()
-        torch.manual_seed(3)
-        b = mb.qRIMBlock(recurrent_layer=layer, **kw).state_dict()
-        assert sorted(a) == sorted(b)
-        for k in a:
-            assert torch.equal(a[k], b[k]), (layer, k)
+    g = golden("qmri")
+    hp = {k: v for k, v in QRIM_HP.items() if k != "time_steps"}
+    for i in range(int(g["nblk"])):
+        torch.manual_seed(40 + i)
+        blk = mb.qRIMBlock(recurrent_layer=LAYERS[int(g["blk%d_cfg" % i][0])], depth=2, time_steps=QRIM_HP["time_steps"],
+                           conv_dim=2, no_dc=True, linear_forward_model=mb.SignalForwardModel(sequence="MEGRE"), **hp)
+        assert_reference_init(g, "blk%d_w_" % i, blk.state_dict())
+    torch.manual_seed(77)
+    assert_reference_init(g, "model_w_", mb.qCIRIM(oqnets_cfg(num_cascades=2)).state_dict())
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
-def test_sens_net_initialiser_and_bookkeeping_match_reference():
+def test_sens_net_initialiser_and_bookkeeping_match_reference(golden):
+    """BaseSensitivityModel against the reference's weights and low-frequency bookkeeping stored in tests/golden; a VarNet
+    with use_sens_net builds that network first (base.py:81-94), so it draws the same weights from the same seed."""
     import mridc_b200 as mb
-    from oracle.make_golden import _ref_sens_model
+    from mridc_b200 import synth
+    from oracle import nets as onets
 
-    Sens = _ref_sens_model(ref_import.Ref())
-    torch.manual_seed(9)
-    a = Sens(4, 3, mask_type="1D").state_dict()
-    torch.manual_seed(9)
-    b = mb.BaseSensitivityModel(4, 3, mask_type="1D").state_dict()
-    assert sorted(a) == sorted(b) and all(torch.equal(a[k], b[k]) for k in a)
-    g = torch.Generator().manual_seed(3)
+    g = golden("sens")
+    for i in range(int(g["nsens"])):
+        chans, pools, mtype, _, _, normalize, mcenter, nlf = (int(v) for v in g["sens%d_cfg" % i])
+        kw = dict(mask_type=["1D", "2D"][mtype], normalize=bool(normalize), mask_center=bool(mcenter))
+        torch.manual_seed(60 + i)
+        assert_reference_init(g, "sens%d_w_" % i, mb.BaseSensitivityModel(chans, pools, **kw).state_dict())
+        cfg = dict(synth.varnet_cfg(num_cascades=1), use_sens_net=True, sens_chans=chans, sens_pools=pools,
+                   sens_mask_type=kw["mask_type"], sens_normalize=kw["normalize"], sens_mask_center=kw["mask_center"])
+        torch.manual_seed(60 + i)
+        sd = mb.VarNet(cfg).state_dict()
+        assert_reference_init(g, "sens%d_w_" % i, {k[len("sens_net."):]: v for k, v in sd.items() if k.startswith("sens_net.")})
+        pad, n = mb.BaseSensitivityModel.get_pad_and_num_low_freqs(torch.from_numpy(g["sens%d_mask" % i]),
+                                                                   None if nlf < 0 else nlf)
+        assert np.array_equal(pad.numpy(), g["sens%d_pad" % i]) and np.array_equal(n.numpy(), g["sens%d_nlf" % i]), i
+    # more masks and low-frequency counts: the restatement, pinned to the same stored vectors by test_oracle_golden.py
+    gen = torch.Generator().manual_seed(3)
     for _ in range(5):
-        m = (torch.rand(3, 1, 1, 24, 1, generator=g) < 0.5).float()
+        m = (torch.rand(3, 1, 1, 24, 1, generator=gen) < 0.5).float()
         m[:, 0, 0, 10:14, 0] = 1
         for nlf in (None, 0, 4):
-            pa, na = Sens.get_pad_and_num_low_freqs(m, nlf)
+            pa, na = onets.sens_pad_and_num_low_freqs(m, nlf)
             pb, nb = mb.BaseSensitivityModel.get_pad_and_num_low_freqs(m, nlf)
             assert torch.equal(pa, pb) and torch.equal(na, nb)
-    # a model with use_sens_net builds the network first (base.py:81-94): same keys / RNG order as the reference
-    from mridc_b200 import synth
-
-    cfg = dict(synth.varnet_cfg(num_cascades=1), use_sens_net=True, sens_chans=4, sens_pools=2, sens_mask_type="2D",
-               sens_normalize=True, sens_mask_center=True)
-    torch.manual_seed(11)
-    ours = mb.VarNet(cfg).state_dict()
-    torch.manual_seed(11)
-    ref_first = Sens(4, 2, fft_centered=False, fft_normalization="backward", spatial_dims=[-2, -1], coil_dim=1,
-                     mask_type="2D", normalize=True, mask_center=True).state_dict()
-    for k, v in ref_first.items():
-        assert torch.equal(ours["sens_net." + k], v), k
 
 
 def _replay_apply_mask(golden, device):
