@@ -210,34 +210,17 @@ int mrb_normunet_out(const void* x, const void* mean_std, void* out, int B, int 
                      int normalize, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------
- * Tensor-core (tcgen05 / TMEM, error-compensated bf16 hi/lo split, fp32 accumulation) RIM regulariser,
- * channels-last fp32 activations.  Same arithmetic as mrb_conv2d / mrb_gru_cell_1x1 to ~3e-6 relative per operator
- * (products are evaluated as a_hi*b_hi + a_hi*b_lo + a_lo*b_hi with 16-17 significant bits per operand); used by
- * RIMBlock's time loop (rim_block.py:217-249) when the layer geometry matches (64 channels, cell kernel size 1).
+ * Tensor-core (tcgen05 / TMEM, error-compensated bf16 hi/lo split, fp32 accumulation) RIM regulariser, used by RIMBlock's
+ * time loop (rim_block.py:217-249) when the layer geometry matches (64 channels, cell kernel size 1).  Same arithmetic as
+ * mrb_conv2d / mrb_gru_cell_1x1 to ~3e-6 relative per operator (products are evaluated as a_hi*b_hi + a_hi*b_lo +
+ * a_lo*b_hi with 16-17 significant bits per operand).
  * Weights are packed once per parameter version into the UMMA shared-memory layout (bf16 hi/lo split).
- * (The profiling hooks of this kernel live in the tools-only build, tools/libmridc_b200_tools.so.)
+ * (The profiling hooks of these kernels live in the tools-only build, tools/libmridc_b200_tools.so.)
  * ------------------------------------------------------------------------------------------------- */
-/* size of the packed weights in 4-byte units: kind 0 = conv k x k (cin 64), 1 = GRU 1x1 (64 -> 64), 2 = conv 5x5 over 4 channels */
+/* size of the packed weights in 4-byte units: kind 0 = conv k x k (cin 64); any other kind: 0 */
 size_t mrb_tc_packed_floats(int kind, int cout, int cin, int k);
 /* w [cout, 64, k, k] (conv_layers.py:78-85) */
 int mrb_tc_pack_conv(const void* w, void* dst, int cout, int cin, int k, void* stream);
-/* w_ih, w_hh [3*ch, 64] (rnn_cells.py:23-38) */
-int mrb_tc_pack_gru(const void* w_ih, const void* w_hh, void* dst, int ch, int cx, void* stream);
-/* w [cout, 4, 5, 5] */
-int mrb_tc_pack_conv5x5x4(const void* w, void* dst, int cout, void* stream);
-/* ConvNonlinear k x k, dilation dil, replicate padding, 64 -> cout, NHWC in/out, bias, optional ReLU */
-int mrb_tc_conv_nhwc(const void* x, const void* wpack, const void* bias, void* out, int B, int H, int W, int cout,
-                     int k, int dil, int relu, void* stream);
-/* ConvNonlinear 5x5 over the 4-channel RIM gradient [B,H,W,4] -> [B,H,W,cout] */
-int mrb_tc_conv5x5x4_nhwc(const void* x, const void* wpack, const void* bias, void* out, int B, int H, int W,
-                          int cout, int relu, void* stream);
-/* ConvGRUCell (kernel size 1): x, h, h_out [B,H,W,64]; b_ih [192] or null */
-int mrb_tc_gru_nhwc(const void* x, const void* h, const void* wpack, const void* b_ih, void* h_out, int B, int H,
-                    int W, int ch, void* stream);
-/* IndRNNCell (kernel size 1, rnn_cells.py:264-391): x, h, h_out [B,H,W,ch]; wpack = mrb_tc_pack_conv of ih.weight
- * [ch, 64, 1, 1]; b_ih [ch] or null; hh [ch] (the per-channel recurrent weight): h_out = ReLU(ih(x) + hh * h) */
-int mrb_tc_indrnn_nhwc(const void* x, const void* h, const void* wpack, const void* b_ih, const void* hh, void* h_out,
-                       int B, int H, int W, int ch, void* stream);
 /* ---------------------------------------------------------------------------------------------------
  * Second-generation tensor-core engine: split-bf16 ("BH") activations, TMA + shared-memory operands.
  * BH layout: [B][H+4][W+4][hi 64 bf16 | lo 64 bf16] (x ~= hi + lo; 256 B per pixel; replicate border of 2 pixels, which
@@ -251,11 +234,9 @@ int mrb_bh_to_nhwc(const void* bh, void* x, int B, int H, int W, void* stream);
 /* packed ConvGRUCell weights for mrb_tc2_gru: w_ih, w_hh [192, 64] (rnn_cells.py:23-38) */
 size_t mrb_tc2_gru_packed_bytes(void);
 int mrb_tc2_pack_gru(const void* w_ih, const void* w_hh, void* dst, int ch, int cx, void* stream);
-/* ConvNonlinear on BH tensors (conv_layers.py:36-123): 5x5 over the fp32 4-channel RIM gradient [B,H,W,4] -> BH, and
- * k x k (dilation dil, dil*(k-1)/2 <= 2) BH -> BH; wpack as for mrb_tc_conv5x5x4_nhwc / mrb_tc_conv_nhwc; cout == 64.
- * x_bh needs a valid replicate border; the border of the outputs is not a replicate copy. */
-int mrb_tc_conv5x5x4_bh(const void* x, const void* wpack, const void* bias, void* out_bh, int B, int H, int W, int cout,
-                        int relu, void* stream);
+/* ConvNonlinear on BH tensors (conv_layers.py:36-123): k x k (dilation dil, dil*(k-1)/2 <= 2) BH -> BH, bias, optional
+ * ReLU; wpack from mrb_tc_pack_conv; cout == 64.  x_bh needs a valid replicate border; the border of the output is not a
+ * replicate copy. */
 int mrb_tc_conv_bh(const void* x_bh, const void* wpack, const void* bias, void* out_bh, int B, int H, int W, int cout, int k,
                    int dil, int relu, void* stream);
 /* First RIM conv fed by bulk copies.  "G8" input layout: the conv input [eta.re, eta.im, grad.re, grad.im] of a position as
@@ -303,10 +284,6 @@ int mrb_tc2_gru(const void* x_bh, const void* h_bh, const void* wpack, const voi
  * not alias x or h.  Pointwise over all positions like mrb_tc2_gru. */
 int mrb_tc2_indrnn(const void* x_bh, const void* h_bh, const void* wpack, const void* b_ih, const void* hh, void* out_bh, int B,
                    int H, int W, void* stream);
-/* Final RIM conv (rim_block.py:239-248): k x k (odd), dilation dil, replicate padding, cin -> 2 channels, no bias,
- * x [B,H,W,cin] channels-last, out [B,H,W,2] = eta + conv(x). */
-int mrb_conv_c2_nhwc_residual(const void* x, const void* w, const void* bias, const void* eta, void* out, int B,
-                              int H, int W, int cin, int k, int dil, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------
  * Quantitative MRI (qRIM / qCIRIM, BASELINE.json configs[4]): pointwise kernels around the fused DC operator.

@@ -54,16 +54,9 @@ SIGNATURES = {
     "mrb_normunet_out": (_i, [_vp, _vp, _vp, _i, _i, _ll, _i, _vp]),
     "mrb_tc_packed_floats": (_sz, [_i, _i, _i, _i]),
     "mrb_tc_pack_conv": (_i, [_vp, _vp, _i, _i, _i, _vp]),
-    "mrb_tc_pack_gru": (_i, [_vp, _vp, _vp, _i, _i, _vp]),
-    "mrb_tc_pack_conv5x5x4": (_i, [_vp, _vp, _i, _vp]),
-    "mrb_tc_conv_nhwc": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp]),
-    "mrb_tc_conv5x5x4_nhwc": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
-    "mrb_tc_gru_nhwc": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
-    "mrb_tc_indrnn_nhwc": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     "mrb_bh_bytes": (_sz, [_i, _i, _i]),
     "mrb_bh_from_nhwc": (_i, [_vp, _vp, _i, _i, _i, _vp]),
     "mrb_bh_to_nhwc": (_i, [_vp, _vp, _i, _i, _i, _vp]),
-    "mrb_tc_conv5x5x4_bh": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "mrb_tc_conv_bh": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "mrb_conv_c2_bh_residual": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     "mrb_bh_fix_border": (_i, [_vp, _i, _i, _i, _vp]),
@@ -78,7 +71,6 @@ SIGNATURES = {
     "mrb_tc2_pack_gru": (_i, [_vp, _vp, _vp, _i, _i, _vp]),
     "mrb_tc2_gru": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     "mrb_tc2_indrnn": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
-    "mrb_conv_c2_nhwc_residual": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "mrb_metrics_workspace_bytes": (_sz, [_i]),
     "mrb_abs_max_normalize": (_i, [_vp, _ll, _i, _vp, _vp, _vp]),
     "mrb_recon_metrics": (_i, [_vp, _vp, _i, _i, _i, _i, _d, _vp, _vp, _vp]),

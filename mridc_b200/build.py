@@ -24,7 +24,7 @@ NVCC_FLAGS = [
     "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC",
     "--expt-relaxed-constexpr",
-] + os.environ.get("MRIDC_B200_NVCC_EXTRA", "").split()  # experiments: e.g. -DMRB_GRU2_GROUPS=1 (part of the build digest)
+] + os.environ.get("MRIDC_B200_NVCC_EXTRA", "").split()  # extra nvcc flags for experiments (part of the build digest)
 
 
 def _nvcc():

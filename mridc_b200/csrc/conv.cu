@@ -311,79 +311,8 @@ __global__ void mgu_gates_kernel(const float* __restrict__ ih, const float* __re
     }
 }
 
-// Final RIM conv on channels-last input: cin -> 2 channels, replicate padding, fused eta update.
-// CTA = 32 x 8 output pixels, 128 threads, each thread two pixels (y, y+4) x both outputs.  The input halo patch is
-// staged through shared memory in chunks of 16 channels (pixel stride padded to 20 floats: conflict-free LDS.128),
-// weights (k*k*cin float2) are broadcast from shared memory and shared by the thread's two pixels.
-constexpr int C2_TX = 32, C2_TY = 8, C2_CH = 16, C2_PSTR = 20;
-__global__ void __launch_bounds__(128) conv_c2_nhwc_kernel(const float* __restrict__ x, const float* __restrict__ w,
-                                                           const float* __restrict__ bias,
-                                                           const float* __restrict__ eta, float* __restrict__ out,
-                                                           int B, int H, int W, int cin, int k, int dil) {
-    extern __shared__ float4 c2smem[];
-    const int kk = k * k;
-    const int pad = dil * (k - 1) / 2;
-    const int PW = C2_TX + 2 * pad, PH = C2_TY + 2 * pad;
-    float2* w2 = reinterpret_cast<float2*>(c2smem);                        // [tap][ci] -> (w[0][ci][tap], w[1][ci][tap])
-    float* patch = reinterpret_cast<float*>(w2 + (size_t)kk * cin);        // [PH*PW][C2_PSTR]
-    for (int t = threadIdx.x; t < kk * cin; t += blockDim.x) {
-        int ci = t % cin, tap = t / cin;
-        w2[t] = make_float2(w[(long long)ci * kk + tap], w[((long long)cin + ci) * kk + tap]);
-    }
-    const int tiles_x = (W + C2_TX - 1) / C2_TX;
-    const int ty = blockIdx.x / tiles_x, tx = blockIdx.x - ty * tiles_x;
-    const int x0 = tx * C2_TX, y0 = ty * C2_TY;
-    const int b = blockIdx.y;
-    const int lx = threadIdx.x & 31, ly = threadIdx.x >> 5;  // pixels (lx, ly) and (lx, ly + 4)
-    float acc[2][2] = {{0.f, 0.f}, {0.f, 0.f}};
-    const float* xb = x + (long long)b * H * W * cin;
-    for (int c0 = 0; c0 < cin; c0 += C2_CH) {
-        __syncthreads();
-        // stage the patch chunk: one float4 per (pixel, quarter)
-        for (int t = threadIdx.x; t < PH * PW * 4; t += blockDim.x) {
-            const int q = t & 3, pp = t >> 2;
-            const int py = pp / PW, px = pp - py * PW;
-            const int gy = min(max(y0 - pad + py, 0), H - 1), gx = min(max(x0 - pad + px, 0), W - 1);
-            const float4 v = __ldg(reinterpret_cast<const float4*>(xb + ((long long)gy * W + gx) * cin + c0 + q * 4));
-            *reinterpret_cast<float4*>(patch + (size_t)pp * C2_PSTR + q * 4) = v;
-        }
-        __syncthreads();
-        for (int tap = 0; tap < kk; ++tap) {
-            const int dy = (tap / k) * dil, dx = (tap % k) * dil;
-            const float* p0 = patch + (size_t)((ly + dy) * PW + lx + dx) * C2_PSTR;
-            const float* p1 = p0 + (size_t)4 * PW * C2_PSTR;
-            const float4* wp = reinterpret_cast<const float4*>(w2 + (size_t)tap * cin + c0);
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const float4 a = *reinterpret_cast<const float4*>(p0 + q * 4);
-                const float4 c = *reinterpret_cast<const float4*>(p1 + q * 4);
-                const float4 wa = wp[2 * q], wb = wp[2 * q + 1];  // (w0[c],w1[c],w0[c+1],w1[c+1]), (c+2, c+3)
-                acc[0][0] = fmaf(a.x, wa.x, acc[0][0]); acc[0][1] = fmaf(a.x, wa.y, acc[0][1]);
-                acc[0][0] = fmaf(a.y, wa.z, acc[0][0]); acc[0][1] = fmaf(a.y, wa.w, acc[0][1]);
-                acc[0][0] = fmaf(a.z, wb.x, acc[0][0]); acc[0][1] = fmaf(a.z, wb.y, acc[0][1]);
-                acc[0][0] = fmaf(a.w, wb.z, acc[0][0]); acc[0][1] = fmaf(a.w, wb.w, acc[0][1]);
-                acc[1][0] = fmaf(c.x, wa.x, acc[1][0]); acc[1][1] = fmaf(c.x, wa.y, acc[1][1]);
-                acc[1][0] = fmaf(c.y, wa.z, acc[1][0]); acc[1][1] = fmaf(c.y, wa.w, acc[1][1]);
-                acc[1][0] = fmaf(c.z, wb.x, acc[1][0]); acc[1][1] = fmaf(c.z, wb.y, acc[1][1]);
-                acc[1][0] = fmaf(c.w, wb.z, acc[1][0]); acc[1][1] = fmaf(c.w, wb.w, acc[1][1]);
-            }
-        }
-    }
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-        const int oy = y0 + ly + 4 * i, ox = x0 + lx;
-        if (oy < H && ox < W) {
-            const long long p = ((long long)b * H + oy) * W + ox;
-            float o0 = acc[i][0], o1 = acc[i][1];
-            if (bias) { o0 += bias[0]; o1 += bias[1]; }
-            const float2 e = reinterpret_cast<const float2*>(eta)[p];
-            reinterpret_cast<float2*>(out)[p] = make_float2(e.x + o0, e.y + o1);
-        }
-    }
-}
-
-// Fast path of the same operator for the shipped geometry (k = 3, dilation 1): CTA = 32 x 16 output pixels, 128 threads,
-// each thread FOUR vertically adjacent pixels x both outputs.
+// Final RIM conv (k = 3, dilation 1) on a BH source: 64 -> 2 channels, replicate padding (the BH border), fused eta update.
+// CTA = 32 x 16 output pixels, 128 threads, each thread FOUR vertically adjacent pixels x both outputs.
 //   * the 18 x 34 halo patch travels in chunks of F_CH channels through a cp.async.cg double buffer (pixel stride padded
 //     by 4 floats: conflict-free LDS.128), so the global latency of chunk c+1 hides behind the arithmetic of chunk c;
 //   * the three kernel rows reuse the six patch rows a thread holds in registers (2x fewer shared-memory reads than
@@ -398,7 +327,7 @@ __device__ __forceinline__ void ffma2(float2& acc, float a0, float a1, float b0,
     asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(c) : "l"(a), "l"(b));
     asm("mov.b64 {%0, %1}, %2;" : "=f"(acc.x), "=f"(acc.y) : "l"(c));
 }
-template <int ROWS, int F_CH, bool BH>
+template <int ROWS, int F_CH>
 __global__ void __launch_bounds__(128) conv_c2_k3_kernel(const float* __restrict__ x, const float* __restrict__ w,
                                                          const float* __restrict__ bias, const float* __restrict__ eta,
                                                          float* __restrict__ out, int B, int H, int W, int cin) {
@@ -419,7 +348,7 @@ __global__ void __launch_bounds__(128) conv_c2_k3_kernel(const float* __restrict
     // BH source (conv_tc2.cu): [B][H+4][W+4][64 hi bf16 | 64 lo bf16] with a valid replicate border: taps are plain offsets;
     // a staged position holds [F_CH hi | F_CH lo] bf16 (F_CH/2 + F_CH/2 words) and the fp32 value is rebuilt as hi + lo
     const int Hp = H + 4, Wp = W + 4;
-    const float* xb = BH ? x + (long long)b * Hp * Wp * 64 : x + (long long)b * H * W * cin;
+    const float* xb = x + (long long)b * Hp * Wp * 64;
     const uint32_t patch_u32 = (uint32_t)__cvta_generic_to_shared(patch);
     // staging list of this thread: float4 t = tid + 128*i of the [F_PH*F_PW pixels][2 quads] chunk; the clamped source
     // offsets are the same for every chunk (computed once), the shared-memory offset is linear in i
@@ -430,19 +359,14 @@ __global__ void __launch_bounds__(128) conv_c2_k3_kernel(const float* __restrict
         const int t = threadIdx.x + 128 * i;
         const int q = t % NQ, pp = t / NQ;
         const int py = pp / F_PW, px = pp - py * F_PW;
-        if (BH) {
-            // quads 0 .. NQ/2-1: the chunk's hi bf16 (16 B each), NQ/2 .. NQ-1: its lo bf16 (128 B further)
-            const int gy = min(max(y0 + 1 + py, 0), Hp - 1), gx = min(max(x0 + 1 + px, 0), Wp - 1);
-            goff[i] = t < F_PH * F_PW * NQ ? (gy * Wp + gx) * 64 + (q < NQ / 2 ? q * 4 : 32 + (q - NQ / 2) * 4) : -1;
-        } else {
-            const int gy = min(max(y0 - 1 + py, 0), H - 1), gx = min(max(x0 - 1 + px, 0), W - 1);
-            goff[i] = t < F_PH * F_PW * NQ ? (gy * W + gx) * cin + q * 4 : -1;  // H*W*cin < 2^31 (checked on the host)
-        }
+        // quads 0 .. NQ/2-1: the chunk's hi bf16 (16 B each), NQ/2 .. NQ-1: its lo bf16 (128 B further)
+        const int gy = min(max(y0 + 1 + py, 0), Hp - 1), gx = min(max(x0 + 1 + px, 0), Wp - 1);
+        goff[i] = t < F_PH * F_PW * NQ ? (gy * Wp + gx) * 64 + (q < NQ / 2 ? q * 4 : 32 + (q - NQ / 2) * 4) : -1;
     }
     const uint32_t soff0 = (uint32_t)(((threadIdx.x / NQ) * F_PS + (threadIdx.x % NQ) * 4) * 4);
     auto stage = [&](int chunk, int buf) {
         const uint32_t dst = patch_u32 + (uint32_t)(buf * F_PH * F_PW * F_PS * 4) + soff0;
-        const float* g = xb + chunk * (BH ? F_CH / 2 : F_CH);  // BH: F_CH bf16 = F_CH/2 words per chunk and half
+        const float* g = xb + chunk * (F_CH / 2);  // F_CH bf16 = F_CH/2 words per chunk and half
 #pragma unroll
         for (int i = 0; i < kStage; ++i)
             if (goff[i] >= 0)
@@ -472,16 +396,12 @@ __global__ void __launch_bounds__(128) conv_c2_k3_kernel(const float* __restrict
 #pragma unroll
                 for (int r = 0; r < ROWS + 2; ++r) {
                     const float* pp = pb + (size_t)((ROWS * yg + r) * F_PW + lx + dx) * F_PS;
-                    if (BH) {
-                        const uint2 hw = *reinterpret_cast<const uint2*>(pp + q * 2);
-                        const uint2 lw = *reinterpret_cast<const uint2*>(pp + F_CH / 2 + q * 2);
-                        xr[r] = make_float4(__uint_as_float(hw.x << 16) + __uint_as_float(lw.x << 16),
-                                            __uint_as_float(hw.x & 0xffff0000u) + __uint_as_float(lw.x & 0xffff0000u),
-                                            __uint_as_float(hw.y << 16) + __uint_as_float(lw.y << 16),
-                                            __uint_as_float(hw.y & 0xffff0000u) + __uint_as_float(lw.y & 0xffff0000u));
-                    } else {
-                        xr[r] = *reinterpret_cast<const float4*>(pp + q * 4);
-                    }
+                    const uint2 hw = *reinterpret_cast<const uint2*>(pp + q * 2);
+                    const uint2 lw = *reinterpret_cast<const uint2*>(pp + F_CH / 2 + q * 2);
+                    xr[r] = make_float4(__uint_as_float(hw.x << 16) + __uint_as_float(lw.x << 16),
+                                        __uint_as_float(hw.x & 0xffff0000u) + __uint_as_float(lw.x & 0xffff0000u),
+                                        __uint_as_float(hw.y << 16) + __uint_as_float(lw.y << 16),
+                                        __uint_as_float(hw.y & 0xffff0000u) + __uint_as_float(lw.y & 0xffff0000u));
                 }
 #pragma unroll
                 for (int dy = 0; dy < 3; ++dy) {
@@ -513,22 +433,22 @@ __global__ void __launch_bounds__(128) conv_c2_k3_kernel(const float* __restrict
     }
 }
 
-template <int ROWS, int F_CH, bool BH>
+template <int ROWS, int F_CH>
 static int launch_c2_k3(const float* x, const float* w, const float* bias, const float* eta, float* out, int B, int H, int W,
                         int cin, cudaStream_t st) {
     constexpr int F_TY = 4 * ROWS, F_PH = F_TY + 2, F_PS = F_CH + 4;
     const size_t smem3 = (size_t)9 * (cin / 4) * 2 * sizeof(float4) + (size_t)2 * F_PH * F_PW * F_PS * sizeof(float);
     MRB_REQUIRE(smem3 <= 200 * 1024 && (long long)H * W * cin < 2147483647LL, MRB_EUNSUPPORTED,
-                "mrb_conv_c2_nhwc_residual: image or channel count too large");
-    MRB_REQUIRE(!BH || ((long long)(H + 4) * (W + 4) * 64 < 2147483647LL && cin == 64), MRB_EUNSUPPORTED,
+                "mrb_conv_c2_bh_residual: image or channel count too large");
+    MRB_REQUIRE((long long)(H + 4) * (W + 4) * 64 < 2147483647LL && cin == 64, MRB_EUNSUPPORTED,
                 "mrb_conv_c2_bh_residual: needs 64 channels and < 2^31 words per image");
     static bool attr_set = false;
     if (!attr_set) {
-        MRB_CUDA(cudaFuncSetAttribute(conv_c2_k3_kernel<ROWS, F_CH, BH>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        MRB_CUDA(cudaFuncSetAttribute(conv_c2_k3_kernel<ROWS, F_CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
         attr_set = true;
     }
     dim3 grid3((unsigned)(ceil_div(W, F_TX) * ceil_div(H, F_TY)), (unsigned)B);
-    conv_c2_k3_kernel<ROWS, F_CH, BH><<<grid3, 128, smem3, st>>>(x, w, bias, eta, out, B, H, W, cin);
+    conv_c2_k3_kernel<ROWS, F_CH><<<grid3, 128, smem3, st>>>(x, w, bias, eta, out, B, H, W, cin);
     MRB_LAUNCHED();
     return MRB_OK;
 }
@@ -537,35 +457,13 @@ static int launch_c2_k3(const float* x, const float* w, const float* bias, const
 
 using namespace mrb;
 
-extern "C" int mrb_conv_c2_nhwc_residual(const void* x, const void* w, const void* bias, const void* eta, void* out,
-                                         int B, int H, int W, int cin, int k, int dil, void* stream) {
-    MRB_REQUIRE(x && w && eta && out, MRB_EINVAL, "mrb_conv_c2_nhwc_residual: null pointer");
-    MRB_REQUIRE(B >= 1 && H >= 1 && W >= 1 && cin >= 16 && (cin % 16) == 0 && (k % 2) == 1 && dil >= 1 && B <= 65535,
-                MRB_EINVAL, "mrb_conv_c2_nhwc_residual: bad shape (cin must be a multiple of 16, k odd)");
-    if (k == 3 && dil == 1 && (cin % 32) == 0 && !getenv("MRB_C2_GENERIC")) {
-        // 4 rows per thread, 16-channel chunks (98 KB, two CTAs per SM): 48.5 us at B=4 vs 53.8 (8-channel chunks, three
-        // CTAs), 57-59 (2 rows per thread) and 87 for the generic kernel below
-        return launch_c2_k3<4, 16, false>((const float*)x, (const float*)w, (const float*)bias, (const float*)eta, (float*)out, B, H, W,
-                                   cin, (cudaStream_t)stream);
-    }
-    const int pad = dil * (k - 1) / 2;
-    size_t smem = (size_t)k * k * cin * sizeof(float2) +
-                  (size_t)(C2_TX + 2 * pad) * (C2_TY + 2 * pad) * C2_PSTR * sizeof(float);
-    MRB_REQUIRE(smem <= 96 * 1024, MRB_EUNSUPPORTED, "mrb_conv_c2_nhwc_residual: kernel / dilation too large");
-    MRB_CUDA(cudaFuncSetAttribute(conv_c2_nhwc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
-    dim3 grid((unsigned)(ceil_div(W, C2_TX) * ceil_div(H, C2_TY)), (unsigned)B);
-    conv_c2_nhwc_kernel<<<grid, 128, smem, (cudaStream_t)stream>>>(
-        (const float*)x, (const float*)w, (const float*)bias, (const float*)eta, (float*)out, B, H, W, cin, k, dil);
-    MRB_LAUNCHED();
-    return MRB_OK;
-}
-
-// The same final conv on a BH source (64 channels, k = 3, dilation 1; the border of x must be valid: mrb_bh_fix_border)
+// The final conv on a BH source (64 channels, k = 3, dilation 1; the border of x must be valid: mrb_bh_fix_border).
+// 4 rows per thread, 16-channel chunks (98 KB, two CTAs per SM).
 extern "C" int mrb_conv_c2_bh_residual(const void* x_bh, const void* w, const void* bias, const void* eta, void* out, int B,
                                        int H, int W, void* stream) {
     MRB_REQUIRE(x_bh && w && eta && out, MRB_EINVAL, "mrb_conv_c2_bh_residual: null pointer");
     MRB_REQUIRE(B >= 1 && H >= 1 && W >= 1 && B <= 65535, MRB_EINVAL, "mrb_conv_c2_bh_residual: bad shape");
-    return launch_c2_k3<4, 16, true>((const float*)x_bh, (const float*)w, (const float*)bias, (const float*)eta, (float*)out, B, H,
+    return launch_c2_k3<4, 16>((const float*)x_bh, (const float*)w, (const float*)bias, (const float*)eta, (float*)out, B, H,
                                      W, 64, (cudaStream_t)stream);
 }
 

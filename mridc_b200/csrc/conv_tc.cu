@@ -1,7 +1,9 @@
-// Tensor-core (tcgen05 / TMEM) implicit-GEMM kernels for the RIM regulariser, NHWC fp32 activations.
+// Tensor-core (tcgen05 / TMEM) implicit-GEMM k x k convolution of the RIM regulariser on BH activations.
 //
-// Reference behaviour: ConvNonlinear (rim/conv_layers.py:36-123, replicate padding) and ConvGRUCell with
-// kernel_size 1 (rim/rnn_cells.py:93-127), as used by RIMBlock's time loop (rim/rim_block.py:217-249).
+// Reference behaviour: ConvNonlinear (rim/conv_layers.py:36-123, replicate padding) with 64 input and 64 output channels,
+// as used for the second convolution of RIMBlock's time loop (rim/rim_block.py:217-249).  Input and output are BH tensors
+// (conv_tc2.cu: [B][H+4][W+4][64 hi bf16 | 64 lo bf16], replicate border of the input valid), so the replicate padding
+// is the tensor's own border and a tap is a plain offset into the flat positions.
 //
 // Numerics: the reference is fp32 and the end-to-end tolerance (rel-L2 1e-4) rules out plain TF32 / BF16 operands
 // (SURVEY section 7: 9.3e-4 / 9.9e-3).  Every product is therefore evaluated as an error-compensated split sum
@@ -13,23 +15,22 @@
 // at half the tensor-pipe rate and twice the instruction count (K = 8 instead of 16 per MMA) -- the kernels were
 // bound by exactly those two.
 //
-// Structure: one persistent CTA per SM.  Work item = (128-pixel tile, half of the output channels).
-//   * B operand = the weights of the CTA's channel half (hi and lo, pre-packed in the UMMA K-major SWIZZLE_128B
-//     layout): copied to shared memory once and resident for the whole kernel.
+// Structure: one persistent CTA per SM.  Work item = one 128-position tile, all 64 output channels.  Segment = one tap
+// (64 input channels = one K chunk of 64 bf16).
+//   * B operand = the weights of one tap (hi rows | lo rows, pre-packed in the UMMA K-major SWIZZLE_128B layout by
+//     mrb_tc_pack_conv), streamed from L2 through a small ring of shared-memory slots by the weight-streaming lane.
 //   * A operand = activations, held in TENSOR MEMORY (tcgen05.mma with A from TMEM): a ring of TMEM stages of
-//     64 columns (32 hi + 32 lo columns of packed bf16 pairs = one 64-channel K chunk for the 128 pixels/lanes).  Shared memory
-//     therefore carries no activation traffic for the MMAs, and the ring is deep (5-6 stages) although the
-//     resident weights fill most of shared memory -- the mbarrier round trip loader -> MMA -> commit -> loader
-//     measured at ~2k cycles needs that depth.
-//   loader warps (2 groups x 4, alternating segments): coalesced gather of a [128 px x 64 ch] fp32 chunk per
-//                     "segment" (source tensor, tap offset with replicate clamp, channel chunk) with the next
-//                     segment's loads in flight in registers; a per-warp 4 KB swizzled staging tile turns the
-//                     coalesced (4 rows x 128 B per instruction) view into row ownership (thread = pixel = TMEM
-//                     lane); split into hi/lo and tcgen05.st into the stage;
-//   MMA warp (1 lane) 4 k-steps (K = 16) x 3 tcgen05.mma.kind::f16 per segment (A from TMEM, B descriptor in smem) and
-//                     tcgen05.commit of the stage back to the loaders / of the accumulator to the epilogue;
-//   epilogue warps (8) tcgen05.ld the accumulator (one pixel per thread, 2 warps per lane quadrant), apply
-//                     bias + ReLU or the GRU gates, and write NHWC.
+//     64 columns (32 hi + 32 lo columns of packed bf16 pairs = one 64-channel K chunk for the 128 positions/lanes).
+//     Shared memory therefore carries no activation traffic for the MMAs.
+//   loader warps (2 groups x 4, alternating (tile, kernel row) units): cp.async gather of the warp's 32 positions plus
+//                     the halo of one kernel row into a swizzled staging tile (current + next in flight); tap kx of that
+//                     row is staging row lane + kx*dil, copied to the TMEM stage with tcgen05.st (thread = position = TMEM
+//                     lane);
+//   MMA warp (1 lane) 4 k-steps (K = 16) x 2 stacked tcgen05.mma.kind::f16 per segment (A from TMEM, B descriptor in smem)
+//                     and tcgen05.commit of the stage back to the loaders / of the accumulator to the epilogue;
+//   epilogue warps (8) tcgen05.ld the accumulator (one position per thread, 2 warps per lane quadrant), apply bias and
+//                     optional ReLU, split into hi / lo bf16 and stage the tile in the TMA box layout;
+//   TMA store lane    the two box stores of each tile.
 #include <cuda.h>
 
 #include "tc_ptx.cuh"
@@ -38,27 +39,24 @@ namespace mrb {
 namespace tc {
 
 constexpr int TILE_M = 128;
+constexpr int COUT = 64;                      // output channels (all of them in one CTA)
 constexpr int KC = 32;                        // TMEM columns of one K chunk half (hi or lo): 64 bf16 channels, packed in pairs
 constexpr int KCH = 64;                       // channels per K chunk (one 128-byte row of bf16 in the B operand)
 constexpr int A_STAGE_COLS = 2 * KC;          // hi + lo
 constexpr int EPI_WARPS = 8;                  // 2 warps per TMEM lane quadrant (each takes half of the channels)
-constexpr int LOAD_GROUPS = 2, LOAD_WARPS = 4 * LOAD_GROUPS;  // loader groups alternate segments
-constexpr int MMA_WARPS = 2;                  // two issuing lanes (alternate segments): one thread cannot feed the pipe
+constexpr int LOAD_GROUPS = 2, LOAD_WARPS = 4 * LOAD_GROUPS;  // loader groups alternate (tile, kernel row) units
+constexpr int MMA_WARPS = 2;                  // MMA issuer + TMA store lane
 constexpr int THREADS = (EPI_WARPS + LOAD_WARPS + MMA_WARPS + 1) * 32;  // + weight-streaming warp
 constexpr int B_STAGES = 6;                   // max depth of the streamed-weights ring (Params::b_stages)
 constexpr int MAX_SEGS = 25;
 constexpr int MAX_STAGES = 6;
-constexpr int TBUF_BYTES = 2 * 32 * 128;      // per loader warp staging tile: 32 pixels x 64 fp32 channels, as two
-                                              // [32 rows x 128 B] swizzled halves (channels 0-31 | 32-63)
-constexpr int EPI_ROW_BYTES = 80;             // 64 B of payload per pixel, padded: conflict-free for both access patterns
-constexpr int EPI_TILE_BYTES = 32 * EPI_ROW_BYTES;
-constexpr int HALO_ROWS = 40;                 // halo mode: 32 pixels + 2*pad on each side of up to two image-row pieces
+constexpr int W_CHUNK_BYTES = COUT * 128;     // hi (or lo) rows of one weight chunk
 
-enum Mode { MODE_CONV_RELU = 0, MODE_GRU = 1, MODE_CONV_NOACT = 2 };
 constexpr int BH_PAD = 2;                     // replicate border of the BH activation layout (conv_tc2.cu)
 constexpr int BH_PX_BYTES = 256;              // 64 hi + 64 lo bf16 per position
 constexpr int OUT_BOX_BYTES = TILE_M * 128;   // one [128 positions x 64 bf16] TMA box
-constexpr int BIAS_FLOATS = 384;              // GRU: 3 x 64 gate biases; conv: bias [0,128) | IndRNN recurrent weights [128,256)
+constexpr int HALO_ROWS = 32 + 2 * BH_PAD;    // staging rows of one loader unit at most: 32 positions + pad on each side
+constexpr int BIAS_FLOATS = COUT;
 
 // Profiling hooks (per-role cycle counters, role switches) exist only in the tools build (-DMRB_TC_PROF,
 // tools/libmridc_b200_tools.so); the product kernel carries none of them.
@@ -70,84 +68,38 @@ constexpr int BIAS_FLOATS = 384;              // GRU: 3 x 64 gate biases; conv: 
 #define TC_DBG(P, flag) false
 #endif
 
-struct Segment {
-    short src;     // 0 / 1: which input tensor
-    short dy, dx;  // pixel offset of this tap (replicate clamp)
-    short c0;      // first channel of the 64-channel chunk in the source (or im2col chunk index when im2col != 0)
-    short wchunk;  // weight chunk index
-    short dcol;    // accumulator column offset
-    short n;       // MMA N for this segment
-    short first;   // non-stacked issue: 1: first contribution to its accumulator columns (overwrite); 2: GRU x-part
-                   // (see umma_first_split).  Stacked issue derives "first" from the segment index (see the issuers).
-};
-
 struct Params {
-    const float* src[2];     // NHWC inputs [B, H, W, cs]
-    int cs[2];               // channels per pixel of each source
-    const void* wpack;       // packed bf16 weights: [half][chunk][hi|lo][n rows x 128 B swizzled]
-    const float* bias;       // conv: [Cout]; GRU: b_ih [3*Ch] (may be null)
-    const float* hprev;      // GRU / IndRNN: previous hidden state NHWC [P, Ch]
-    const float* add_scale;  // conv modes, IndRNN (rnn_cells.py:391): out = act(conv + bias + add_scale[c] * hprev[p][c]); null = off
-    float* out;              // NHWC [P, Cout]
-    int B, H, W;
-    long long P;             // B*H*W pixels
+    const uint8_t* src;      // BH input (replicate border valid)
+    const void* wpack;       // packed bf16 weights: [tap][hi|lo][64 rows x 128 B swizzled]
+    const float* bias;       // [64] (may be null)
+    int B, H, W;             // image size
+    long long P;             // flat positions of the BH layout, B (H+4)(W+4): the tiles run over them
     int n_tiles;
-    int nseg;                // segments (64-channel K chunks) per tile; the global segment stream s = item * nseg + sgi
-                             // is dealt round-robin to the loader groups, the TMEM stages, the weight ring and the issuers
-    int wchunk_rows;         // rows (N) of one weight chunk
-    int n_wchunks;
-    int acc_cols;            // TMEM columns of one accumulator buffer
-    int acc_bufs;            // 1 or 2 accumulator buffers
+    int nseg;                // segments (taps) per tile; the global segment stream s = item * nseg + sgi is dealt to
+                             // the TMEM stages and the weight ring
+    int acc_cols;            // TMEM columns of one accumulator buffer: [hi*hi chain | cross-term chain]
+    int acc_bufs;            // accumulator buffers
     int tmem_cols;           // allocation: 512
-    int cout;                // output channels per pixel (both halves)
-    int n_split;             // 1 or 2: CTAs per pixel tile (each takes cout / n_split output channels)
-    int nhalf;               // output channels handled per item (cout / n_split)
-    int mode;
-    int stream_b;            // 1: weights are not resident; a dedicated lane streams the B chunk of every segment
-                             // (hi rows | lo rows, wchunk_rows*256 B) through a ring of b_stages slots
+    int relu;
     int b_stages;            // depth of the streamed-weights ring (<= B_STAGES)
-    int tb_depth;            // cp.async staging tiles per loader warp (2 or 3)
-    int tb_half;             // bytes of one staging half (32 rows x 128 B, or HALO_ROWS rows in halo mode)
+    int tb_depth;            // cp.async staging tiles per loader warp
+    int tb_half;             // bytes of one staging half (32 + 2*pad rows x 128 B)
     int tb_bytes;            // bytes of one staging tile (2 halves)
-    int halo;                // 1: k x k conv, one gather per (tile, kernel row) feeds the k taps of that row (see loaders)
-    int ksz, dil;            // conv geometry (halo mode)
+    int ksz, dil;            // conv geometry
     int stages;              // A stages in TMEM (columns acc_bufs*acc_cols + 64*s)
-    int im2col;              // != 0: source 0 is [B,H,W,4] and chunk c0 holds taps 16*c0 .. 16*c0+15 of a 5x5 window
-                             // (1: gathered tap by tap from global memory, 2: from a halo patch in shared memory)
-    int ngroups;             // conv: number of independent accumulator groups (each [hi*hi | cross], 2*nhalf columns);
-                             // the tensor core's fp32 accumulation truncates, so its error grows linearly with the
-                             // chain length -- short chains summed in the epilogue (RN fp32) keep it at fp32 level
-    int pos_padded;          // tiles run over the flat positions of the BH layout, [B][H+4][W+4] (P = B (H+4)(W+4)); H, W stay
-                             // the image size.  Required by src_bh / out_bh.
-    int src_bh;              // source 0 is a BH tensor (bf16 hi | lo per position, replicate border valid): the loaders
-                             // copy rows to TMEM without conversion and address taps as plain offsets (no clamping)
-    int out_bh;              // the epilogue splits its fp32 results into hi / lo bf16 (cout == 64).  1: the tile is staged in the
-                             // TMA box layout and stored by a TMA store lane (one issuer); 2: straight st.global from the
-                             // thread that owns the position (used where the 32 KB of the output tile buy a deeper weight
-                             // ring and a second MMA issuer instead)
-    int group_cols;          // TMEM columns between the accumulator groups of the two issuers (0 with one group)
-    int n_issuers;           // 1 or 2 MMA-issuing lanes (2: the global segment stream alternates; issuer i owns
-                             // accumulator group i)
-    int stacked;             // 1: stacked-B issue (2 MMAs per k-step); requires small_off == n of every segment
-    int small_off;           // != 0: the two cross terms (lo*hi, hi*lo) accumulate in columns dcol + small_off, so the
-                             // long hi*hi chain sees 3x fewer (truncating) tensor-core accumulations; summed in the epilogue
 #ifdef MRB_TC_PROF
     unsigned long long* prof; // optional [gridDim.x][16] cycle counters (tools/tc_roles.py)
     int debug;                // role switches: 1 skip MMAs, 2 skip global loads, 4 skip epilogue math, 8 skip tcgen05.st
 #endif
-    Segment seg[MAX_SEGS];
 };
 
-template <bool GRU>
 __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ CUtensorMap tm_out, const Params P) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
-    // layout: [weights resident][loader staging tiles][streamed-weights ring][barriers][bias][epilogue exchange]
+    // layout: [output tile][streamed-weights ring][loader staging tiles][barriers][bias]
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    const int wbytes_chunk = P.wchunk_rows * 128;  // bytes of the hi (or lo) rows of one weight chunk
-    uint8_t* out_s = smem;                                            // out_bh: [hi box | lo box] output tile (1024-aligned)
-    uint8_t* w_s = smem + (P.out_bh == 1 ? 2 * OUT_BOX_BYTES : 0);         // [n_wchunks][hi|lo][rows*128]
-    uint8_t* bst_s = w_s + (P.stream_b ? 0 : (size_t)P.n_wchunks * 2 * wbytes_chunk);  // [b_stages][2*wbytes_chunk] if stream_b
-    uint8_t* tb_s = bst_s + (P.stream_b ? (size_t)P.b_stages * 2 * wbytes_chunk : 0);  // [LOAD_WARPS][depth][tb_bytes]
+    uint8_t* out_s = smem;                                            // [hi box | lo box] output tile (1024-aligned)
+    uint8_t* bst_s = smem + 2 * OUT_BOX_BYTES;                        // [b_stages][2*W_CHUNK_BYTES]
+    uint8_t* tb_s = bst_s + (size_t)P.b_stages * 2 * W_CHUNK_BYTES;   // [LOAD_WARPS][depth][tb_bytes]
     uint64_t* bars = (uint64_t*)(tb_s + (size_t)LOAD_WARPS * P.tb_depth * P.tb_bytes);
     uint64_t* full = bars;                          // [MAX_STAGES]
     uint64_t* empty = bars + MAX_STAGES;            // [MAX_STAGES]
@@ -156,17 +108,15 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
     uint32_t* tmem_slot = (uint32_t*)(acc_empty + 2);
     uint64_t* b_full = acc_empty + 4;               // [B_STAGES]
     uint64_t* b_empty = b_full + B_STAGES;          // [B_STAGES]
-    uint64_t* out_free = acc_empty + 3;             // [1] out_bh: the TMA stores of the previous tile have read out_s
-    uint64_t* out_ready = b_empty + B_STAGES;       // [1] out_bh: every epilogue warp has written its part of the output tile
+    uint64_t* out_free = acc_empty + 3;             // [1] the TMA stores of the previous tile have read out_s
+    uint64_t* out_ready = b_empty + B_STAGES;       // [1] every epilogue warp has written its part of the output tile
     float* bias_s = (float*)(out_ready + 2);        // [BIAS_FLOATS] (16-byte aligned): bias staged once per CTA
-    uint8_t* epi_s = (uint8_t*)(bias_s + BIAS_FLOATS);  // GRU: [EPI_WARPS][2][32 px][EPI_ROW_BYTES] per-warp exchange tiles
 
-    // warp index through a shuffle: provably warp-uniform for the compiler (role branches and the MMA issuers' operands
+    // warp index through a shuffle: provably warp-uniform for the compiler (role branches and the MMA issuer's operands
     // then live in uniform registers)
     const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
-    const int half = blockIdx.x % P.n_split;
-    const int first_tile = blockIdx.x / P.n_split;
-    const int tile_stride = gridDim.x / P.n_split;
+    const int first_tile = blockIdx.x;
+    const int tile_stride = gridDim.x;
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < P.stages; ++s) {
@@ -174,7 +124,7 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
             mbar_init(&empty[s], 1);
         }
         for (int b = 0; b < 2; ++b) {
-            mbar_init(&acc_full[b], P.n_issuers);
+            mbar_init(&acc_full[b], 1);
             mbar_init(&acc_empty[b], EPI_WARPS);  // one arrival per epilogue warp
         }
         for (int b = 0; b < B_STAGES; ++b) {
@@ -185,29 +135,8 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
         mbar_init(out_ready, EPI_WARPS);
         fence_barrier_init();
     }
-    {
-        // GRU: the r and z biases are pre-scaled by -log2(e) for sigmoid_fused()
-        const int nb = GRU ? 3 * P.cout : P.cout;
-        for (int i = threadIdx.x; i < nb; i += THREADS) {
-            const float b = P.bias ? P.bias[i] : 0.f;
-            bias_s[i] = (GRU && i < 2 * P.cout) ? -kLog2e * b : b;
-        }
-        if (!GRU && P.add_scale)  // IndRNN recurrent weights, second row of the table
-            for (int i = threadIdx.x; i < P.cout; i += THREADS) bias_s[128 + i] = P.add_scale[i];
-    }
+    for (int i = threadIdx.x; i < COUT; i += THREADS) bias_s[i] = P.bias ? P.bias[i] : 0.f;
     if (warp == EPI_WARPS + LOAD_WARPS) tmem_alloc(tmem_slot, (uint32_t)P.tmem_cols);
-    // resident weights of this half: straight copy (already swizzled by the packer)
-    if (!P.stream_b) {
-        const float4* g = reinterpret_cast<const float4*>(P.wpack) + (size_t)half * P.n_wchunks * 2 * wbytes_chunk / 16;
-        const uint32_t s = smem_u32(w_s);
-        const int n16 = P.n_wchunks * 2 * wbytes_chunk / 16;
-        for (int i = threadIdx.x; i < n16; i += THREADS) {
-            const float4 v = __ldg(g + i);
-            asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(s + 16u * (uint32_t)i), "f"(v.x), "f"(v.y), "f"(v.z),
-                         "f"(v.w)
-                         : "memory");
-        }
-    }
     fence_proxy_async();
     tc_fence_before();
     __syncthreads();
@@ -218,17 +147,15 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
     for (int t = first_tile; t < P.n_tiles; t += tile_stride) ++n_items;
     if (warp >= EPI_WARPS && warp < EPI_WARPS + LOAD_WARPS) {
         // ============================== LOADERS ==============================
-        // The global segment stream s = item * nseg + sgi is dealt to the two loader groups (generic / patch mode:
-        // alternate segments; halo mode: alternate (tile, kernel row) units of k segments); segment s goes to TMEM stage
-        // s % stages.
+        // The global segment stream s = item * nseg + sgi is dealt to the two loader groups in (tile, kernel row) units
+        // of k segments; segment s goes to TMEM stage s % stages.
         const int lw = warp - EPI_WARPS;
         const int grp = lw >> 2;                     // loader group
         const int quad = lw & 3;                     // == warp % 4: the TMEM lane quadrant this warp may write
         const int c16 = lane & 7;                    // 16-byte chunk within a 128-byte half row (coalesced view)
-        const int rl0 = lane >> 3;                   // rows rl0 + 4*i of the warp's 32 rows (coalesced view)
+        const int rl0 = lane >> 3;                   // rows rl0 + 4*i of the staging tile (coalesced view)
         const uint32_t tb_u32 = smem_u32(tb_s + (size_t)lw * P.tb_depth * P.tb_bytes);  // tb_depth staging tiles of this warp
-        const uint32_t HB = (uint32_t)P.tb_half;     // channels 32-63 of a staging row live HB bytes after channels 0-31
-        const uint32_t W32 = (uint32_t)P.W, H32 = (uint32_t)P.H;
+        const uint32_t HB = (uint32_t)P.tb_half;     // the lo half of a staging row lives HB bytes after the hi half
         const bool ld_on = !TC_DBG(P, 2);
         TCP(long long t_start = clock64(), t_wait = 0, t_st = 0, t_issue = 0, t_stw = 0, c0;)
 
@@ -239,44 +166,26 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
             stage += n;
             while (stage >= P.stages) { stage -= P.stages; phase ^= 1u; }
         };
-        // staging row `row` of tile tb (64 fp32 channels) -> bf16 hi/lo split -> TMEM stage (thread = pixel = TMEM lane
-        // quad*32 + lane): columns [0,32) = hi pairs, [32,64) = lo pairs
+        // staging row `row` of tile tb (64 hi bf16 in half 0, 64 lo bf16 in half 1) -> TMEM stage (thread = position =
+        // TMEM lane quad*32 + lane): columns [0,32) = hi pairs, [32,64) = lo pairs -- a straight copy
         auto store_stage = [&](uint32_t tb, int row, int stg) {
             const uint32_t ta = tmem_base + ((uint32_t)(quad * 32) << 16) + a_col0 + (uint32_t)(stg * A_STAGE_COLS);
-            if (P.src_bh) {
-                // BH source: the staging row already holds 64 hi bf16 (half 0) and 64 lo bf16 (half 1) -- straight copy
-#pragma unroll
-                for (int hf = 0; hf < 2; ++hf) {
-                    uint32_t v[32];
-#pragma unroll
-                    for (int c = 0; c < 8; ++c) {
-                        const float4 a = lds128(tb + hf * HB + swz(row, c));
-                        v[4 * c] = __float_as_uint(a.x); v[4 * c + 1] = __float_as_uint(a.y);
-                        v[4 * c + 2] = __float_as_uint(a.z); v[4 * c + 3] = __float_as_uint(a.w);
-                    }
-                    if (!TC_DBG(P, 8)) {
-                        tmem_st16(ta + hf * KC, v);
-                        tmem_st16(ta + hf * KC + 16, v + 16);
-                    }
-                }
-                return;
-            }
 #pragma unroll
             for (int hf = 0; hf < 2; ++hf) {
-                uint32_t hi[16], lo[16];
+                uint32_t v[32];
 #pragma unroll
                 for (int c = 0; c < 8; ++c) {
                     const float4 a = lds128(tb + hf * HB + swz(row, c));
-                    split_bf16x2(a.x, a.y, hi[2 * c], lo[2 * c]);
-                    split_bf16x2(a.z, a.w, hi[2 * c + 1], lo[2 * c + 1]);
+                    v[4 * c] = __float_as_uint(a.x); v[4 * c + 1] = __float_as_uint(a.y);
+                    v[4 * c + 2] = __float_as_uint(a.z); v[4 * c + 3] = __float_as_uint(a.w);
                 }
                 if (!TC_DBG(P, 8)) {
-                    tmem_st16(ta + hf * 16, hi);
-                    tmem_st16(ta + KC + hf * 16, lo);
+                    tmem_st16(ta + hf * KC, v);
+                    tmem_st16(ta + hf * KC + 16, v + 16);
                 }
             }
         };
-        // wait for the stage, convert + store one staging row per lane, hand the stage to the issuers
+        // wait for the stage, copy one staging row per lane, hand the stage to the issuer
         auto fill_stage = [&](uint32_t tb, int row) {
             TCP(c0 = clock64();)
             mbar_wait_sleep(&empty[stage], phase ^ 1, 40);
@@ -292,388 +201,55 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
             TCP(t_st += clock64() - c0; t_stw += clock64() - c2;)
         };
 
-        if (P.halo && P.src_bh) {
-            // ---- halo mode on a BH source: flat positions, valid replicate border => taps are plain offsets ----
-            // unit = (tile, kernel row ky): the warp's 32 positions plus pad on each side of flat row offset
-            // (ky*dil - pad) * pitch; tap kx reads staging row lane + kx*dil.  Positions outside the tensor are zero-filled
-            // (they only feed border positions, whose results are not used).
-            const int k = P.ksz, dil = P.dil, pad = dil * (k - 1) / 2;
-            const uint8_t* src = reinterpret_cast<const uint8_t*>(P.src[0]);
-            const long long pitch = P.W + 2 * BH_PAD;
-            const int n_units = n_items * k;
-            const int nrows = 32 + 2 * pad;
-            auto issue_halo = [&](int tile, int ky, int slot) {
-                const long long q0 = (long long)tile * TILE_M + quad * 32 - pad + (long long)(ky * dil - pad) * pitch;
-                const uint32_t sbase = tb_u32 + (uint32_t)(slot * P.tb_bytes);
+        // unit = (tile, kernel row ky): the warp's 32 positions plus pad on each side of flat row offset
+        // (ky*dil - pad) * pitch; tap kx reads staging row lane + kx*dil.  Positions outside the tensor are zero-filled
+        // (they only feed border positions, whose results are not used).
+        const int k = P.ksz, dil = P.dil, pad = dil * (k - 1) / 2;
+        const long long pitch = P.W + 2 * BH_PAD;
+        const int n_units = n_items * k;
+        const int nrows = 32 + 2 * pad;
+        auto issue_halo = [&](int tile, int ky, int slot) {
+            const long long q0 = (long long)tile * TILE_M + quad * 32 - pad + (long long)(ky * dil - pad) * pitch;
+            const uint32_t sbase = tb_u32 + (uint32_t)(slot * P.tb_bytes);
 #pragma unroll
-                for (int i = 0; i < HALO_ROWS / 4; ++i) {
-                    const int sr = rl0 + 4 * i;
-                    if (sr >= nrows) break;  // the staging tile has exactly nrows rows (a zero-fill would land in the lo half)
-                    const long long q = q0 + sr;
-                    const bool ok = q >= 0 && q < P.P;
-                    const uint8_t* g = src + q * BH_PX_BYTES + c16 * 16;
-                    const uint32_t nb = (ok && ld_on) ? 16u : 0u;
-                    cp_async16(sbase + swz(sr, c16), ok ? (const void*)g : (const void*)src, nb, true);
-                    cp_async16(sbase + HB + swz(sr, c16), ok ? (const void*)(g + 128) : (const void*)src, nb, true);
-                }
-            };
-            int pf_u = grp, pf_tile = first_tile, pf_ky = grp, pf_slot = 0;
+            for (int i = 0; i < HALO_ROWS / 4; ++i) {
+                const int sr = rl0 + 4 * i;
+                if (sr >= nrows) break;  // the staging tile has exactly nrows rows (a zero-fill would land in the lo half)
+                const long long q = q0 + sr;
+                const bool ok = q >= 0 && q < P.P;
+                const uint8_t* g = P.src + q * BH_PX_BYTES + c16 * 16;
+                const uint32_t nb = (ok && ld_on) ? 16u : 0u;
+                cp_async16(sbase + swz(sr, c16), ok ? (const void*)g : (const void*)P.src, nb, true);
+                cp_async16(sbase + HB + swz(sr, c16), ok ? (const void*)(g + 128) : (const void*)P.src, nb, true);
+            }
+        };
+        int pf_u = grp, pf_tile = first_tile, pf_ky = grp, pf_slot = 0;
+        while (pf_ky >= k) { pf_ky -= k; pf_tile += tile_stride; }
+        auto prefetch_unit = [&]() {
+            if (pf_u < n_units) issue_halo(pf_tile, pf_ky, pf_slot);
+            asm volatile("cp.async.commit_group;" ::: "memory");
+            pf_u += LOAD_GROUPS;
+            pf_ky += LOAD_GROUPS;
             while (pf_ky >= k) { pf_ky -= k; pf_tile += tile_stride; }
-            auto prefetch_unit = [&]() {
-                if (pf_u < n_units) issue_halo(pf_tile, pf_ky, pf_slot);
-                asm volatile("cp.async.commit_group;" ::: "memory");
-                pf_u += LOAD_GROUPS;
-                pf_ky += LOAD_GROUPS;
-                while (pf_ky >= k) { pf_ky -= k; pf_tile += tile_stride; }
-                pf_slot ^= 1;
-            };
+            pf_slot ^= 1;
+        };
+        prefetch_unit();
+        int slot = 0;
+        stage_set((long long)grp * k);
+        for (int u = grp; u < n_units; u += LOAD_GROUPS) {
+            TCP(c0 = clock64();)
             prefetch_unit();
-            int slot = 0;
-            stage_set((long long)grp * k);
-            for (int u = grp; u < n_units; u += LOAD_GROUPS) {
-                TCP(c0 = clock64();)
-                prefetch_unit();
-                TCP(t_issue += clock64() - c0;)
-                asm volatile("cp.async.wait_group 1;" ::: "memory");
-                __syncwarp();
-                const uint32_t tb = tb_u32 + (uint32_t)(slot * P.tb_bytes);
-                for (int kx = 0; kx < k; ++kx) {
-                    fill_stage(tb, lane + kx * dil);
-                    stage_adv(1);
-                }
-                __syncwarp();  // every lane has read its rows before the slot is refilled
-                stage_adv(k * (LOAD_GROUPS - 1));  // the other group's unit
-                slot ^= 1;
+            TCP(t_issue += clock64() - c0;)
+            asm volatile("cp.async.wait_group 1;" ::: "memory");
+            __syncwarp();
+            const uint32_t tb = tb_u32 + (uint32_t)(slot * P.tb_bytes);
+            for (int kx = 0; kx < k; ++kx) {
+                fill_stage(tb, lane + kx * dil);
+                stage_adv(1);
             }
-        } else if (P.halo) {
-            // ---- halo mode (k x k conv over 64 channels) ----
-            // The k taps of one kernel row read the same image row shifted by dil pixels.  One gather per (tile, kernel
-            // row) brings the warp's 32 pixels plus pad = dil*(k-1)/2 pixels on each side (replicate clamp applied to the
-            // source column) into a staging tile; tap kx then reads staging row lane + kx*dil.  A warp's 32 pixels may
-            // straddle two image rows: the second piece gets its own 2*pad halo (rows shifted by another 2*pad).
-            // Cuts the gathers (issue slots and L2 traffic) by k.  The two loader groups take alternate units.
-            const int k = P.ksz, dil = P.dil, pad = dil * (k - 1) / 2;
-            const int cs = P.cs[0];
-            const float* src = P.src[0];
-            const int n_units = n_items * k;
-            // per-tile geometry of this lane's staging rows s = rl0 + 4*i
-            int xoff[HALO_ROWS / 4];
-            unsigned selB = 0, rowok = 0;
-            int nA = 32;
-            long long rowA = 0, rowB = 0;  // (b*H + y) of the two pieces (before the tap's dy)
-            int yA = 0, yB = 0;
-            auto tile_geometry = [&](int tile) {
-                const long long p0 = (long long)tile * TILE_M + quad * 32;
-                selB = 0; rowok = 0;
-                if (p0 >= P.P) return;
-                const uint32_t q = (uint32_t)p0;
-                const uint32_t t = q / W32;
-                const int x0 = (int)(q - t * W32);
-                const uint32_t b0 = t / H32;
-                yA = (int)(t - b0 * H32);
-                rowA = (long long)b0 * P.H;
-                nA = min(32, P.W - x0);
-                const bool hasB = nA < 32 && p0 + nA < P.P;
-                yB = yA + 1;
-                rowB = rowA;
-                if (yB == P.H) { yB = 0; rowB += P.H; }
-                const int nrows = 32 + 2 * pad + (nA < 32 ? 2 * pad : 0);
-#pragma unroll
-                for (int i = 0; i < HALO_ROWS / 4; ++i) {
-                    const int sr = rl0 + 4 * i;
-                    const bool inB = sr >= nA + 2 * pad;
-                    const int vx = inB ? sr - nA - 3 * pad : x0 - pad + sr;
-                    xoff[i] = min(max(vx, 0), P.W - 1) * cs;
-                    if (inB) selB |= 1u << i;
-                    if (sr < nrows && (!inB || hasB)) rowok |= 1u << i;
-                }
-            };
-            int geo_tile = -1;
-            auto issue_halo = [&](int tile, int ky, int slot) {
-                if (tile != geo_tile) { geo_tile = tile; tile_geometry(tile); }
-                const int dy = ky * dil - pad;
-                const float* gA = src + (rowA + min(max(yA + dy, 0), P.H - 1)) * P.W * cs + c16 * 4;
-                const float* gB = src + (rowB + min(max(yB + dy, 0), P.H - 1)) * P.W * cs + c16 * 4;
-                const uint32_t sbase = tb_u32 + (uint32_t)(slot * P.tb_bytes);
-#pragma unroll
-                for (int i = 0; i < HALO_ROWS / 4; ++i) {
-                    const bool ok = (rowok >> i) & 1u;
-                    const float* g = (((selB >> i) & 1u) ? gB : gA) + xoff[i];
-                    const uint32_t nb = (ok && ld_on) ? 16u : 0u;
-                    cp_async16(sbase + swz(rl0 + 4 * i, c16), ok ? (const void*)g : (const void*)src, nb, true);
-                    cp_async16(sbase + HB + swz(rl0 + 4 * i, c16), ok ? (const void*)(g + 32) : (const void*)src, nb, true);
-                }
-            };
-            int pf_u = grp, pf_tile = first_tile, pf_ky = grp, pf_slot = 0;
-            while (pf_ky >= k) { pf_ky -= k; pf_tile += tile_stride; }
-            auto prefetch_unit = [&]() {
-                if (pf_u < n_units) issue_halo(pf_tile, pf_ky, pf_slot);
-                asm volatile("cp.async.commit_group;" ::: "memory");
-                pf_u += LOAD_GROUPS;
-                pf_ky += LOAD_GROUPS;
-                while (pf_ky >= k) { pf_ky -= k; pf_tile += tile_stride; }
-                pf_slot ^= 1;
-            };
-            prefetch_unit();
-            int slot = 0, ky = grp, tile = first_tile;
-            while (ky >= k) { ky -= k; tile += tile_stride; }
-            stage_set((long long)grp * k);
-            for (int u = grp; u < n_units; u += LOAD_GROUPS) {
-                // nA of the tile being consumed (the prefetch cursor may already be on the next tile)
-                const long long p0 = (long long)tile * TILE_M + quad * 32;
-                const uint32_t q = p0 < P.P ? (uint32_t)p0 : 0u;
-                const int nA_cur = min(32, P.W - (int)(q % W32));
-                TCP(c0 = clock64();)
-                prefetch_unit();
-                TCP(t_issue += clock64() - c0;)
-                asm volatile("cp.async.wait_group 1;" ::: "memory");
-                __syncwarp();
-                const uint32_t tb = tb_u32 + (uint32_t)(slot * P.tb_bytes);
-                const int row0 = lane + (lane >= nA_cur ? 2 * pad : 0);
-                for (int kx = 0; kx < k; ++kx) {
-                    fill_stage(tb, row0 + kx * dil);
-                    stage_adv(1);
-                }
-                __syncwarp();  // every lane has read its rows before the slot is refilled
-                stage_adv(k * (LOAD_GROUPS - 1));  // the other group's unit
-                slot ^= 1;
-                ky += LOAD_GROUPS;
-                while (ky >= k) { ky -= k; tile += tile_stride; }
-            }
-        } else if (P.im2col == 2) {
-            // ---- 5x5 x 4-channel im2col from a halo patch (nseg == LOAD_GROUPS: group g assembles K chunk g) ----
-            // One gather per tile brings the warp's 32 pixels (+2 on each side, two-piece layout as above) of the five
-            // image rows y-2..y+2 into a [5][HALO_ROWS] x 16 B patch; the two K chunks (16 taps x 4 channels each, taps
-            // 25..31 zero) are then assembled from shared memory: tap (ky, kx) of pixel `lane` is patch[ky][row0 + kx].
-            const float* src = P.src[0];
-            constexpr int PAD = 2, NE = (5 * HALO_ROWS + 31) / 32;  // patch elements per lane
-            int eoff[NE];      // clamped source column (in floats) of patch element e = lane + 32*i
-            unsigned eB = 0, eok = 0;
-            int nA = 32, yA = 0, yB = 0;
-            long long rowA = 0, rowB = 0;
-            // pos_padded: the tile's positions are those of the BH layout (rows of W + 4 positions, H + 4 rows per image);
-            // position (yp, xp) reads the source window centred at (yp - 2, xp - 2), clamped -- exact for interior
-            // positions, and the results at border positions are not used
-            const int roff = P.pos_padded ? BH_PAD : 0;                    // position -> source coordinate offset
-            const uint32_t Wq = (uint32_t)(P.W + 2 * roff), Hq = (uint32_t)(P.H + 2 * roff);  // position grid
-            auto tile_geometry = [&](int tile) {
-                const long long p0 = (long long)tile * TILE_M + quad * 32;
-                eB = 0; eok = 0;
-                if (p0 >= P.P) return;
-                const uint32_t q = (uint32_t)p0;
-                const uint32_t t = q / Wq;
-                const int xq = (int)(q - t * Wq);
-                const int x0 = xq - roff;
-                const uint32_t b0 = t / Hq;
-                const int yq = (int)(t - b0 * Hq);
-                yA = yq - roff;
-                rowA = (long long)b0 * P.H;
-                nA = min(32, (int)Wq - xq);
-                const bool hasB = nA < 32 && p0 + nA < P.P;
-                yB = yA + 1;
-                rowB = rowA;
-                if (yq + 1 == (int)Hq) { yB = -roff; rowB += P.H; }
-                const int nrows = 32 + 2 * PAD + (nA < 32 ? 2 * PAD : 0);
-#pragma unroll
-                for (int i = 0; i < NE; ++i) {
-                    const int e = lane + 32 * i;
-                    const int sr = e % HALO_ROWS;
-                    const bool inB = sr >= nA + 2 * PAD;
-                    const int vx = inB ? sr - nA - 3 * PAD - roff : x0 - PAD + sr;
-                    eoff[i] = min(max(vx, 0), P.W - 1) * 4;
-                    if (inB) eB |= 1u << i;
-                    if (e < 5 * HALO_ROWS && sr < nrows && (!inB || hasB)) eok |= 1u << i;
-                }
-            };
-            auto issue_patch = [&](int tile, int slot) {
-                tile_geometry(tile);
-                const uint32_t sbase = tb_u32 + (uint32_t)(slot * P.tb_bytes);
-#pragma unroll
-                for (int i = 0; i < NE; ++i) {
-                    const int e = lane + 32 * i;
-                    const int ky = e / HALO_ROWS;
-                    const bool ok = (eok >> i) & 1u;
-                    const bool inB = (eB >> i) & 1u;
-                    const int yy = min(max((inB ? yB : yA) + ky - PAD, 0), P.H - 1);
-                    const float* g = src + ((inB ? rowB : rowA) + yy) * P.W * 4 + eoff[i];
-                    cp_async16(sbase + 16u * (uint32_t)e, ok ? (const void*)g : (const void*)src, (ok && ld_on) ? 16u : 0u, true);
-                }
-            };
-            int pf_t = 0, pf_tile = first_tile, pf_slot = 0;
-            auto prefetch_patch = [&]() {
-                if (pf_t < n_items) issue_patch(pf_tile, pf_slot);
-                asm volatile("cp.async.commit_group;" ::: "memory");
-                ++pf_t;
-                pf_tile += tile_stride;
-                pf_slot ^= 1;
-            };
-            prefetch_patch();
-            int slot = 0, tile = first_tile;
-            stage_set(grp);
-            for (int it = 0; it < n_items; ++it, tile += tile_stride) {
-                const long long p0 = (long long)tile * TILE_M + quad * 32;
-                const uint32_t q = p0 < P.P ? (uint32_t)p0 : 0u;
-                const int nA_cur = min(32, (int)Wq - (int)(q % Wq));
-                TCP(c0 = clock64();)
-                prefetch_patch();
-                TCP(t_issue += clock64() - c0;)
-                asm volatile("cp.async.wait_group 1;" ::: "memory");
-                __syncwarp();
-                const uint32_t tb = tb_u32 + (uint32_t)(slot * P.tb_bytes);
-                const int row0 = lane + (lane >= nA_cur ? 2 * PAD : 0);
-                TCP(c0 = clock64();)
-                mbar_wait_sleep(&empty[stage], phase ^ 1, 40);
-                TCP(t_wait += clock64() - c0;)
-                tc_fence_after();
-                TCP(c0 = clock64();)
-                const uint32_t ta = tmem_base + ((uint32_t)(quad * 32) << 16) + a_col0 + (uint32_t)(stage * A_STAGE_COLS);
-#pragma unroll
-                for (int hf = 0; hf < 2; ++hf) {
-                    uint32_t hi[16], lo[16];
-#pragma unroll
-                    for (int c = 0; c < 8; ++c) {
-                        const int t = grp * 16 + hf * 8 + c;            // tap index (K chunk g holds taps 16g .. 16g+15)
-                        const int ky = (t * 13) >> 6, kx = t - 5 * ky;  // t / 5, t % 5 for t < 32
-                        float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-                        if (t < 25) a = lds128(tb + 16u * (uint32_t)(ky * HALO_ROWS + row0 + kx));
-                        split_bf16x2(a.x, a.y, hi[2 * c], lo[2 * c]);
-                        split_bf16x2(a.z, a.w, hi[2 * c + 1], lo[2 * c + 1]);
-                    }
-                    if (!TC_DBG(P, 8)) {
-                        tmem_st16(ta + hf * 16, hi);
-                        tmem_st16(ta + KC + hf * 16, lo);
-                    }
-                }
-                tmem_st_wait();
-                tc_fence_before();
-                __syncwarp();
-            if (lane == 0) mbar_arrive(&full[stage]);
-                TCP(t_st += clock64() - c0;)
-                stage_adv(LOAD_GROUPS);
-                __syncwarp();  // every lane has read its taps before the slot is refilled
-                slot ^= 1;
-            }
-        } else {
-            // ---- generic path: one gather per segment (1x1 kernels: GRU / IndRNN; small images) ----
-            int pb[8], py[8], px[8];
-            bool pv[8];
-            int coords_tile = -1;
-            bool uniform_rows = false;
-            // cp.async gather of one segment into staging tile `slot` (no registers held while in flight); all gathers
-            // bypass L1 (.cg): every activation is read once
-            auto issue_loads = [&](int tile, int sgi, int slot) {
-                const Segment sg = P.seg[sgi];
-                const float* src = P.src[sg.src];
-                const int cs = P.cs[sg.src];
-                const uint32_t sbase = tb_u32 + (uint32_t)(slot * P.tb_bytes);
-                const long long gstep = 4ll * cs;
-                if (!P.im2col && sg.dy == 0 && sg.dx == 0) {
-                    // centre tap / 1x1 kernel: pixel p is row p of the [P, cs] matrix -- no (b, y, x) decomposition, no clamp
-                    const long long p0 = (long long)tile * TILE_M + quad * 32 + rl0;
-                    const float* g = src + p0 * cs + sg.c0 + c16 * 4;
-                    if ((long long)(tile + 1) * TILE_M <= P.P) {  // whole tile inside the image stack: no per-row predicate
-                        const uint32_t nbytes = ld_on ? 16u : 0u;
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) {
-                            cp_async16(sbase + swz(rl0 + 4 * i, c16), g + i * gstep, nbytes, true);
-                            cp_async16(sbase + HB + swz(rl0 + 4 * i, c16), g + i * gstep + 32, nbytes, true);
-                        }
-                        return;
-                    }
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        const bool ok = p0 + 4 * i < P.P;
-                        const uint32_t nbytes = (ok && ld_on) ? 16u : 0u;
-                        cp_async16(sbase + swz(rl0 + 4 * i, c16), ok ? g + i * gstep : src, nbytes, true);
-                        cp_async16(sbase + HB + swz(rl0 + 4 * i, c16), ok ? g + i * gstep + 32 : src, nbytes, true);
-                    }
-                    return;
-                }
-                if (tile != coords_tile) {
-                    coords_tile = tile;
-                    // one division pair per tile; rows rl0 + 4*i follow by carry (x -> y -> b)
-                    const long long p0 = (long long)tile * TILE_M + quad * 32 + rl0;
-                    const uint32_t q = p0 < P.P ? (uint32_t)p0 : 0u;  // P.P < 2^31 (checked on the host)
-                    const uint32_t t = q / W32;
-                    int x = (int)(q - t * W32);
-                    const uint32_t b0 = t / H32;
-                    int y = (int)(t - b0 * H32), b = (int)b0;
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        pv[i] = p0 + 4 * i < P.P;
-                        px[i] = pv[i] ? x : 0; py[i] = pv[i] ? y : 0; pb[i] = pv[i] ? b : 0;
-                        x += 4;
-                        while (x >= P.W) {
-                            x -= P.W;
-                            if (++y == P.H) { y = 0; ++b; }
-                        }
-                    }
-                    uniform_rows = pv[7] && py[7] == py[0] && pb[7] == pb[0];
-                }
-                if (!P.im2col && uniform_rows) {
-                    // fast path: rows rl0 + 4*i are 4 pixels apart on one image row; only y may clamp (uniformly)
-                    const int xlo = px[0] + sg.dx, xhi = px[0] + 28 + sg.dx;
-                    if (xlo >= 0 && xhi < P.W) {
-                        const int yy = min(max(py[0] + sg.dy, 0), P.H - 1);
-                        const float* g = src + (((long long)pb[0] * P.H + yy) * P.W + xlo) * cs + sg.c0 + c16 * 4;
-                        const uint32_t nbytes = ld_on ? 16u : 0u;
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) {
-                            cp_async16(sbase + swz(rl0 + 4 * i, c16), g + i * gstep, nbytes, true);
-                            cp_async16(sbase + HB + swz(rl0 + 4 * i, c16), g + i * gstep + 32, nbytes, true);
-                        }
-                        return;
-                    }
-                }
-#pragma unroll
-                for (int hf = 0; hf < 2; ++hf) {
-                    int dy = sg.dy, dx = sg.dx, coff = sg.c0 + hf * 32 + c16 * 4;
-                    bool tap_ok = true;
-                    if (P.im2col) {
-                        // chunk (hf, c16) of the im2col row = tap t of the 5x5 window (4 channels = one float4)
-                        const int t = sg.c0 * 16 + hf * 8 + c16;
-                        tap_ok = t < 25;
-                        dy = t / 5 - 2; dx = t % 5 - 2; coff = 0;
-                    }
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        const int yy = min(max(py[i] + dy, 0), P.H - 1);
-                        const int xx = min(max(px[i] + dx, 0), P.W - 1);
-                        const float* g = src + (((long long)pb[i] * P.H + yy) * P.W + xx) * cs + coff;
-                        const uint32_t nbytes = (pv[i] && tap_ok && ld_on) ? 16u : 0u;  // 0 -> zero fill
-                        cp_async16(sbase + hf * HB + swz(rl0 + 4 * i, c16), g, nbytes, true);
-                    }
-                }
-            };
-            const long long n_total = (long long)n_items * P.nseg;  // length of the global segment stream
-            const int D = P.tb_depth;
-            // prefetch cursor over this group's segments s = grp, grp + LOAD_GROUPS, ...
-            long long pf_s = grp;
-            int pf_tile = first_tile, pf_sgi = grp, pf_slot = 0;
-            while (pf_sgi >= P.nseg) { pf_sgi -= P.nseg; pf_tile += tile_stride; }
-            auto prefetch_next = [&]() {
-                if (pf_s < n_total) issue_loads(pf_tile, pf_sgi, pf_slot);
-                asm volatile("cp.async.commit_group;" ::: "memory");
-                pf_s += LOAD_GROUPS;
-                pf_sgi += LOAD_GROUPS;
-                while (pf_sgi >= P.nseg) { pf_sgi -= P.nseg; pf_tile += tile_stride; }
-                if (++pf_slot == D) pf_slot = 0;
-            };
-            for (int n = 0; n < D - 1; ++n) prefetch_next();
-            int slot = 0;
-            stage_set(grp);
-            for (long long s = grp; s < n_total; s += LOAD_GROUPS) {
-                TCP(c0 = clock64();)
-                prefetch_next();
-                TCP(t_issue += clock64() - c0;)
-                if (D == 2) asm volatile("cp.async.wait_group 1;" ::: "memory");
-                else asm volatile("cp.async.wait_group 2;" ::: "memory");
-                __syncwarp();
-                fill_stage(tb_u32 + (uint32_t)(slot * P.tb_bytes), lane);
-                __syncwarp();  // every lane has read its row before the slot is refilled
-                if (++slot == D) slot = 0;
-                stage_adv(LOAD_GROUPS);
-            }
+            __syncwarp();  // every lane has read its rows before the slot is refilled
+            stage_adv(k * (LOAD_GROUPS - 1));  // the other group's unit
+            slot ^= 1;
         }
         asm volatile("cp.async.wait_group 0;" ::: "memory");
 #ifdef MRB_TC_PROF
@@ -682,112 +258,67 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
             o[0] = clock64() - t_start; o[1] = t_wait; o[2] = t_st; o[3] = t_issue; o[13] = t_stw;
         }
 #endif
-    } else if (warp >= EPI_WARPS + LOAD_WARPS && warp < EPI_WARPS + LOAD_WARPS + MMA_WARPS) {
-        // ============================== MMA ISSUERS ==============================
-        // Issuer mi handles segments mi, mi + NI, ... of every tile.  All MMAs of one issuer go to its own accumulator
-        // group, so the two issue streams need no mutual ordering; the assignment does not depend on the tile index,
-        // so a pixel's result is bit-identical run to run and whatever the batch it is part of.
-        const int mi = warp - (EPI_WARPS + LOAD_WARPS);
-        if (mi < P.n_issuers) {  // whole warp, warp-uniform control flow (see umma_commit)
-            const int NI = P.n_issuers;
-            TCP(const bool prof = P.prof != nullptr;)
-            int stage = mi % P.stages;
-            uint32_t phase = (uint32_t)(mi / P.stages) & 1u;
-            int bs = mi % P.b_stages;
-            uint32_t bphase = (uint32_t)(mi / P.b_stages) & 1u;
-            TCP(long long t_start = clock64(), t_wfull = 0, t_wacc = 0, t_mma = 0, t_commit = 0, t_wb = 0, t_prep = 0, c0 = 0, c1 = 0;)
-            int buf = 0;
-            uint32_t acc_phase = 0;
-            const uint32_t tmem_u = uni(tmem_base);
-            const uint32_t w_u32 = smem_u32(w_s), bst_u32 = smem_u32(bst_s);
-            const uint32_t grp_off = (uint32_t)(mi * P.group_cols);
-            // loop-invariant operands of the stacked issue (segments of a conv all have N = nhalf, wchunk = segment index)
-            const uint64_t desc0 = make_desc(w_u32);
-            const uint32_t idesc_n = make_idesc(TILE_M, P.nhalf), idesc_2n = make_idesc(TILE_M, 2 * P.nhalf);
-            for (int tile = first_tile; tile < P.n_tiles; tile += tile_stride) {
+    } else if (warp == EPI_WARPS + LOAD_WARPS) {
+        // ============================== MMA ISSUER ==============================
+        // Segments are issued in order into one accumulator buffer per tile, so a position's result is bit-identical run
+        // to run and whatever the batch it is part of.  Whole warp, warp-uniform control flow (see umma_commit).
+        TCP(const bool prof = P.prof != nullptr;)
+        int stage = 0;
+        uint32_t phase = 0;
+        int bs = 0;
+        uint32_t bphase = 0;
+        TCP(long long t_start = clock64(), t_wfull = 0, t_wacc = 0, t_mma = 0, t_commit = 0, t_wb = 0, t_prep = 0, c0 = 0, c1 = 0;)
+        int buf = 0;
+        uint32_t acc_phase = 0;
+        const uint32_t tmem_u = uni(tmem_base);
+        const uint32_t bst_u32 = smem_u32(bst_s);
+        // loop-invariant operands: every segment has N = 64 and the same accumulator columns; only the weight slot moves
+        const uint64_t desc0 = make_desc(bst_u32);
+        constexpr uint32_t idesc_n = make_idesc(TILE_M, COUT), idesc_2n = make_idesc(TILE_M, 2 * COUT);
+        for (int tile = first_tile; tile < P.n_tiles; tile += tile_stride) {
+            TCP(if (prof) c0 = clock64();)
+            mbar_wait(&acc_empty[buf], acc_phase ^ 1);
+            TCP(if (prof) t_wacc += clock64() - c0;)
+            tc_fence_after();
+            const uint32_t d = tmem_u + (uint32_t)(buf * P.acc_cols);
+            for (int sgi = 0; sgi < P.nseg; ++sgi) {
+                TCP(if (prof) c1 = clock64();)
+                // every MMA operand is derived from kernel parameters and uniform loop state (no shared-memory table, no
+                // shuffles): it stays in uniform registers, and it is ready before the waits return
+                const uint64_t dbh = desc0 + (uint64_t)((bs * 2 * W_CHUNK_BYTES) >> 4);
+                const uint32_t a_hi = tmem_u + a_col0 + (uint32_t)(stage * A_STAGE_COLS);
                 TCP(if (prof) c0 = clock64();)
-                mbar_wait(&acc_empty[buf], acc_phase ^ 1);
-                TCP(if (prof) t_wacc += clock64() - c0;)
+                mbar_wait(&b_full[bs], bphase);
+                TCP(if (prof) t_wb += clock64() - c0;)
+                TCP(if (prof) c0 = clock64();)
+                mbar_wait(&full[stage], phase);
+                TCP(if (prof) t_wfull += clock64() - c0;)
                 tc_fence_after();
-                const uint32_t d_base = tmem_u + (uint32_t)(buf * P.acc_cols) + grp_off;
-                for (int sgi = mi; sgi < P.nseg; sgi += NI) {
-                    TCP(if (prof) c1 = clock64();)
-                    // every MMA operand is derived from kernel parameters and uniform loop state (no shared-memory
-                    // table, no shuffles): it stays in uniform registers, and it is ready before the waits return
-                    SegIssue si;
-                    uint32_t d = d_base;
-                    if (P.stacked) {
-                        // stacked convs: every segment has the same N and accumulator columns; only the weight chunk moves
-                        const uint32_t b_hi = P.stream_b ? bst_u32 + (uint32_t)(bs * 2 * wbytes_chunk)
-                                                         : w_u32 + (uint32_t)(sgi * 2 * wbytes_chunk);
-                        si.dbh = desc0 + (uint64_t)((b_hi - w_u32) >> 4);
-                        si.dbl = 0;
-                        si.idesc = idesc_n;
-                        si.idesc2n = idesc_2n;
-                        si.first = 0;
-                    } else {
-                        const Segment sg = P.seg[sgi];
-                        const uint32_t b_hi = P.stream_b ? bst_u32 + (uint32_t)(bs * 2 * wbytes_chunk)
-                                                         : w_u32 + (uint32_t)(sg.wchunk * 2 * wbytes_chunk);
-                        si.dbh = make_desc(b_hi);
-                        si.dbl = make_desc(b_hi + wbytes_chunk);
-                        si.idesc = make_idesc(TILE_M, sg.n);
-                        si.idesc2n = make_idesc(TILE_M, 2 * sg.n);
-                        si.first = (uint32_t)sg.first;
-                        d += (uint32_t)sg.dcol;
-                    }
-                    const uint32_t a_hi = tmem_u + a_col0 + (uint32_t)(stage * A_STAGE_COLS);
-                    if (P.stream_b) {
-                        TCP(if (prof) c0 = clock64();)
-                        mbar_wait(&b_full[bs], bphase);
-                        TCP(if (prof) t_wb += clock64() - c0;)
-                    }
-                    TCP(if (prof) c0 = clock64();)
-                    mbar_wait(&full[stage], phase);
-                    TCP(if (prof) t_wfull += clock64() - c0;)
-                    tc_fence_after();
-                    TCP(if (prof) { c0 = clock64(); t_prep += c0 - c1; })
-                    if (TC_DBG(P, 1)) {
-                    } else if (P.stacked) {
-                        // first segment of this issuer's accumulator group in this tile (sgi == mi): the N = 2n MMA of
-                        // k-step 0 overwrites [main | cross]; everything after it accumulates (MMAs of one thread
-                        // execute in order)
-                        umma_segment_ts_stacked(d, d + (uint32_t)P.small_off, a_hi, a_hi + KC, si.dbh, si.idesc2n, si.idesc,
-                                                sgi < NI ? 0u : 1u);
-                    } else if (si.first == 2) {
-                        // GRU x-part: r/z columns accumulate onto the h-part, the i_n columns start here
-                        umma_first_split(d, a_hi + KC, si.dbh, make_idesc(TILE_M, 2 * P.nhalf), make_idesc(TILE_M, P.nhalf),
-                                         (uint32_t)(2 * P.nhalf));
-                        umma_segment_ts(d, d, a_hi, a_hi + KC, si.dbh, si.dbl, si.idesc, 1u, 1u, 1u);
-                    } else {
-                        umma_segment_ts(d, d + (uint32_t)P.small_off, a_hi, a_hi + KC, si.dbh, si.dbl, si.idesc,
-                                        si.first ? 0u : 1u, 1u, 0u);
-                    }
-                    TCP(if (prof) { t_mma += clock64() - c0; c0 = clock64(); })
-                    umma_commit(&empty[stage]);  // stage reusable once these MMAs have read it
-                    // distance (in the global segment stream) to this issuer's next segment: NI inside the tile, else
-                    // to segment mi of the next tile
-                    const int delta = (sgi + NI < P.nseg) ? NI : (P.nseg - sgi + mi);
-                    if (P.stream_b) {
-                        umma_commit(&b_empty[bs]);
-                        bs += delta;
-                        while (bs >= P.b_stages) { bs -= P.b_stages; bphase ^= 1u; }
-                    }
-                    TCP(if (prof) t_commit += clock64() - c0;)
-                    stage += delta;
-                    while (stage >= P.stages) { stage -= P.stages; phase ^= 1u; }
+                TCP(if (prof) { c0 = clock64(); t_prep += c0 - c1; })
+                if (!TC_DBG(P, 1)) {
+                    // the N = 2n MMA of k-step 0 of the first segment overwrites [main | cross]; everything after it
+                    // accumulates (MMAs of one thread execute in order)
+                    umma_segment_ts_stacked(d, d + (uint32_t)COUT, a_hi, a_hi + KC, dbh, idesc_2n, idesc_n, sgi == 0 ? 0u : 1u);
                 }
-                umma_commit(&acc_full[buf]);
-                if (++buf == P.acc_bufs) { buf = 0; acc_phase ^= 1u; }
+                TCP(if (prof) { t_mma += clock64() - c0; c0 = clock64(); })
+                umma_commit(&empty[stage]);  // stage reusable once these MMAs have read it
+                umma_commit(&b_empty[bs]);
+                if (++bs == P.b_stages) { bs = 0; bphase ^= 1u; }
+                TCP(if (prof) t_commit += clock64() - c0;)
+                if (++stage == P.stages) { stage = 0; phase ^= 1u; }
             }
+            umma_commit(&acc_full[buf]);
+            if (++buf == P.acc_bufs) { buf = 0; acc_phase ^= 1u; }
+        }
 #ifdef MRB_TC_PROF
-            if (prof && mi == 0 && lane == 0) {
-                unsigned long long* o = P.prof + (size_t)blockIdx.x * 16;
-                o[4] = clock64() - t_start; o[5] = t_wfull; o[6] = t_wacc; o[7] = t_mma; o[10] = t_commit; o[11] = t_wb; o[12] = t_prep;
-            }
+        if (prof && lane == 0) {
+            unsigned long long* o = P.prof + (size_t)blockIdx.x * 16;
+            o[4] = clock64() - t_start; o[5] = t_wfull; o[6] = t_wacc; o[7] = t_mma; o[10] = t_commit; o[11] = t_wb; o[12] = t_prep;
+        }
 #endif
-        } else if (P.out_bh == 1 && mi == 1 && lane == 0) {
-            // ============================== TMA STORE LANE (out_bh; requires n_issuers == 1) ==============================
+    } else if (warp == EPI_WARPS + LOAD_WARPS + 1) {
+        // ============================== TMA STORE LANE ==============================
+        if (lane == 0) {
             const uint32_t out_u32 = smem_u32(out_s);
             uint32_t oph = 0;
             for (int tile = first_tile; tile < P.n_tiles; tile += tile_stride) {
@@ -802,16 +333,16 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
             asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");  // stores complete before the CTA exits
         }
     } else if (warp == EPI_WARPS + LOAD_WARPS + MMA_WARPS) {
-        // ============================== WEIGHT STREAMER (stream_b) ==============================
-        // one lane, one bulk copy (cp.async.bulk, 2*wbytes_chunk contiguous bytes: hi rows | lo rows) per segment
-        if (P.stream_b && lane == 0) {
+        // ============================== WEIGHT STREAMER ==============================
+        // one lane, one bulk copy (cp.async.bulk, 2*W_CHUNK_BYTES contiguous bytes: hi rows | lo rows) per segment
+        if (lane == 0) {
             int bs = 0;
             uint32_t bphase = 0;
-            const uint32_t bytes = (uint32_t)(2 * wbytes_chunk);
+            const uint32_t bytes = (uint32_t)(2 * W_CHUNK_BYTES);
             for (int it = 0; it < n_items; ++it) {
                 for (int sgi = 0; sgi < P.nseg; ++sgi) {
                     mbar_wait_sleep(&b_empty[bs], bphase ^ 1, 64);
-                    const uint8_t* gsrc = reinterpret_cast<const uint8_t*>(P.wpack) + (size_t)P.seg[sgi].wchunk * bytes;
+                    const uint8_t* gsrc = reinterpret_cast<const uint8_t*>(P.wpack) + (size_t)sgi * bytes;
                     const uint32_t bar = smem_u32(&b_full[bs]);
                     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
                     asm volatile(
@@ -826,135 +357,33 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
     } else {
         // ============================== EPILOGUE ==============================
         const int quad = warp & 3;             // TMEM lane quadrant this warp may access
-        const int chalf = warp >> 2;           // which half of this item's channels the warp handles
-        const int m = quad * 32 + lane;        // TMEM lane = pixel row of the tile
-        const int j_lo = chalf * (P.nhalf / 2), j_hi = j_lo + P.nhalf / 2;
-        int it = 0;
+        const int chalf = warp >> 2;           // which half of the channels the warp handles
+        const int m = quad * 32 + lane;        // TMEM lane = position row of the tile
+        const int j_lo = chalf * (COUT / 2);
         const uint32_t bias_u32 = smem_u32(bias_s);
         const uint32_t out_u32 = smem_u32(out_s);
         uint32_t oph = 0;
-        // out_bh: 8 consecutive channels (chunk c8 = channel / 8) of this thread's position -> hi / lo bf16 in the output tile
-        auto emit8 = [&](int c8, const float* v, long long pos, bool ok) {
+        // 8 consecutive channels (chunk c8 = channel / 8) of this thread's position -> hi / lo bf16 in the output tile
+        auto emit8 = [&](int c8, const float* v) {
             uint32_t hi[4], lo[4];
 #pragma unroll
             for (int i = 0; i < 4; ++i) split_bf16x2(v[2 * i], v[2 * i + 1], hi[i], lo[i]);
-            if (P.out_bh == 1) {  // output tile in the TMA box layout (stored by the TMA store lane)
-                sts128u(out_u32 + swz(m, c8), make_uint4(hi[0], hi[1], hi[2], hi[3]));
-                sts128u(out_u32 + OUT_BOX_BYTES + swz(m, c8), make_uint4(lo[0], lo[1], lo[2], lo[3]));
-            } else if (ok) {      // out_bh == 2: straight to global memory from the thread that owns the position
-                uint8_t* g = reinterpret_cast<uint8_t*>(P.out) + pos * BH_PX_BYTES + c8 * 16;
-                *reinterpret_cast<uint4*>(g) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                *reinterpret_cast<uint4*>(g + 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-            }
+            sts128u(out_u32 + swz(m, c8), make_uint4(hi[0], hi[1], hi[2], hi[3]));
+            sts128u(out_u32 + OUT_BOX_BYTES + swz(m, c8), make_uint4(lo[0], lo[1], lo[2], lo[3]));
         };
-        const uint32_t et0 = smem_u32(epi_s) + (uint32_t)(warp * 2 * EPI_TILE_BYTES);  // this warp's two exchange tiles
-        // h_prev of a tile (independent of the MMAs): asynchronous coalesced copy into an exchange tile, issued one tile
-        // ahead so that its latency never shows
-        // global side of the exchange: lane -> pixel (lane >> 2) + 8*k of the warp's 32, 16-byte piece lane & 3
-        const long long xoff = ((long long)(quad * 32 + (lane >> 2))) * P.cout + half * P.nhalf + j_lo + (lane & 3) * 4;
-        const uint32_t xs = (uint32_t)((lane >> 2) * EPI_ROW_BYTES + (lane & 3) * 16);
-        auto fetch_hprev = [&](int tile, uint32_t dst) {
-            const float* g = P.hprev + (long long)tile * TILE_M * P.cout + xoff;
-            if (tile < P.n_tiles && (long long)(tile + 1) * TILE_M <= P.P) {  // whole tile inside: no per-row predicate
-#pragma unroll
-                for (int k = 0; k < 4; ++k) cp_async16(dst + xs + (uint32_t)(8 * k * EPI_ROW_BYTES), g + 8 * k * P.cout, 16u, true);
-            } else {
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    const long long pp = (long long)tile * TILE_M + quad * 32 + (lane >> 2) + 8 * k;
-                    const bool ok = tile < P.n_tiles && pp < P.P;
-                    cp_async16(dst + xs + (uint32_t)(8 * k * EPI_ROW_BYTES), ok ? (const void*)(g + 8 * k * P.cout) : (const void*)P.out,
-                               ok ? 16u : 0u, true);
-                }
-            }
-            asm volatile("cp.async.commit_group;" ::: "memory");
-        };
-        if (GRU && !TC_DBG(P, 4)) fetch_hprev(first_tile, et0);
         TCP(long long e_start = clock64(), e_wait = 0;)
         int buf = 0;
         uint32_t acc_phase = 0;
-        for (int tile = first_tile; tile < P.n_tiles; tile += tile_stride, ++it) {
+        for (int tile = first_tile; tile < P.n_tiles; tile += tile_stride) {
             const uint32_t t0 = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(buf * P.acc_cols);
-            const long long p = (long long)tile * TILE_M + m;
-            const bool valid = p < P.P;
-            const int ch0 = half * P.nhalf;
             bool released = false;
-            const uint32_t et = et0 + (uint32_t)((it & 1) * EPI_TILE_BYTES);
-            if (GRU && !TC_DBG(P, 4)) {
-                fetch_hprev(tile + tile_stride, et0 + (uint32_t)(((it + 1) & 1) * EPI_TILE_BYTES));  // next tile, other buffer
-                asm volatile("cp.async.wait_group 1;" ::: "memory");                                 // this tile's has landed
-                __syncwarp();
-            }
             TCP(long long c0 = clock64();)
             mbar_wait_sleep(&acc_full[buf], acc_phase, 64);
             TCP(e_wait += clock64() - c0;)
             tc_fence_after();
-            if (TC_DBG(P, 4)) {
-            } else if (GRU) {
-                // nhalf == 32: this warp owns 16 channels (64 B) of its 32 pixels.  Thread = pixel is what TMEM dictates,
-                // but as a global access pattern it touches 32 different 128-byte lines per instruction (the L1 data
-                // pipe was the busiest unit of the kernel, 64 %).  h_prev and the new state therefore go through a
-                // per-warp exchange tile: global side = 4 lanes per pixel x 16 B (8 lines per instruction).
-                const int nh = P.nhalf;  // hidden channels of this half
-                const int Ch = P.cout;
-                float o[16];
-                {
-                    float ar[8], az[8], xn[8], hn[8];
-#pragma unroll
-                    for (int jb = 0; jb < 2; ++jb) {
-                        const int j = j_lo + 8 * jb;
-                        tmem_ld8x4(t0 + j, t0 + nh + j, t0 + 2 * nh + j, t0 + 3 * nh + j, hn, ar, az, xn);
-                        if (jb == 1) {  // both halves of this thread's accumulator columns are in registers
-                            tc_fence_before();
-                            __syncwarp();
-                            if (lane == 0) mbar_arrive(&acc_empty[buf]);
-                            released = true;
-                        }
-                        const float4 h0 = lds128(et + (uint32_t)(lane * EPI_ROW_BYTES + jb * 32));
-                        const float4 h1 = lds128(et + (uint32_t)(lane * EPI_ROW_BYTES + jb * 32 + 16));
-                        const float hp[8] = {h0.x, h0.y, h0.z, h0.w, h1.x, h1.y, h1.z, h1.w};
-#pragma unroll
-                        for (int q4 = 0; q4 < 8; q4 += 4) {
-                            const int c = ch0 + j + q4;  // multiple of 4: 128-bit reads of the bias table
-                            const float4 br4 = lds128(bias_u32 + 4u * (uint32_t)c);
-                            const float4 bz4 = lds128(bias_u32 + 4u * (uint32_t)(Ch + c));
-                            const float4 bn4 = lds128(bias_u32 + 4u * (uint32_t)(2 * Ch + c));
-                            const float br[4] = {br4.x, br4.y, br4.z, br4.w}, bz[4] = {bz4.x, bz4.y, bz4.z, bz4.w};
-                            const float bn[4] = {bn4.x, bn4.y, bn4.z, bn4.w};
-#pragma unroll
-                            for (int u = 0; u < 4; ++u) {
-                                const int q = q4 + u;
-                                // rnn_cells.py:121-125 (ih + hh of the r and z gates were summed by the tensor core)
-                                const float r = sigmoid_fused(ar[q], br[u]);
-                                const float z = sigmoid_fused(az[q], bz[u]);
-                                const float n = tanh_acc(fmaf(r, hn[q], xn[q] + bn[u]));
-                                o[jb * 8 + q] = fmaf(z, hp[q], n * (1.f - z));
-                            }
-                        }
-                    }
-                }
-                __syncwarp();  // every lane has read its h_prev row: the tile can take the results
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-                    sts128(et + (uint32_t)(lane * EPI_ROW_BYTES + i * 16), make_float4(o[4 * i], o[4 * i + 1], o[4 * i + 2], o[4 * i + 3]));
-                __syncwarp();
-                {
-                    float* g = P.out + (long long)tile * TILE_M * Ch + xoff;
-                    if ((long long)(tile + 1) * TILE_M <= P.P) {
-#pragma unroll
-                        for (int k = 0; k < 4; ++k)
-                            *reinterpret_cast<float4*>(g + 8 * k * Ch) = lds128(et + xs + (uint32_t)(8 * k * EPI_ROW_BYTES));
-                    } else {
-#pragma unroll
-                        for (int k = 0; k < 4; ++k)
-                            if ((long long)tile * TILE_M + quad * 32 + (lane >> 2) + 8 * k < P.P)
-                                *reinterpret_cast<float4*>(g + 8 * k * Ch) = lds128(et + xs + (uint32_t)(8 * k * EPI_ROW_BYTES));
-                    }
-                }
-                __syncwarp();  // stores have read the tile before the next h_prev block lands in it
-            } else if (P.out_bh && P.ngroups == 1 && P.nhalf == 64 && P.small_off == 64) {
-                // BH output, one accumulator group [main | cross]: all 32 channels of this thread with two batched loads,
-                // the buffer goes back to the MMA issuer before any arithmetic
+            if (!TC_DBG(P, 4)) {
+                // accumulator [main | cross]: all 32 channels of this thread with two batched loads, the buffer goes back
+                // to the MMA issuer before any arithmetic
                 float o[32];
 #pragma unroll
                 for (int jb = 0; jb < 2; ++jb) {
@@ -971,119 +400,18 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&acc_empty[buf]);
                 released = true;
-                const bool relu = P.mode == MODE_CONV_RELU;
-                if (P.out_bh == 1) mbar_wait_sleep(out_free, oph ^ 1, 32);  // the previous tile's stores have read the output tile
+                mbar_wait_sleep(out_free, oph ^ 1, 32);  // the previous tile's stores have read the output tile
 #pragma unroll
                 for (int jb = 0; jb < 4; ++jb) {
-                    const float4 b0 = lds128(bias_u32 + 4u * (uint32_t)(ch0 + j_lo + jb * 8));
-                    const float4 b1 = lds128(bias_u32 + 4u * (uint32_t)(ch0 + j_lo + jb * 8 + 4));
+                    const float4 b0 = lds128(bias_u32 + 4u * (uint32_t)(j_lo + jb * 8));
+                    const float4 b1 = lds128(bias_u32 + 4u * (uint32_t)(j_lo + jb * 8 + 4));
                     float v[8] = {o[jb * 8 + 0] + b0.x, o[jb * 8 + 1] + b0.y, o[jb * 8 + 2] + b0.z, o[jb * 8 + 3] + b0.w,
                                   o[jb * 8 + 4] + b1.x, o[jb * 8 + 5] + b1.y, o[jb * 8 + 6] + b1.z, o[jb * 8 + 7] + b1.w};
-                    if (relu) {
+                    if (P.relu) {
 #pragma unroll
                         for (int q = 0; q < 8; ++q) v[q] = fmaxf(v[q], 0.f);
                     }
-                    emit8((ch0 + j_lo) / 8 + jb, v, p, valid);
-                }
-            } else if (P.ngroups == 2 && P.nhalf == 64 && P.acc_bufs == 1) {
-                // single accumulator buffer (3x3 conv): sum the four accumulator regions into registers first and hand
-                // the buffer back to the MMA issuers BEFORE the bias / ReLU / global stores
-                float o[32];
-#pragma unroll
-                for (int jb = 0; jb < 4; ++jb) {
-                    const int j = j_lo + jb * 8;
-                    float a[8], a2[8], b1[8], b2[8];
-                    tmem_ld8x4(t0 + j, t0 + 64 + j, t0 + 128 + j, t0 + 192 + j, a, a2, b1, b2);
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) o[jb * 8 + q] = (a[q] + a2[q]) + (b1[q] + b2[q]);
-                }
-                tc_fence_before();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&acc_empty[buf]);
-                released = true;
-                if (P.out_bh) {
-                    const bool relu = P.mode == MODE_CONV_RELU;
-                    if (P.out_bh == 1) mbar_wait_sleep(out_free, oph ^ 1, 32);  // the previous tile's stores have read the output tile
-#pragma unroll
-                    for (int jb = 0; jb < 4; ++jb) {
-                        const float4 b0 = lds128(bias_u32 + 4u * (uint32_t)(ch0 + j_lo + jb * 8));
-                        const float4 b1 = lds128(bias_u32 + 4u * (uint32_t)(ch0 + j_lo + jb * 8 + 4));
-                        float v[8] = {o[jb * 8 + 0] + b0.x, o[jb * 8 + 1] + b0.y, o[jb * 8 + 2] + b0.z, o[jb * 8 + 3] + b0.w,
-                                      o[jb * 8 + 4] + b1.x, o[jb * 8 + 5] + b1.y, o[jb * 8 + 6] + b1.z, o[jb * 8 + 7] + b1.w};
-                        if (relu) {
-#pragma unroll
-                            for (int q = 0; q < 8; ++q) v[q] = fmaxf(v[q], 0.f);
-                        }
-                        emit8((ch0 + j_lo) / 8 + jb, v, p, valid);
-                    }
-                } else if (valid) {
-                    const bool relu = P.mode == MODE_CONV_RELU;
-                    float4* op = reinterpret_cast<float4*>(P.out + p * P.cout + ch0 + j_lo);
-#pragma unroll
-                    for (int jb = 0; jb < 8; ++jb) {
-                        const float4 bi = lds128(bias_u32 + 4u * (uint32_t)(ch0 + j_lo + jb * 4));
-                        float4 v = make_float4(o[jb * 4 + 0] + bi.x, o[jb * 4 + 1] + bi.y, o[jb * 4 + 2] + bi.z, o[jb * 4 + 3] + bi.w);
-                        if (P.add_scale) {  // IndRNN: + hh * h_prev (rnn_cells.py:391)
-                            const float4 hv = __ldg(reinterpret_cast<const float4*>(P.hprev + p * P.cout + ch0 + j_lo) + jb);
-                            const float4 sc = lds128(bias_u32 + 4u * (uint32_t)(128 + ch0 + j_lo + jb * 4));
-                            v = make_float4(v.x + sc.x * hv.x, v.y + sc.y * hv.y, v.z + sc.z * hv.z, v.w + sc.w * hv.w);
-                        }
-                        if (relu) v = make_float4(fmaxf(v.x, 0.f), fmaxf(v.y, 0.f), fmaxf(v.z, 0.f), fmaxf(v.w, 0.f));
-                        op[jb] = v;
-                    }
-                }
-            } else {
-                for (int j = j_lo; j < j_hi; j += 8) {
-                    float a[8], a2[8], b1[8], b2[8];
-                    if (P.ngroups == 2) {
-                        // [main g0 | cross g0 | main g1 | cross g1]: four loads, one wait
-                        tmem_ld8x4(t0 + j, t0 + P.small_off + j, t0 + 2 * P.nhalf + j, t0 + 2 * P.nhalf + P.small_off + j, a, a2, b1,
-                                   b2);
-#pragma unroll
-                        for (int q = 0; q < 8; ++q) a[q] = (a[q] + a2[q]) + (b1[q] + b2[q]);
-                    } else {
-                        tmem_ld8(t0 + j, a);
-                        if (P.small_off) {
-                            tmem_ld8(t0 + P.small_off + j, a2);
-#pragma unroll
-                            for (int q = 0; q < 8; ++q) a[q] += a2[q];
-                            for (int g = 1; g < P.ngroups; ++g) {
-                                tmem_ld8(t0 + g * 2 * P.nhalf + j, b1);
-                                tmem_ld8(t0 + g * 2 * P.nhalf + P.small_off + j, b2);
-#pragma unroll
-                                for (int q = 0; q < 8; ++q) a[q] += b1[q] + b2[q];
-                            }
-                        }
-                    }
-                    if (P.out_bh == 1 && j == j_lo) mbar_wait_sleep(out_free, oph ^ 1, 32);  // previous tile's stores have read out_s
-                    if (valid || P.out_bh) {
-                        float o[8];
-                        const float4 bi0 = lds128(bias_u32 + 4u * (uint32_t)(ch0 + j));
-                        const float4 bi1 = lds128(bias_u32 + 4u * (uint32_t)(ch0 + j + 4));
-                        const float bi[8] = {bi0.x, bi0.y, bi0.z, bi0.w, bi1.x, bi1.y, bi1.z, bi1.w};
-                        const bool relu = P.mode == MODE_CONV_RELU;
-                        float hs[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-                        if (P.add_scale) {  // IndRNN: + hh * h_prev (rnn_cells.py:391)
-                            const float4* hp4 = reinterpret_cast<const float4*>(P.hprev + p * P.cout + ch0 + j);
-                            const float4 h0 = __ldg(hp4), h1 = __ldg(hp4 + 1);
-                            const float4 s0 = lds128(bias_u32 + 4u * (uint32_t)(128 + ch0 + j));
-                            const float4 s1 = lds128(bias_u32 + 4u * (uint32_t)(128 + ch0 + j + 4));
-                            hs[0] = s0.x * h0.x; hs[1] = s0.y * h0.y; hs[2] = s0.z * h0.z; hs[3] = s0.w * h0.w;
-                            hs[4] = s1.x * h1.x; hs[5] = s1.y * h1.y; hs[6] = s1.z * h1.z; hs[7] = s1.w * h1.w;
-                        }
-#pragma unroll
-                        for (int q = 0; q < 8; ++q) {
-                            const float v = (a[q] + bi[q]) + hs[q];
-                            o[q] = relu ? fmaxf(v, 0.f) : v;
-                        }
-                        if (P.out_bh) {
-                            emit8((ch0 + j) / 8, o, p, valid);
-                        } else {
-                            float4* op = reinterpret_cast<float4*>(P.out + p * P.cout + ch0 + j);
-                            op[0] = make_float4(o[0], o[1], o[2], o[3]);
-                            op[1] = make_float4(o[4], o[5], o[6], o[7]);
-                        }
-                    }
+                    emit8(j_lo / 8 + jb, v);
                 }
             }
             if (!released) {
@@ -1091,14 +419,12 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&acc_empty[buf]);
             }
-            if (P.out_bh == 1) {
-                // the tile's [128 positions x (64 hi | 64 lo)] boxes are complete once all eight epilogue warps have
-                // arrived; the TMA store lane (second MMA warp) takes it from there
-                fence_proxy_async();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(out_ready);
-                oph ^= 1;
-            }
+            // the tile's [128 positions x (64 hi | 64 lo)] boxes are complete once all eight epilogue warps have
+            // arrived; the TMA store lane takes it from there
+            fence_proxy_async();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(out_ready);
+            oph ^= 1;
             if (++buf == P.acc_bufs) { buf = 0; acc_phase ^= 1u; }
         }
 #ifdef MRB_TC_PROF
@@ -1131,7 +457,7 @@ __global__ void pack_weights_kernel(PackDesc D, uint16_t* dst) {
             const int tap = ch;
             const int co = half * D.nhalf + r, ci = k;
             if (co < D.cout && ci < D.cin) v = D.w[((long long)co * D.cin + ci) * D.ksz * D.ksz + tap];
-        } else if (D.mode == 1) {
+        } else {
             // chunk 0: w_hh with rows [n ; r ; z] of this half (accumulator columns [0, 3*nhalf));
             // chunk 1: w_ih with rows [r ; z ; n] (columns [nhalf, 4*nhalf)): the r and z columns are shared
             const int Ch = D.cout;
@@ -1141,12 +467,6 @@ __global__ void pack_weights_kernel(PackDesc D, uint16_t* dst) {
             const int row = g * Ch + half * D.nhalf + j;
             const float* w = is_hh ? D.w2 : D.w;
             v = w[(long long)row * D.cin + k];
-        } else {
-            // im2col of a 5x5 window over 4 channels: K index = tap*4 + ci, chunk ch covers taps 16*ch .. 16*ch+15
-            const int kk = ch * KCH + k;
-            const int tap = kk >> 2, ci = kk & 3;
-            const int co = half * D.nhalf + r;
-            if (tap < 25 && co < D.cout) v = D.w[((long long)co * 4 + ci) * 25 + tap];
         }
         const uint16_t hi = bf16_rn_bits(v);
         const float hif = __uint_as_float((uint32_t)hi << 16);
@@ -1166,10 +486,8 @@ int pack_launch(const PackDesc& D, void* dst, cudaStream_t st) {
 }
 
 static size_t smem_needed(const Params& P) {
-    const size_t chunk2 = (size_t)2 * P.wchunk_rows * 128;
-    const size_t wres = P.stream_b ? (size_t)P.b_stages * chunk2 : (size_t)P.n_wchunks * chunk2;
-    return 1024 + (P.out_bh == 1 ? (size_t)2 * OUT_BOX_BYTES : 0) + wres + (size_t)LOAD_WARPS * P.tb_depth * P.tb_bytes + 256 +
-           2 * B_STAGES * 8 + BIAS_FLOATS * sizeof(float) + (P.mode == MODE_GRU ? (size_t)EPI_WARPS * 2 * EPI_TILE_BYTES : 0);
+    return 1024 + (size_t)2 * OUT_BOX_BYTES + (size_t)P.b_stages * 2 * W_CHUNK_BYTES +
+           (size_t)LOAD_WARPS * P.tb_depth * P.tb_bytes + 256 + 2 * B_STAGES * 8 + BIAS_FLOATS * sizeof(float);
 }
 
 #ifdef MRB_TC_PROF
@@ -1177,7 +495,7 @@ static int g_debug = 0;
 static unsigned long long* g_prof = nullptr;
 #endif
 
-static int launch(Params& P, cudaStream_t st) {
+static int launch(Params& P, void* out, cudaStream_t st) {
 #ifdef MRB_TC_PROF
     P.debug = g_debug;
     P.prof = g_prof;
@@ -1188,48 +506,30 @@ static int launch(Params& P, cudaStream_t st) {
     if (P.stages > MAX_STAGES) P.stages = MAX_STAGES;
     MRB_REQUIRE(P.stages >= 2, MRB_EUNSUPPORTED, "tensor-core conv: accumulator leaves no room for the TMEM A ring");
     MRB_REQUIRE(P.P < 2147483647LL, MRB_EUNSUPPORTED, "tensor-core conv: too many pixels");
-    MRB_REQUIRE(P.nseg >= P.n_issuers && P.nseg <= MAX_SEGS, MRB_EUNSUPPORTED, "tensor-core conv: bad segment count");
-    // two issuers share the rings safely only if a slot / stage is always revisited by the same issuer inside a tile
-    // (tiles are separated by the accumulator hand-shake): ring depths must be even
-    MRB_REQUIRE(P.im2col != 2 || P.nseg == LOAD_GROUPS, MRB_EUNSUPPORTED, "tensor-core conv: patch mode needs one K chunk per loader group");
-    MRB_REQUIRE(!(P.src_bh || P.out_bh) || P.pos_padded, MRB_EINVAL, "tensor-core conv: BH tensors need padded positions");
-    MRB_REQUIRE(!P.out_bh || (P.cout == 64 && P.n_split == 1), MRB_EUNSUPPORTED, "tensor-core conv: BH output needs 64 channels");
-    MRB_REQUIRE(P.out_bh != 1 || P.n_issuers == 1, MRB_EUNSUPPORTED,
-                "tensor-core conv: the TMA-store variant needs one MMA issuer (the second MMA warp stores)");
+    MRB_REQUIRE(P.nseg >= 1 && P.nseg <= MAX_SEGS, MRB_EUNSUPPORTED, "tensor-core conv: bad segment count");
     CUtensorMap tm_out;
     memset(&tm_out, 0, sizeof(tm_out));
-    if (P.out_bh == 1) {
-        int rc = tc2::make_bh_tmap(&tm_out, P.out, P.P, TILE_M);
-        if (rc) return rc;
-    }
-    // BH source in halo mode: 32 + 2*pad flat positions per unit (no two-piece layout)
-    const int halo_rows = (P.halo && P.src_bh) ? 32 + P.dil * (P.ksz - 1) : HALO_ROWS;
-    P.tb_half = (P.halo ? halo_rows : 32) * 128;
+    int rc = tc2::make_bh_tmap(&tm_out, out, P.P, TILE_M);
+    if (rc) return rc;
+    // 32 + 2*pad flat positions per unit
+    P.tb_half = (32 + P.dil * (P.ksz - 1)) * 128;
     P.tb_bytes = 2 * P.tb_half;
-    P.tb_depth = P.halo ? 2 : 3;  // halo mode: one staging tile feeds k segments, current + next is enough
-    if (P.b_stages == 0) P.b_stages = B_STAGES;
-    if (smem_needed(P) > max_smem) P.tb_depth = 2;
-    while (P.stream_b && P.b_stages > 2 && smem_needed(P) > max_smem) --P.b_stages;
-    if (P.n_issuers == 2) {  // see above: even ring depths for two issuers
-        if (P.stream_b && (P.b_stages & 1)) --P.b_stages;
-        if (P.stages & 1) --P.stages;
-    }
-    MRB_REQUIRE(smem_needed(P) <= max_smem, MRB_EUNSUPPORTED, "tensor-core conv: weights do not fit shared memory");
+    P.tb_depth = 2;  // one staging tile feeds k segments: current + next is enough
+    P.b_stages = B_STAGES;
+    while (P.b_stages > 2 && smem_needed(P) > max_smem) --P.b_stages;
+    MRB_REQUIRE(smem_needed(P) <= max_smem, MRB_EUNSUPPORTED, "tensor-core conv: staging does not fit shared memory");
     static bool attr_set = false;  // per-process, not per launch (the attribute calls are not free)
     if (!attr_set) {
-        MRB_CUDA(cudaFuncSetAttribute(tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_smem));
-        MRB_CUDA(cudaFuncSetAttribute(tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_smem));
+        MRB_CUDA(cudaFuncSetAttribute(tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_smem));
         attr_set = true;
     }
-    int sms = device_sm_count();
-    int grid = (sms / P.n_split) * P.n_split;  // groups of n_split CTAs share a pixel tile
-    if (grid > P.n_split * P.n_tiles) grid = P.n_split * P.n_tiles;
+    int grid = device_sm_count();
+    if (grid > P.n_tiles) grid = P.n_tiles;
     // Every launch asks for the full opt-in shared memory (one CTA per SM anyway): all tensor-core kernels of the time
     // step then run with the same shared-memory carve-out.  Alternating this kernel between a ~195 KB and a ~227 KB
     // configuration (two different carve-outs) produced sporadic "Warp Illegal Instruction" traps in the weight streamer
-    // and hangs on the B200 (reproduced with tools/stress_bh.py conv3+conv5; same-size sequences never failed).
-    if (P.mode == MODE_GRU) tc_kernel<true><<<grid, THREADS, max_smem, st>>>(tm_out, P);
-    else tc_kernel<false><<<grid, THREADS, max_smem, st>>>(tm_out, P);
+    // and hangs on the B200; same-size sequences never failed.
+    tc_kernel<<<grid, THREADS, max_smem, st>>>(tm_out, P);
     MRB_LAUNCHED();
     return MRB_OK;
 }
@@ -1245,12 +545,11 @@ extern "C" void mrb_tc_set_prof(void* buf) { tc::g_prof = (unsigned long long*)b
 #endif
 
 extern "C" size_t mrb_tc_packed_floats(int kind, int cout, int cin, int k) {
-    // kind 0: conv k x k (cin == 64); 1: GRU 1x1 (cout = hidden, cin = 64 for both inputs); 2: conv 5x5 x 4ch.
+    // kind 0: conv k x k (cin == 64); no other kind is packed here (0 is returned).
     // Size of the packed bf16 hi/lo image, in 4-byte units (one chunk = 2 x rows x 128 B = 2 * rows * 32 floats).
     (void)cin;
     if (kind == 0) return (size_t)(k * k) * 2 * cout * 32;
-    if (kind == 1) return (size_t)2 * 2 * 2 * (3 * cout / 2) * 32;
-    return (size_t)2 * 2 * cout * 32;
+    return 0;
 }
 
 extern "C" int mrb_tc_pack_conv(const void* w, void* dst, int cout, int cin, int k, void* stream) {
@@ -1263,196 +562,36 @@ extern "C" int mrb_tc_pack_conv(const void* w, void* dst, int cout, int cin, int
     return MRB_OK;
 }
 
-extern "C" int mrb_tc_pack_gru(const void* w_ih, const void* w_hh, void* dst, int ch, int cx, void* stream) {
-    MRB_REQUIRE(w_ih && w_hh && dst, MRB_EINVAL, "mrb_tc_pack_gru: null pointer");
-    MRB_REQUIRE(ch == 64 && cx == 64, MRB_EUNSUPPORTED, "mrb_tc_pack_gru: tensor-core GRU needs 64 input and hidden channels");
-    tc::PackDesc D{(const float*)w_ih, (const float*)w_hh, 1, ch, cx, 1, ch / 2, 3 * ch / 2, 2, 2};
-    tc::pack_weights_kernel<<<64, 256, 0, (cudaStream_t)stream>>>(D, (uint16_t*)dst);
-    MRB_LAUNCHED();
-    return MRB_OK;
-}
-
-extern "C" int mrb_tc_pack_conv5x5x4(const void* w, void* dst, int cout, void* stream) {
-    MRB_REQUIRE(w && dst, MRB_EINVAL, "mrb_tc_pack_conv5x5x4: null pointer");
-    MRB_REQUIRE((cout % 32) == 0 && cout >= 32 && cout <= 128, MRB_EUNSUPPORTED, "mrb_tc_pack_conv5x5x4: bad cout");
-    tc::PackDesc D{(const float*)w, nullptr, 2, cout, 4, 5, cout, cout, 2, 1};  // not split: N = cout per CTA
-    tc::pack_weights_kernel<<<64, 256, 0, (cudaStream_t)stream>>>(D, (uint16_t*)dst);
-    MRB_LAUNCHED();
-    return MRB_OK;
-}
-
-static int tc_common(tc::Params& P, int B, int H, int W, int pos_padded = 0) {
+// ConvNonlinear k x k (dilated, replicate padding), 64 -> 64 channels, bias + optional ReLU, on BH tensors (conv_tc2.cu):
+// x_bh with a valid replicate border (mrb_bh_fix_border), out_bh written at all (H+4)(W+4) positions (interior = the conv
+// output; its border is not a replicate copy).
+extern "C" int mrb_tc_conv_bh(const void* x_bh, const void* wpack, const void* bias, void* out_bh, int B, int H, int W, int cout,
+                              int k, int dil, int relu, void* stream) {
+    MRB_REQUIRE(x_bh && wpack && out_bh, MRB_EINVAL, "mrb_tc_conv_bh: null pointer");
+    MRB_REQUIRE(cout == 64, MRB_EUNSUPPORTED, "mrb_tc_conv_bh: 64 output channels only");
+    MRB_REQUIRE((k % 2) == 1 && k * k <= tc::MAX_SEGS && dil >= 1, MRB_EUNSUPPORTED, "mrb_tc_conv_bh: unsupported geometry");
+    MRB_REQUIRE(dil * (k - 1) / 2 <= tc::BH_PAD, MRB_EUNSUPPORTED, "mrb_tc_conv_bh: the receptive field exceeds the BH border");
     MRB_REQUIRE(B >= 1 && H >= 1 && W >= 1, MRB_EINVAL, "tensor-core conv: bad shape");
+    tc::Params P;
+    memset(&P, 0, sizeof(P));
     P.B = B; P.H = H; P.W = W;
-    P.pos_padded = pos_padded;
-    P.P = pos_padded ? (long long)B * (H + 2 * tc::BH_PAD) * (W + 2 * tc::BH_PAD) : (long long)B * H * W;
+    P.P = (long long)B * (H + 2 * tc::BH_PAD) * (W + 2 * tc::BH_PAD);
     long long nt = (P.P + tc::TILE_M - 1) / tc::TILE_M;
     MRB_REQUIRE(nt <= 2147483647LL, MRB_EUNSUPPORTED, "tensor-core conv: too many pixels");
     P.n_tiles = (int)nt;
-    return MRB_OK;
-}
-
-// ConvNonlinear k x k (dilated, replicate padding), 64 -> cout channels, NHWC, bias + optional ReLU.
-static int tc_conv_launch(const void* x, const void* wpack, const void* bias, const void* hprev, const void* add_scale,
-                          void* out, int B, int H, int W, int cout, int k, int dil, int relu, void* stream, int bh = 0);
-
-// The same ConvNonlinear on BH tensors (conv_tc2.cu): x_bh with a valid replicate border (mrb_bh_fix_border), out_bh
-// written at all (H+4)(W+4) positions (interior = the conv output; its border is not a replicate copy).
-extern "C" int mrb_tc_conv_bh(const void* x_bh, const void* wpack, const void* bias, void* out_bh, int B, int H, int W, int cout,
-                              int k, int dil, int relu, void* stream) {
-    MRB_REQUIRE(cout == 64, MRB_EUNSUPPORTED, "mrb_tc_conv_bh: 64 output channels only");
-    MRB_REQUIRE(dil * (k - 1) / 2 <= tc::BH_PAD, MRB_EUNSUPPORTED, "mrb_tc_conv_bh: the receptive field exceeds the BH border");
-    return tc_conv_launch(x_bh, wpack, bias, nullptr, nullptr, out_bh, B, H, W, cout, k, dil, relu, stream, 1);
-}
-
-extern "C" int mrb_tc_conv_nhwc(const void* x, const void* wpack, const void* bias, void* out, int B, int H, int W,
-                                int cout, int k, int dil, int relu, void* stream) {
-    return tc_conv_launch(x, wpack, bias, nullptr, nullptr, out, B, H, W, cout, k, dil, relu, stream);
-}
-
-// IndRNNCell with kernel size 1 (rnn_cells.py:264-391): ReLU(ih(x) + hh * h) = the 1x1 conv with the recurrent term in the
-// epilogue
-extern "C" int mrb_tc_indrnn_nhwc(const void* x, const void* h, const void* wpack, const void* b_ih, const void* hh,
-                                  void* h_out, int B, int H, int W, int ch, void* stream) {
-    MRB_REQUIRE(h && hh, MRB_EINVAL, "mrb_tc_indrnn_nhwc: null pointer");
-    MRB_REQUIRE(h != h_out, MRB_EINVAL, "mrb_tc_indrnn_nhwc: h_out must not alias h");
-    return tc_conv_launch(x, wpack, b_ih, h, hh, h_out, B, H, W, ch, 1, 1, 1, stream);
-}
-
-static int tc_conv_launch(const void* x, const void* wpack, const void* bias, const void* hprev, const void* add_scale,
-                          void* out, int B, int H, int W, int cout, int k, int dil, int relu, void* stream, int bh) {
-    MRB_REQUIRE(x && wpack && out, MRB_EINVAL, "mrb_tc_conv_nhwc: null pointer");
-    MRB_REQUIRE((cout % 32) == 0 && cout >= 32 && cout <= 128 && (k % 2) == 1 && k * k <= tc::MAX_SEGS && dil >= 1,
-                MRB_EUNSUPPORTED, "mrb_tc_conv_nhwc: unsupported geometry");
-    tc::Params P;
-    memset(&P, 0, sizeof(P));
-    int rc = tc_common(P, B, H, W, bh);
-    if (rc) return rc;
-    P.src_bh = bh; P.out_bh = bh;
-    P.src[0] = (const float*)x; P.cs[0] = 64; P.src[1] = nullptr; P.cs[1] = 0;
-    P.wpack = wpack; P.bias = (const float*)bias; P.out = (float*)out;
-    P.hprev = (const float*)hprev; P.add_scale = (const float*)add_scale;
-    // All output channels in one CTA (stacked MMAs of N = 2*cout and cout: half the MMA instructions of a channel
-    // split).  One segment per tap (64 input channels = one 128-byte bf16 row of B); the k*k weight chunks
-    // (2*cout*128 B each: hi rows | lo rows) are streamed from L2 through a small ring -- resident they would leave
-    // no room for the halo staging tiles.
-    P.n_split = 1;
-    P.stream_b = 1;
-    P.cout = cout; P.nhalf = cout;
-    P.wchunk_rows = cout; P.n_wchunks = k * k;
+    P.src = (const uint8_t*)x_bh;
+    P.wpack = wpack; P.bias = (const float*)bias;
+    // One segment per tap (64 input channels = one 128-byte bf16 row of B), stacked MMAs of N = 128 and 64 (half the MMA
+    // instructions of a channel split).  The k*k weight chunks (2*64*128 B each: hi rows | lo rows) are streamed from L2
+    // through a small ring -- resident they would leave no room for the halo staging tiles.
     P.nseg = k * k;
-    // two accumulator groups, one per MMA issuer (the global segment stream alternates between them): fixed
-    // accumulation order inside a group (bit-reproducible), half-length chains (see Params::ngroups); the epilogue
-    // adds the groups.  A 1x1 kernel has a single segment per tile: one issuer, one group, two accumulator buffers.
-    // Ring depths must be EVEN with two issuers: a slot whose consecutive fills belong to different issuers breaks the parity
-    // waits (the issuer that is ahead sees the parity of the previous phase as "complete" and consumes the slot one fill
-    // early -- sporadic traps / hangs on the B200 with a 3-slot ring; launch() enforces it).
-    // BH variant: ONE issuer, output through the TMA store lane.  Measured alternative (MRB_TC_BH_2ISSUERS=1): two issuers
-    // with a 4-slot ring and plain st.global from the epilogue (out_bh = 2) -- 443 vs 371 us at B=16: the thread-per-position
-    // stores (32 cache lines per instruction) compete with the loaders' cp.async for L1 wavefronts.
-    const bool two = P.nseg >= 2 && (!bh || getenv("MRB_TC_BH_2ISSUERS"));
-    P.n_issuers = two ? 2 : 1;
-    P.ngroups = P.n_issuers;
-    if (bh) P.out_bh = P.n_issuers == 2 ? 2 : 1;
-    P.group_cols = 2 * cout;
-    MRB_REQUIRE(P.ngroups * 2 * cout <= 512 - 2 * tc::A_STAGE_COLS, MRB_EUNSUPPORTED, "mrb_tc_conv_nhwc: accumulators exceed TMEM");
-    P.acc_cols = P.ngroups * 2 * cout;  // per group: hi*hi chain + cross-term chain
-    P.small_off = cout;
-    P.stacked = 1;
-    P.acc_bufs = (P.ngroups == 1 && 2 * P.acc_cols <= 512 - 2 * tc::A_STAGE_COLS) ? 2 : 1;
-    P.mode = relu ? tc::MODE_CONV_RELU : tc::MODE_CONV_NOACT;
-    const int pad = dil * (k - 1) / 2;
-    P.ksz = k; P.dil = dil;
-    // halo gathers need the two-piece staging layout to hold (4*pad extra rows) and a warp's 32 pixels on <= 2 image rows
-    P.halo = (4 * pad <= tc::HALO_ROWS - 32 && W >= 32 && !getenv("MRB_TC_NO_HALO")) ? 1 : 0;
-    if (bh) P.halo = 1;  // flat positions: always the halo loader (32 + 2*pad <= HALO_ROWS rows per unit)
-    for (int t = 0; t < k * k; ++t) {
-        tc::Segment& s = P.seg[t];
-        s.src = 0; s.dy = (short)((t / k) * dil - pad); s.dx = (short)((t % k) * dil - pad);
-        s.c0 = 0; s.wchunk = (short)t; s.dcol = 0;
-        s.n = (short)cout;
-        s.first = 0;  // stacked issue: derived from the segment index
-    }
-    return tc::launch(P, (cudaStream_t)stream);
-}
-
-static int tc_conv5_launch(const void* x, const void* wpack, const void* bias, void* out, int B, int H, int W, int cout, int relu,
-                           void* stream, int bh);
-// ConvNonlinear 5x5 over a 4-channel NHWC input (the RIM gradient), cout outputs, bias + ReLU.
-extern "C" int mrb_tc_conv5x5x4_nhwc(const void* x, const void* wpack, const void* bias, void* out, int B, int H, int W,
-                                     int cout, int relu, void* stream) {
-    return tc_conv5_launch(x, wpack, bias, out, B, H, W, cout, relu, stream, 0);
-}
-// The same with a BH output (conv_tc2.cu): x [B,H,W,4] fp32 as above, out_bh written at all (H+4)(W+4) positions
-extern "C" int mrb_tc_conv5x5x4_bh(const void* x, const void* wpack, const void* bias, void* out_bh, int B, int H, int W,
-                                   int cout, int relu, void* stream) {
-    MRB_REQUIRE(cout == 64 && W + 2 * tc::BH_PAD >= 32, MRB_EUNSUPPORTED, "mrb_tc_conv5x5x4_bh: needs 64 output channels and W >= 28");
-    return tc_conv5_launch(x, wpack, bias, out_bh, B, H, W, cout, relu, stream, 1);
-}
-static int tc_conv5_launch(const void* x, const void* wpack, const void* bias, void* out, int B, int H, int W, int cout, int relu,
-                           void* stream, int bh) {
-    MRB_REQUIRE(x && wpack && out, MRB_EINVAL, "mrb_tc_conv5x5x4_nhwc: null pointer");
-    MRB_REQUIRE((cout % 32) == 0 && cout >= 32 && cout <= 128, MRB_EUNSUPPORTED, "mrb_tc_conv5x5x4_nhwc: bad cout");
-    tc::Params P;
-    memset(&P, 0, sizeof(P));
-    int rc = tc_common(P, B, H, W, bh);
-    if (rc) return rc;
-    P.out_bh = bh;
-    P.src[0] = (const float*)x; P.cs[0] = 4;
-    P.wpack = wpack; P.bias = (const float*)bias; P.out = (float*)out;
-    P.n_split = 1;  // all output channels in one CTA: weights (2 chunks x 2 x cout x 128 B) stay resident
-    P.cout = cout; P.nhalf = cout;
-    P.wchunk_rows = cout; P.n_wchunks = 2;
-    P.ngroups = 1;
-    P.n_issuers = 1;
-    P.group_cols = 0;
+    // One accumulator group per buffer (hi*hi chain | cross-term chain, summed in the epilogue), two buffers.  Measured
+    // and removed: two MMA issuers on alternating segments with plain st.global from the epilogue -- 443 vs 371 us at
+    // B = 16: the thread-per-position stores (32 cache lines per instruction) compete with the loaders' cp.async for L1
+    // wavefronts.
     P.acc_cols = 2 * cout;
-    P.small_off = cout;
-    P.stacked = 1;
     P.acc_bufs = 2;
-    P.mode = relu ? tc::MODE_CONV_RELU : tc::MODE_CONV_NOACT;
-    P.im2col = (bh || (W >= 32 && !getenv("MRB_TC_NO_HALO"))) ? 2 : 1;  // 2: taps assembled from a shared-memory halo patch
-    P.nseg = 2;  // K = 25 taps x 4 channels = 100, padded to two 64-wide chunks
-    for (int c = 0; c < 2; ++c) {
-        tc::Segment& s = P.seg[c];
-        s.src = 0; s.dy = 0; s.dx = 0; s.c0 = (short)c; s.wchunk = (short)c; s.dcol = 0;
-        s.n = (short)cout;
-        s.first = 0;
-    }
-    return tc::launch(P, (cudaStream_t)stream);
-}
-
-// ConvGRUCell, kernel size 1, 64 input and 64 hidden channels, NHWC.
-extern "C" int mrb_tc_gru_nhwc(const void* x, const void* h, const void* wpack, const void* b_ih, void* h_out, int B,
-                               int H, int W, int ch, void* stream) {
-    MRB_REQUIRE(x && h && wpack && h_out, MRB_EINVAL, "mrb_tc_gru_nhwc: null pointer");
-    MRB_REQUIRE(h_out != h, MRB_EINVAL, "mrb_tc_gru_nhwc: h_out must not alias h");
-    MRB_REQUIRE(ch == 64, MRB_EUNSUPPORTED, "mrb_tc_gru_nhwc: 64 channels only");
-    tc::Params P;
-    memset(&P, 0, sizeof(P));
-    int rc = tc_common(P, B, H, W);
-    if (rc) return rc;
-    P.src[0] = (const float*)x; P.cs[0] = 64; P.src[1] = (const float*)h; P.cs[1] = 64;
-    P.wpack = wpack; P.bias = (const float*)b_ih; P.hprev = (const float*)h; P.out = (float*)h_out;
-    // Channel split (two CTAs per pixel tile, N = 96 MMAs), weights resident, two 128-column accumulator buffers.
-    P.n_split = 2;
-    P.cout = ch; P.nhalf = ch / 2;
-    P.wchunk_rows = 3 * ch / 2; P.n_wchunks = 2;
-    // accumulator columns (nh = ch/2): [0,nh) = hh_n, [nh,2nh) = r, [2nh,3nh) = z (hh + ih summed by the tensor core),
-    // [3nh,4nh) = ih_n.  h-part: N = 3nh at column 0; x-part: N = 3nh at column nh.  The h segment overwrites its
-    // columns, the x segment accumulates onto r/z and overwrites ih_n (Segment::first = 2).
-    P.ngroups = 1;
-    P.n_issuers = 1;
-    P.group_cols = 0;
-    P.acc_cols = 4 * (ch / 2);
-    P.acc_bufs = 2;
-    P.mode = tc::MODE_GRU;
-    P.nseg = 2;  // segment 0: h (64 channels), segment 1: x
-    for (int i = 0; i < 2; ++i) {
-        tc::Segment& s = P.seg[i];
-        s.src = (short)(i ? 0 : 1); s.dy = 0; s.dx = 0; s.c0 = 0; s.wchunk = (short)i;
-        s.dcol = (short)(i ? ch / 2 : 0); s.n = (short)(3 * ch / 2);
-        s.first = (short)(i == 0 ? 1 : 2);
-    }
-    return tc::launch(P, (cudaStream_t)stream);
+    P.relu = relu;
+    P.ksz = k; P.dil = dil;
+    return tc::launch(P, out_bh, (cudaStream_t)stream);
 }

@@ -49,17 +49,6 @@ constexpr int THREADS2 = (EPI_W + 3) * 32;  // + TMA load lane, MMA issuer, TMA 
 constexpr int NSLOT = 8;           // 16 KB boxes: h ring 4 (two tiles x (h_hi, h_lo)), x ring 2 (x_hi, x_lo), output tile 2
 constexpr int SLOT_BYTES = TILE * 128;
 constexpr int W_CHUNK = 192 * 128; // hi (or lo) rows of one weight chunk
-#ifndef MRB_GRU2_GROUPS
-#define MRB_GRU2_GROUPS 1
-#endif
-// ConvGRU epilogue groups: 1 = all 16 epilogue warps work on one tile at a time (16 channels per warp); 2 = two groups of 8
-// warps on ALTERNATE tiles (32 channels per warp in two passes), meant to overlap one group's SFU-bound gate math with the
-// other group's h_prev unpack / split / store phases.  Same arithmetic per output (bit-identical results, parity-green),
-// but MEASURED SLOWER (278 vs 245 us at B = 16, tools/ab_gru2.sh): a group holds its h boxes and its accumulator buffer
-// until the second pass has read them, half a tile period later than the one-group form, and that delay sits on the
-// TMA -> MMA -> epilogue chain of the tile after next.  Kept as a build-time experiment (-DMRB_GRU2_GROUPS=2).
-constexpr int GRU2_GROUPS = MRB_GRU2_GROUPS;
-constexpr int GRU2_GW = EPI_W / GRU2_GROUPS;  // warps per group = arrivals per tile on the epilogue-side barriers
 
 // ---- TMA ---------------------------------------------------------------------------------------------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -163,15 +152,15 @@ gru2_kernel(const __grid_constant__ CUtensorMap tm_h, const __grid_constant__ CU
     if (threadIdx.x == 0) {
         for (int i = 0; i < 4; ++i) {
             mbar_init(&hfull[i], 1);
-            mbar_init(&hempty[i], 1 + GRU2_GW);
+            mbar_init(&hempty[i], 1 + EPI_W);
         }
         for (int i = 0; i < 2; ++i) {
             mbar_init(&xfull[i], 1);
             mbar_init(&xempty[i], 1);
             mbar_init(&acc_full[i], 1);
-            mbar_init(&acc_empty[i], GRU2_GW);
+            mbar_init(&acc_empty[i], EPI_W);
         }
-        mbar_init(out_ready, GRU2_GW);
+        mbar_init(out_ready, EPI_W);
         mbar_init(&out_free[0], 1);
         mbar_init(&out_free[1], 1);
         fence_barrier_init();
@@ -325,133 +314,123 @@ gru2_kernel(const __grid_constant__ CUtensorMap tm_h, const __grid_constant__ CU
     } else {
         // ============================== EPILOGUE ==============================
         const int quad = warp & 3;   // TMEM lane quadrant
-        const int grp = GRU2_GROUPS == 2 ? (warp >> 3) : 0;               // tiles it = grp, grp + GROUPS, ...
-        const int cg_first = GRU2_GROUPS == 2 ? 2 * ((warp >> 2) & 1) : (warp >> 2);  // first 16-channel block of this warp
+        const int cg = warp >> 2;    // channels 16*cg .. 16*cg + 15
         const int m = quad * 32 + lane;  // tile row = TMEM lane of this thread
         const uint32_t bias_u32 = smem_u32(bias_s);
         const uint32_t ring_u32 = smem_u32(ring), out_u32 = smem_u32(out_s);
         T2P(long long t_e0 = clock64(), t_ew = 0, t_eld = 0, t_emath = 0, t_est = 0, c0;)
-        int it = grp;
-        for (int tile = blockIdx.x + grp * gridDim.x; tile < P.n_tiles; tile += GRU2_GROUPS * gridDim.x, it += GRU2_GROUPS) {
+        int it = 0;
+        for (int tile = blockIdx.x; tile < P.n_tiles; tile += gridDim.x, ++it) {
             const int p = it & 1, buf = it & 1;
             const uint32_t hph = (uint32_t)(it >> 1) & 1u, acc_ph = (uint32_t)(it >> 1) & 1u;
-#pragma unroll
-            for (int sub = 0; sub < GRU2_GROUPS; ++sub) {
-                const int cg = cg_first + sub;  // channels 16*cg .. 16*cg + 15
-                // this thread's two 16-byte chunks (8 channels each) of row m inside a [128 x 128 B] SWIZZLE_128B box
-                const uint32_t ch0 = swz(m, 2 * cg), ch1 = swz(m, 2 * cg + 1);
-                // ---- h_prev of this thread's row and channels from the landed h_hi / h_lo boxes, which are released on
-                // behalf of this warp after its last read.  (An arrival can never be counted for an earlier phase of the
-                // same box: the data this warp has just waited for was loaded after that earlier phase had completed.)
-                float hp[16];
-                {
-                    uint4 hh[2], hl[2];
-                    if (sub == 0) mbar_wait_sleep(&hfull[2 * p], hph, 32);
-                    hh[0] = lds128u(ring_u32 + (uint32_t)((2 * p) * SLOT_BYTES) + ch0);
-                    hh[1] = lds128u(ring_u32 + (uint32_t)((2 * p) * SLOT_BYTES) + ch1);
-                    if (sub == 0) mbar_wait_sleep(&hfull[2 * p + 1], hph, 32);
-                    hl[0] = lds128u(ring_u32 + (uint32_t)((2 * p + 1) * SLOT_BYTES) + ch0);
-                    hl[1] = lds128u(ring_u32 + (uint32_t)((2 * p + 1) * SLOT_BYTES) + ch1);
-                    if (sub == GRU2_GROUPS - 1) {
-                        fence_proxy_async();  // the loads complete before the TMA may refill the boxes (see ind2_kernel)
-                        __syncwarp();
-                        if (lane == 0) {
-                            mbar_arrive(&hempty[2 * p]);
-                            mbar_arrive(&hempty[2 * p + 1]);
-                        }
-                    }
-#pragma unroll
-                    for (int j = 0; j < 2; ++j) {
-                        const uint32_t hw[4] = {hh[j].x, hh[j].y, hh[j].z, hh[j].w}, lw[4] = {hl[j].x, hl[j].y, hl[j].z, hl[j].w};
-#pragma unroll
-                        for (int i = 0; i < 4; ++i)
-                            up2(add2(pk2(bf_lo(hw[i]), bf_hi(hw[i])), pk2(bf_lo(lw[i]), bf_hi(lw[i]))), hp[8 * j + 2 * i],
-                                hp[8 * j + 2 * i + 1]);
-                    }
+            // this thread's two 16-byte chunks (8 channels each) of row m inside a [128 x 128 B] SWIZZLE_128B box
+            const uint32_t ch0 = swz(m, 2 * cg), ch1 = swz(m, 2 * cg + 1);
+            // ---- h_prev of this thread's row and channels from the landed h_hi / h_lo boxes, which are released on
+            // behalf of this warp after its last read.  (An arrival can never be counted for an earlier phase of the
+            // same box: the data this warp has just waited for was loaded after that earlier phase had completed.)
+            float hp[16];
+            {
+                uint4 hh[2], hl[2];
+                mbar_wait_sleep(&hfull[2 * p], hph, 32);
+                hh[0] = lds128u(ring_u32 + (uint32_t)((2 * p) * SLOT_BYTES) + ch0);
+                hh[1] = lds128u(ring_u32 + (uint32_t)((2 * p) * SLOT_BYTES) + ch1);
+                mbar_wait_sleep(&hfull[2 * p + 1], hph, 32);
+                hl[0] = lds128u(ring_u32 + (uint32_t)((2 * p + 1) * SLOT_BYTES) + ch0);
+                hl[1] = lds128u(ring_u32 + (uint32_t)((2 * p + 1) * SLOT_BYTES) + ch1);
+                fence_proxy_async();  // the loads complete before the TMA may refill the boxes (see ind2_kernel)
+                __syncwarp();
+                if (lane == 0) {
+                    mbar_arrive(&hempty[2 * p]);
+                    mbar_arrive(&hempty[2 * p + 1]);
                 }
-                T2P(c0 = clock64();)
-                if (sub == 0) mbar_wait_sleep(&acc_full[buf], acc_ph, 64);
-                T2P(t_ew += clock64() - c0;)
-                tc_fence_after();
-                const uint32_t t0 = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(buf * 256 + cg * 16);
-                float o[16];
 #pragma unroll
-                for (int jb = 0; jb < 2; ++jb) {
-                    float hn[8], ar[8], az[8], xn[8];
-                    T2P(c0 = clock64();)
-                    tmem_ld8x4(t0 + jb * 8, t0 + 64 + jb * 8, t0 + 128 + jb * 8, t0 + 192 + jb * 8, hn, ar, az, xn);
-                    T2P(t_eld += clock64() - c0; c0 = clock64();)
-                    if (jb == 1 && sub == GRU2_GROUPS - 1) {  // all of this warp's accumulator columns are in registers
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) mbar_arrive(&acc_empty[buf]);
-                    }
-                    if (T2_DBG(P, 4)) {
-    #pragma unroll
-                        for (int q = 0; q < 8; ++q) o[jb * 8 + q] = hn[q] + ar[q] + az[q] + xn[q] + hp[jb * 8 + q];
-                    } else
-    #pragma unroll
-                    for (int q4 = 0; q4 < 8; q4 += 4) {
-                        const int c = cg * 16 + jb * 8 + q4;
-                        f32x2 br[2], bz[2], bn[2];
-                        lds128p(bias_u32 + 4u * (uint32_t)c, br[0], br[1]);
-                        lds128p(bias_u32 + 4u * (uint32_t)(64 + c), bz[0], bz[1]);
-                        lds128p(bias_u32 + 4u * (uint32_t)(128 + c), bn[0], bn[1]);
-                        const f32x2 one2 = pk2(1.f, 1.f), nl2 = pk2(-kLog2e, -kLog2e), tl2 = pk2(2.f * kLog2e, 2.f * kLog2e);
-                        const f32x2 m2 = pk2(-2.f, -2.f);
-    #pragma unroll
-                        for (int u = 0; u < 2; ++u) {
-                            const int q = q4 + 2 * u;
-                            // rnn_cells.py:121-125 (ih + hh of the r and z gates were summed by the tensor core) on PAIRS of
-                            // channels: the fp32x2 forms are the same IEEE operations in half the issue slots (22 -> 14
-                            // instructions per output; the 5 SFU operations stay -- Newton reciprocals on the FMA pipe
-                            // measured slower, DESIGN 4.3).  r = 1/(1+ea), z = 1/(1+eb) share ONE
-                            // reciprocal: 1/((1+ea)(1+eb)); the exponents are clamped so that the product stays finite (a
-                            // gate below 2^-60 is zero to fp32 in everything it multiplies)
-                            float a0, a1, b0, b1;
-                            up2(fma2(pk2(ar[q], ar[q + 1]), nl2, br[u]), a0, a1);
-                            up2(fma2(pk2(az[q], az[q + 1]), nl2, bz[u]), b0, b1);
-                            const f32x2 xa = pk2(ex2_approx(fminf(a0, 60.f)), ex2_approx(fminf(a1, 60.f)));
-                            const f32x2 ea = add2(one2, xa);
-                            const f32x2 eb = add2(one2, pk2(ex2_approx(fminf(b0, 60.f)), ex2_approx(fminf(b1, 60.f))));
-                            float p0, p1;
-                            up2(mul2(ea, eb), p0, p1);
-                            const f32x2 ip = pk2(rcp_approx(p0), rcp_approx(p1));
-                            const f32x2 r = mul2(eb, ip), z = mul2(ea, ip);
-                            // n = tanh(ih_n + b_n + r * hh_n) = 1 - 2 / (1 + 2^(2 log2(e) v))
-                            float v0, v1;
-                            up2(mul2(fma2(r, pk2(hn[q], hn[q + 1]), add2(pk2(xn[q], xn[q + 1]), bn[u])), tl2), v0, v1);
-                            float d0, d1;
-                            up2(add2(one2, pk2(ex2_approx(v0), ex2_approx(v1))), d0, d1);
-                            const f32x2 n = fma2(m2, pk2(rcp_approx(d0), rcp_approx(d1)), one2);
-                            // h' = z h + n (1 - z)
-                            up2(fma2(z, pk2(hp[jb * 8 + q], hp[jb * 8 + q + 1]), mul2(n, sub2p(one2, z))), o[jb * 8 + q],
-                                o[jb * 8 + q + 1]);
-                        }
-                    }
-                    T2P(t_emath += clock64() - c0;)
-                }
-                T2P(c0 = clock64();)
-                // ---- hi/lo split into the output tile (rows = positions, same box layout as the inputs) + TMA stores
-                uint32_t hi[8], lo[8];
+                for (int j = 0; j < 2; ++j) {
+                    const uint32_t hw[4] = {hh[j].x, hh[j].y, hh[j].z, hh[j].w}, lw[4] = {hl[j].x, hl[j].y, hl[j].z, hl[j].w};
 #pragma unroll
-                for (int i = 0; i < 8; ++i) split_bf16x2(o[2 * i], o[2 * i + 1], hi[i], lo[i]);
-                // the stores of the previous tile (with two groups: the other group's tile) have read the output tile.  The
-                // store lane signals tile j on out_free[j & 1]; a parity wait only tells neighbouring phases apart, and on
-                // that barrier the phase before the awaited one (tile it - 3) is known to be complete: this group waited
-                // for it before it wrote tile it - 2
-                if (sub == 0 && it >= 1) mbar_wait_sleep(&out_free[(it - 1) & 1], (uint32_t)((it - 1) >> 1) & 1u, 32);
-                sts128u(out_u32 + ch0, make_uint4(hi[0], hi[1], hi[2], hi[3]));
-                sts128u(out_u32 + ch1, make_uint4(hi[4], hi[5], hi[6], hi[7]));
-                sts128u(out_u32 + SLOT_BYTES + ch0, make_uint4(lo[0], lo[1], lo[2], lo[3]));
-                sts128u(out_u32 + SLOT_BYTES + ch1, make_uint4(lo[4], lo[5], lo[6], lo[7]));
-                if (sub == GRU2_GROUPS - 1) {
-                    fence_proxy_async();  // generic-proxy writes -> visible to the TMA (async proxy)
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(out_ready);
+                    for (int i = 0; i < 4; ++i)
+                        up2(add2(pk2(bf_lo(hw[i]), bf_hi(hw[i])), pk2(bf_lo(lw[i]), bf_hi(lw[i]))), hp[8 * j + 2 * i],
+                            hp[8 * j + 2 * i + 1]);
                 }
-                T2P(t_est += clock64() - c0;)
             }
+            T2P(c0 = clock64();)
+            mbar_wait_sleep(&acc_full[buf], acc_ph, 64);
+            T2P(t_ew += clock64() - c0;)
+            tc_fence_after();
+            const uint32_t t0 = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(buf * 256 + cg * 16);
+            float o[16];
+#pragma unroll
+            for (int jb = 0; jb < 2; ++jb) {
+                float hn[8], ar[8], az[8], xn[8];
+                T2P(c0 = clock64();)
+                tmem_ld8x4(t0 + jb * 8, t0 + 64 + jb * 8, t0 + 128 + jb * 8, t0 + 192 + jb * 8, hn, ar, az, xn);
+                T2P(t_eld += clock64() - c0; c0 = clock64();)
+                if (jb == 1) {  // all of this warp's accumulator columns are in registers
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(&acc_empty[buf]);
+                }
+                if (T2_DBG(P, 4)) {
+#pragma unroll
+                    for (int q = 0; q < 8; ++q) o[jb * 8 + q] = hn[q] + ar[q] + az[q] + xn[q] + hp[jb * 8 + q];
+                } else
+#pragma unroll
+                for (int q4 = 0; q4 < 8; q4 += 4) {
+                    const int c = cg * 16 + jb * 8 + q4;
+                    f32x2 br[2], bz[2], bn[2];
+                    lds128p(bias_u32 + 4u * (uint32_t)c, br[0], br[1]);
+                    lds128p(bias_u32 + 4u * (uint32_t)(64 + c), bz[0], bz[1]);
+                    lds128p(bias_u32 + 4u * (uint32_t)(128 + c), bn[0], bn[1]);
+                    const f32x2 one2 = pk2(1.f, 1.f), nl2 = pk2(-kLog2e, -kLog2e), tl2 = pk2(2.f * kLog2e, 2.f * kLog2e);
+                    const f32x2 m2 = pk2(-2.f, -2.f);
+#pragma unroll
+                    for (int u = 0; u < 2; ++u) {
+                        const int q = q4 + 2 * u;
+                        // rnn_cells.py:121-125 (ih + hh of the r and z gates were summed by the tensor core) on PAIRS of
+                        // channels: the fp32x2 forms are the same IEEE operations in half the issue slots (22 -> 14
+                        // instructions per output; the 5 SFU operations stay -- Newton reciprocals on the FMA pipe
+                        // measured slower, DESIGN 4.3).  r = 1/(1+ea), z = 1/(1+eb) share ONE
+                        // reciprocal: 1/((1+ea)(1+eb)); the exponents are clamped so that the product stays finite (a
+                        // gate below 2^-60 is zero to fp32 in everything it multiplies)
+                        float a0, a1, b0, b1;
+                        up2(fma2(pk2(ar[q], ar[q + 1]), nl2, br[u]), a0, a1);
+                        up2(fma2(pk2(az[q], az[q + 1]), nl2, bz[u]), b0, b1);
+                        const f32x2 xa = pk2(ex2_approx(fminf(a0, 60.f)), ex2_approx(fminf(a1, 60.f)));
+                        const f32x2 ea = add2(one2, xa);
+                        const f32x2 eb = add2(one2, pk2(ex2_approx(fminf(b0, 60.f)), ex2_approx(fminf(b1, 60.f))));
+                        float p0, p1;
+                        up2(mul2(ea, eb), p0, p1);
+                        const f32x2 ip = pk2(rcp_approx(p0), rcp_approx(p1));
+                        const f32x2 r = mul2(eb, ip), z = mul2(ea, ip);
+                        // n = tanh(ih_n + b_n + r * hh_n) = 1 - 2 / (1 + 2^(2 log2(e) v))
+                        float v0, v1;
+                        up2(mul2(fma2(r, pk2(hn[q], hn[q + 1]), add2(pk2(xn[q], xn[q + 1]), bn[u])), tl2), v0, v1);
+                        float d0, d1;
+                        up2(add2(one2, pk2(ex2_approx(v0), ex2_approx(v1))), d0, d1);
+                        const f32x2 n = fma2(m2, pk2(rcp_approx(d0), rcp_approx(d1)), one2);
+                        // h' = z h + n (1 - z)
+                        up2(fma2(z, pk2(hp[jb * 8 + q], hp[jb * 8 + q + 1]), mul2(n, sub2p(one2, z))), o[jb * 8 + q],
+                            o[jb * 8 + q + 1]);
+                    }
+                }
+                T2P(t_emath += clock64() - c0;)
+            }
+            T2P(c0 = clock64();)
+            // ---- hi/lo split into the output tile (rows = positions, same box layout as the inputs) + TMA stores
+            uint32_t hi[8], lo[8];
+#pragma unroll
+            for (int i = 0; i < 8; ++i) split_bf16x2(o[2 * i], o[2 * i + 1], hi[i], lo[i]);
+            // the stores of the previous tile have read the output tile.  The store lane signals tile j on
+            // out_free[j & 1]; a parity wait only tells neighbouring phases apart, and on that barrier the phase before the
+            // awaited one (tile it - 3) is known to be complete: this warp waited for it before it wrote tile it - 2
+            if (it >= 1) mbar_wait_sleep(&out_free[(it - 1) & 1], (uint32_t)((it - 1) >> 1) & 1u, 32);
+            sts128u(out_u32 + ch0, make_uint4(hi[0], hi[1], hi[2], hi[3]));
+            sts128u(out_u32 + ch1, make_uint4(hi[4], hi[5], hi[6], hi[7]));
+            sts128u(out_u32 + SLOT_BYTES + ch0, make_uint4(lo[0], lo[1], lo[2], lo[3]));
+            sts128u(out_u32 + SLOT_BYTES + ch1, make_uint4(lo[4], lo[5], lo[6], lo[7]));
+            fence_proxy_async();  // generic-proxy writes -> visible to the TMA (async proxy)
+            __syncwarp();
+            if (lane == 0) mbar_arrive(out_ready);
+            T2P(t_est += clock64() - c0;)
         }
         T2P(if (P.prof && threadIdx.x == 0) { unsigned long long* o = P.prof + blockIdx.x * 16; o[5] = clock64() - t_e0; o[6] = t_ew; o[7] = t_eld; o[8] = t_emath; o[9] = t_est; })
     }

@@ -733,239 +733,6 @@ __global__ void __launch_bounds__(THREADS, 2) row_dc320_kernel(const float2* __r
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// Third form of the W = 320 row kernel: one HALF-WARP per (row, coil), the 16-point leg of 320 = 16 x 20 across the
-// 16 lanes by shuffles.  Lane l holds x[16a + l], a < 20: a 20-point DFT in registers, the twiddle w320^(l p), then for
-// every p a 16-point decimation-in-frequency FFT ACROSS the lanes (4 butterfly stages of __shfl_xor), which leaves
-// X[p + 20 brev4(l)] in lane l; the residual is pointwise, and the inverse runs the mirror image (decimation in time from
-// bit-reversed order) back to the ownership of the loads, so conj(S) meets its sample in the same lane.  No transpose
-// through shared memory and no block-wide barrier inside the transform pair: the 8 warps of a CTA (= one image row,
-// up to 16 coils) run independently between the table set-up and the coil sum.
-// TMA staging: the S row block (C rows of 2560 B) and the packed hybrid k-space rows arrive by 1-D bulk copies on two
-// transaction barriers while the tables are built; conj(S) x result is written IN PLACE over the staged S row, which is
-// then the coil-sum buffer.
-constexpr int S_THREADS = 256;
-inline size_t smem_bytes_s() {
-    return (size_t)2 * MAXC * N * sizeof(float2) + (size_t)N * sizeof(float2) + 2 * (size_t)N1 * N2 * sizeof(float2) + 64;
-}
-__device__ __forceinline__ void mbar_wait0(unsigned bar) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "W_LOOP:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], 0;\n\t"
-        "@p bra W_DONE;\n\t"
-        "bra W_LOOP;\n\t"
-        "W_DONE:\n\t"
-        "}\n" ::"r"(bar)
-        : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned bytes, unsigned bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                     (unsigned)__cvta_generic_to_shared(dst)),
-                 "l"(src), "r"(bytes), "r"(bar)
-                 : "memory");
-}
-
-template <int OUT_MODE>
-__global__ void __launch_bounds__(S_THREADS, 2) row_dc320s_kernel(const float2* __restrict__ eta, const float2* __restrict__ S,
-                                                                  const float2* __restrict__ yh, float* __restrict__ out, int C,
-                                                                  int H, const float2* __restrict__ tw, int rw, float fscale,
-                                                                  float oscale, MaskDesc mask) {
-    extern __shared__ __align__(16) float2 smem[];
-    float2* s_buf = smem;                        // [MAXC][N] staged S rows; later conj(S) * result (the coil-sum buffer)
-    float2* yh_s = s_buf + MAXC * N;             // [MAXC][N] packed hybrid k-space rows (ns2 entries used per coil)
-    float2* eta_s = yh_s + MAXC * N;             // [N]
-    float2* twl_s = eta_s + N;                   // [p][l] w320^(l p)
-    float2* kinfo_s = twl_s + N1 * N2;           // [p][lane]: (mask value, packed slot as int bits) of k = p + 20 brev4(lane)
-    __shared__ __align__(8) unsigned long long bars[2];
-    __shared__ int scan_s[10];
-    const int tid = threadIdx.x;
-    const int h = blockIdx.x, b = blockIdx.y;
-    const int hw = tid >> 4, l = tid & 15;
-    const long long cstride = (long long)H * N;
-    const long long rowoff = ((long long)b * C * H + h) * N;
-    const unsigned s_bar = (unsigned)__cvta_generic_to_shared(&bars[0]), y_bar = (unsigned)__cvta_generic_to_shared(&bars[1]);
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(s_bar));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(y_bar), "r"(C));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(s_bar), "r"((unsigned)(C * N * 8)) : "memory");
-        for (int c = 0; c < C; ++c) bulk_g2s(s_buf + c * N, S + rowoff + (long long)c * cstride, N * 8, s_bar);
-    }
-    // ---- tables (two entries per thread: i = tid and tid + 256 < 320) ----
-    const float2* erow = eta + ((long long)b * H + h) * N;
-    // per-stage twiddles of the lane FFT: stage d (8, 4, 2): lanes with bit d set multiply by w_{2d}^(l mod d) = w320^((l mod d) 160/d)
-    float2 wst[3];
-#pragma unroll
-    for (int s3 = 0; s3 < 3; ++s3) {
-        const int d = 8 >> s3;
-        wst[s3] = (l & d) ? __ldg(&tw[(l & (d - 1)) * (160 / d)]) : make_float2(1.f, 0.f);
-    }
-    int ns;
-    {
-        const int lane = tid & 31, wid = tid >> 5;
-        float mk[2];
-        unsigned bal[2];
-#pragma unroll
-        for (int r = 0; r < 2; ++r) {
-            const int i = tid + 256 * r;
-            const bool in = i < N;
-            if (in) {
-                eta_s[i] = __ldg(&erow[i]);
-                const int pp = i >> 4, ll = i & 15;
-                int e = ll * pp;
-                e -= (e / N) * N;
-                twl_s[i] = __ldg(&tw[e]);
-            }
-            mk[r] = in ? mask_value(mask, b, 0, rot_add(i, rw, N)) : 0.f;
-            bal[r] = __ballot_sync(0xffffffffu, mk[r] != 0.f);
-            if (lane == 0 && (r == 0 || wid < 2)) scan_s[r * 8 + wid] = __popc(bal[r]);
-        }
-        __syncthreads();  // also publishes the barrier initialisation
-        int tot = 0;
-        int woff[2] = {0, 0};
-#pragma unroll
-        for (int w = 0; w < 10; ++w) {
-            const int cnt = scan_s[w];
-            woff[0] += w < wid ? cnt : 0;
-            woff[1] += w < 8 + wid ? cnt : 0;
-            tot += cnt;
-        }
-        ns = tot;
-#pragma unroll
-        for (int r = 0; r < 2; ++r) {
-            const int k = tid + 256 * r;
-            if (k < N) {
-                const int slot = mk[r] != 0.f ? woff[r] + __popc(bal[r] & ((1u << lane) - 1u)) : 0;
-                const int pp = k % N2, q = k / N2;
-                const int j = ((q & 1) << 3) | ((q & 2) << 1) | ((q & 4) >> 1) | ((q & 8) >> 3);
-                kinfo_s[pp * N1 + j] = make_float2(mk[r], __int_as_float(slot));
-            }
-        }
-    }
-    const int ns2 = max(2, (ns + 1) & ~1);
-    const int c = min(hw, C - 1);       // an idle half-warp (C < 16) shadows the last coil and discards its result
-    if (l == 0 && hw < C) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(y_bar), "r"((unsigned)(ns2 * 8)) : "memory");
-        bulk_g2s(yh_s + hw * N, yh + rowoff + (long long)hw * cstride, ns2 * 8, y_bar);
-    }
-    __syncthreads();  // tables complete
-    mbar_wait0(s_bar);
-    // ---- forward: x = S * eta, 20-point DFT over a, twiddle, 16-point DIF across the lanes ----
-    float2* srow = s_buf + c * N + l;
-    cx v[N2];
-#pragma unroll
-    for (int a = 0; a < N2; ++a) {
-        const float2 e = eta_s[N1 * a + l], s0 = srow[N1 * a];
-        v[a] = pk(e.x * s0.x - e.y * s0.y, e.x * s0.y + e.y * s0.x);  // rim_utils.py:47-48
-    }
-    dft20<false>(v);
-    float2 u[N2];
-    u[0] = upk(v[0]);
-#pragma unroll
-    for (int pp = 1; pp < N2; ++pp) {
-        const float2 w = twl_s[pp * N1 + l];
-        u[pp] = mulw<false>(upk(v[pp]), w.x, w.y);
-    }
-#pragma unroll
-    for (int s3 = 0; s3 < 4; ++s3) {
-        const int d = 8 >> s3;
-        const float sg = (l & d) ? -1.f : 1.f;
-#pragma unroll
-        for (int pp = 0; pp < N2; ++pp) {
-            const float px = __shfl_xor_sync(0xffffffffu, u[pp].x, d), py = __shfl_xor_sync(0xffffffffu, u[pp].y, d);
-            const float tx = fmaf(u[pp].x, sg, px), ty = fmaf(u[pp].y, sg, py);  // upper: mine + partner, lower: partner - mine
-            if (s3 < 3) u[pp] = make_float2(tx * wst[s3].x - ty * wst[s3].y, tx * wst[s3].y + ty * wst[s3].x);
-            else u[pp] = make_float2(tx, ty);
-        }
-    }
-    // ---- residual against the hybrid k-space row: lane l holds k = p + 20 brev4(l) (parity of k = parity of p) ----
-    mbar_wait0(y_bar);
-    {
-        const float2* yc = yh_s + c * N;
-#pragma unroll
-        for (int pp = 0; pp < N2; ++pp) {
-            const float2 ki = kinfo_s[pp * N1 + l];
-            const float2 yv = yc[__float_as_int(ki.y)];
-            const float m = ki.x;  // 0 on unsampled columns
-            if (pp & 1) {
-                const float ys = rw != 0 ? -1.f : 1.f;
-                u[pp] = make_float2(m * (u[pp].x * fscale - ys * yv.x), m * (u[pp].y * fscale - ys * yv.y));
-            } else {
-                u[pp] = make_float2(m * (u[pp].x * fscale - yv.x), m * (u[pp].y * fscale - yv.y));  // rim_utils.py:54
-            }
-        }
-    }
-    // ---- inverse: 16-point DIT across the lanes (from bit-reversed order), conjugate twiddle, inverse 20-point DFT ----
-#pragma unroll
-    for (int s3 = 3; s3 >= 0; --s3) {
-        const int d = 8 >> s3;
-        const float sg = (l & d) ? -1.f : 1.f;
-#pragma unroll
-        for (int pp = 0; pp < N2; ++pp) {
-            float2 t = u[pp];
-            if (s3 < 3) t = make_float2(t.x * wst[s3].x + t.y * wst[s3].y, t.y * wst[s3].x - t.x * wst[s3].y);  // * conj(w)
-            const float px = __shfl_xor_sync(0xffffffffu, t.x, d), py = __shfl_xor_sync(0xffffffffu, t.y, d);
-            u[pp] = make_float2(fmaf(t.x, sg, px), fmaf(t.y, sg, py));
-        }
-    }
-    v[0] = pk(u[0]);
-#pragma unroll
-    for (int pp = 1; pp < N2; ++pp) {
-        const float2 w = twl_s[pp * N1 + l];
-        v[pp] = pk(mulw<true>(u[pp], w.x, w.y));
-    }
-    dft20<true>(v);
-    if (hw < C) {
-#pragma unroll
-        for (int a = 0; a < N2; ++a) {
-            const float2 s0 = srow[N1 * a], x = upk(v[a]);
-            srow[N1 * a] = make_float2(x.x * s0.x + x.y * s0.y, x.y * s0.x - x.x * s0.y);  // x * conj(S), in place
-        }
-    }
-    __syncthreads();
-    // ---- coil sum in coil order (rim_utils.py:61-62) + outputs ----
-#pragma unroll
-    for (int r = 0; r < 2; ++r) {
-        const int d = tid + 256 * r;
-        if (d >= N) break;
-        float2 acc = make_float2(0.f, 0.f);
-        for (int cc = 0; cc < C; ++cc) {
-            const float2 q = s_buf[cc * N + d];
-            acc.x += q.x;
-            acc.y += q.y;
-        }
-        const float2 e = eta_s[d];
-        if (OUT_MODE == 3) {
-            const float gx = acc.x * oscale, gy = acc.y * oscale;
-            const uint32_t h01 = bf16x2_rn(e.x, e.y), h23 = bf16x2_rn(gx, gy);
-            const uint32_t l01 = bf16x2_rn(e.x - __uint_as_float(h01 << 16), e.y - __uint_as_float(h01 & 0xffff0000u));
-            const uint32_t l23 = bf16x2_rn(gx - __uint_as_float(h23 << 16), gy - __uint_as_float(h23 & 0xffff0000u));
-            const uint4 val = make_uint4(h01, h23, l01, l23);
-            constexpr int Wp = N + 4;
-            const int Hp = H + 4;
-            uint4* base = reinterpret_cast<uint4*>(out) + (2 * Wp + 2) + ((long long)b * Hp + h + 2) * Wp;
-            const int r0 = h == 0 ? -2 : 0, r1 = h == H - 1 ? 2 : 0;
-            for (int rr = r0; rr <= r1; ++rr) {
-                uint4* row = base + (long long)rr * Wp;
-                row[d + 2] = val;
-                if (d == 0) row[0] = row[1] = val;
-                if (d == N - 1) row[N + 2] = row[N + 3] = val;
-            }
-        } else if (OUT_MODE == 2) {
-            reinterpret_cast<float4*>(out)[((long long)b * H + h) * N + d] = make_float4(e.x, e.y, acc.x * oscale, acc.y * oscale);
-        } else {
-            const long long HW = (long long)H * N;
-            float* o = out + (long long)b * 4 * HW + (long long)h * N + d;
-            o[0] = e.x;
-            o[HW] = e.y;
-            o[2 * HW] = acc.x * oscale;
-            o[3 * HW] = acc.y * oscale;
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------------------------
 // 320-point forms of the VarNet-side operators (vn_block.py:51-87,109-119): the same register-resident 16 x 20 transform as
 // fft.cu's fft320_kernel (16 lines per CTA, one shared-memory transpose) with the surrounding arithmetic in its loads and
 // stores.  Centring is the pair of thread-constant signs of that kernel, so every tensor stays in STORAGE order:
@@ -1319,24 +1086,6 @@ extern "C" int mrb_dc_rim_grad_hybrid(const void* eta, const void* yh, const voi
     const size_t smem = g.smem_row + (size_t)W * sizeof(unsigned short);
     if (W == r320::N && C <= r320::MAXC && !getenv("MRIDC_B200_DC_STOCKHAM")) {
         // register-resident two-pass row transforms (both fastMRI geometries have 320 columns)
-        if (getenv("MRIDC_B200_DC_V3")) {
-            // half-warp-per-coil form (lane FFT by shuffles, TMA-staged S / yh rows): parity-green, but 2736 instructions per
-            // warp and 2 coil rows against the 1728 per 1.5 coil rows of the kernel below -- measured 150 vs 124 us at B = 16
-            // (tools/dc_ab.py), so it is kept as an experiment behind this switch
-            const size_t sm3 = r320::smem_bytes_s();
-#define MRB_ROW_DCS(MODE)                                                                                              \
-    do {                                                                                                               \
-        if ((rc = set_smem(r320::row_dc320s_kernel<MODE>))) return rc;                                                 \
-        r320::row_dc320s_kernel<MODE><<<dim3(H, B), r320::S_THREADS, sm3, st>>>(                                       \
-            (const float2*)eta, (const float2*)S, (const float2*)yh, (float*)out, C, H, g.pw.tw, rw, fs, os, m);       \
-    } while (0)
-            if (out_nhwc == 2) MRB_ROW_DCS(3);
-            else if (out_nhwc) MRB_ROW_DCS(2);
-            else MRB_ROW_DCS(1);
-#undef MRB_ROW_DCS
-            MRB_LAUNCHED();
-            return MRB_OK;
-        }
         const size_t sm = r320::smem_bytes(C);
         if (out_nhwc == 2) {
             if ((rc = set_smem(r320::row_dc320_kernel<3>))) return rc;

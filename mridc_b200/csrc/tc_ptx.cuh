@@ -103,62 +103,6 @@ __device__ __forceinline__ void umma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, u
         "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
-// One segment = 4 k-steps x (lo*hi, hi*lo -> ds ; hi*hi -> d), issued from a single asm block: the issuing thread is
-// latency-bound (one dependent scalar instruction every few cycles, ~45 cycles minimum between MMAs measured with
-// tools/tc_microbench.py), so nothing but the MMAs themselves may sit between them.
-// skip_first != 0: the first MMA (lo*hi of k-step 0) has been issued separately by umma_first_split().
-__device__ __forceinline__ void umma_segment_ts(uint32_t d, uint32_t ds, uint32_t a_hi, uint32_t a_lo, uint64_t dbh,
-                                                uint64_t dbl, uint32_t idesc, uint32_t acc_small0, uint32_t acc_big0,
-                                                uint32_t skip_first) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred ps, pb, pt, pe, pf;\n\t"
-        "elect.sync _|pe, 0xffffffff;\n\t"
-        "setp.eq.b32 pf, %9, 0;\n\t"
-        "and.pred pf, pf, pe;\n\t"
-        ".reg .b32 ah1, ah2, ah3, al1, al2, al3;\n\t"
-        ".reg .b64 bh1, bh2, bh3, bl1, bl2, bl3;\n\t"
-        "setp.ne.b32 ps, %7, 0;\n\t"
-        "setp.ne.b32 pb, %8, 0;\n\t"
-        "setp.eq.b32 pt, 0, 0;\n\t"
-        "add.u32 ah1, %2, 8;\n\t add.u32 ah2, %2, 16;\n\t add.u32 ah3, %2, 24;\n\t"
-        "add.u32 al1, %3, 8;\n\t add.u32 al2, %3, 16;\n\t add.u32 al3, %3, 24;\n\t"
-        "add.u64 bh1, %4, 2;\n\t add.u64 bh2, %4, 4;\n\t add.u64 bh3, %4, 6;\n\t"
-        "add.u64 bl1, %5, 2;\n\t add.u64 bl2, %5, 4;\n\t add.u64 bl3, %5, 6;\n\t"
-        "@pf tcgen05.mma.cta_group::1.kind::f16 [%1], [%3], %4, %6, ps;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], [%2], %5, %6, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], [%2], %4, %6, pb;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], [al1], bh1, %6, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], [ah1], bl1, %6, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], [ah1], bh1, %6, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], [al2], bh2, %6, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], [ah2], bl2, %6, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], [ah2], bh2, %6, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], [al3], bh3, %6, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], [ah3], bl3, %6, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], [ah3], bh3, %6, pt;\n\t"
-        "}\n" ::"r"(d),
-        "r"(ds), "r"(a_hi), "r"(a_lo), "l"(dbh), "l"(dbl), "r"(idesc), "r"(acc_small0), "r"(acc_big0), "r"(skip_first)
-        : "memory");
-}
-// First MMA of a segment whose accumulator columns are partly shared with an earlier segment (GRU x-part: the r and z
-// columns already hold the h-part, the n columns are fresh): rows [0, n_acc) of the B chunk accumulate, rows
-// [n_acc, n_acc + n_new) overwrite.  Replaces the epilogue's re-zeroing of the accumulators.
-__device__ __forceinline__ void umma_first_split(uint32_t ds, uint32_t a, uint64_t db, uint32_t idesc_acc, uint32_t idesc_new,
-                                                 uint32_t n_acc) {
-    const uint64_t db2 = db + (uint64_t)((n_acc * 128u) >> 4);  // n_acc is a multiple of 8: whole 1024-byte row groups
-    asm volatile(
-        "{\n\t"
-        ".reg .pred pe, pt, pz;\n\t"
-        "elect.sync _|pe, 0xffffffff;\n\t"
-        "setp.eq.b32 pt, 0, 0;\n\t"
-        "setp.ne.b32 pz, 0, 0;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], [%2], %3, %5, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], [%2], %4, %6, pz;\n\t"
-        "}\n" ::"r"(ds),
-        "r"(ds + n_acc), "r"(a), "l"(db), "l"(db2), "r"(idesc_acc), "r"(idesc_new)
-        : "memory");
-}
 // Stacked-B variant (2 MMAs per k-step instead of 3): the packed weight chunk holds the hi rows immediately followed
 // by the lo rows, so ONE descriptor with N = 2n multiplies a_hi by [b_hi ; b_lo] -> columns [d, d+n) = a_hi*b_hi and
 // [d+n, d+2n) = a_hi*b_lo; the second MMA adds a_lo*b_hi (N = n) onto the cross-term columns [d+n, d+2n).
@@ -190,10 +134,6 @@ __device__ __forceinline__ void umma_segment_ts_stacked(uint32_t d, uint32_t dsm
 // lane-0 broadcast: tells the compiler that a value is warp-uniform (see umma_commit)
 __device__ __forceinline__ uint32_t uni(uint32_t v) { return __shfl_sync(0xffffffffu, v, 0); }
 __device__ __forceinline__ uint64_t uni64(uint64_t v) { return ((uint64_t)uni((uint32_t)(v >> 32)) << 32) | uni((uint32_t)v); }
-struct SegIssue {  // per-segment operands of the MMA issuer
-    uint64_t dbh, dbl;
-    uint32_t idesc, first, idesc2n;
-};
 // registers -> TMEM: 16 consecutive columns of this thread's lane
 __device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t* v) {
     asm volatile(
@@ -204,19 +144,6 @@ __device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t* v) {
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
-// TMEM -> registers: 8 consecutive columns of this thread's lane.  The wait is part of the same asm statement so
-// that no consumer of v[] can be scheduled before the asynchronous load has landed.
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float* v) {
-    uint32_t r[8];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];\n\t"
-        "tcgen05.wait::ld.sync.aligned;"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-        : "r"(taddr)
-        : "memory");
-#pragma unroll
-    for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
 // four 8-column loads with a single wait (GRU epilogue: hh_n, r, z, ih_n blocks)
 __device__ __forceinline__ void tmem_ld8x4(uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, float* v0, float* v1, float* v2,
                                            float* v3) {
@@ -382,7 +309,7 @@ __device__ __forceinline__ void tma_store_2d(const void* m, uint32_t src, int c0
 struct PackDesc {
     const float* w;       // conv: [Cout][Cin][k][k]; GRU: w_ih [3Ch][Cx] then w_hh via w2
     const float* w2;
-    int mode;             // 0 conv taps (chunk = tap), 1 GRU (chunk 0 = hh, 1 = ih), 2 im2col 5x5x4 (chunk = 16 taps)
+    int mode;             // 0 conv taps (chunk = tap), 1 GRU (chunk 0 = hh, 1 = ih)
     int cout, cin, ksz;   // conv geometry
     int nhalf;            // output channels per split part
     int rows;             // rows per chunk

@@ -409,7 +409,7 @@ class RIMBlock(nn.Module):
 
         if self._tc_engine is None:
             self._tc_engine = RimTcEngine(self) if RimTcEngine.supported(self) else False
-        use_tc = bool(self._tc_engine) and RimTcEngine.supported(self) and _lib.require_cuda(eta, "eta") is not None
+        use_tc = bool(self._tc_engine) and self._tc_engine.covers(W) and _lib.require_cuda(eta, "eta") is not None
         if use_tc:
             # tensor-core (tcgen05, split-bf16) engine for the whole time loop
             etas, hx = self._tc_engine.run(eta, masked_kspace, sense, mcan, sigma, hx if hx_given else None, ws, yhyb,

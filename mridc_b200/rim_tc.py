@@ -2,13 +2,13 @@
 
 Used by ``RIMBlock.forward`` when the block has the geometry of the shipped CIRIM/RIM configs
 (projects/reconstruction/model_zoo/conf/base_{cirim,rim}_run.yaml, recurrent_layer GRU or IndRNN): two
-ConvNonlinear(ReLU) + ConvGRUCell / IndRNNCell (kernel 1) stages with 64 channels and a final 64->2 ConvNonlinear.  Anything else
-runs on the generic exact-fp32 CUDA-core kernels.  Both paths are CUDA; neither is a CPU fallback.
+ConvNonlinear(ReLU) + ConvGRUCell / IndRNNCell (kernel 1) stages with 64 channels and a final 64->2 ConvNonlinear, on images
+at least 28 pixels wide (``covers``).  Anything else runs on the generic exact-fp32 CUDA-core kernels.  Both paths are
+CUDA; neither is a CPU fallback.
 
-ConvGRU blocks run on the second-generation kernels: every activation of the time loop lives in the "BH" layout
-([B][H+4][W+4][64 hi bf16 | 64 lo bf16], see conv_tc2.cu) -- the hi/lo split is done once by the producing kernel's epilogue,
-the ConvGRU cell is fed by TMA, and the replicate padding of ConvNonlinear is the tensor's own border.  IndRNN blocks use the
-first-generation kernels on fp32 channels-last activations.
+Every activation of the time loop lives in the "BH" layout ([B][H+4][W+4][64 hi bf16 | 64 lo bf16], see conv_tc2.cu): the
+hi/lo split is done once by the producing kernel's epilogue, the ConvGRU / IndRNN cells are fed by TMA, and the replicate
+padding of ConvNonlinear is the tensor's own border.
 """
 import os
 
@@ -21,8 +21,6 @@ def _enabled():
     return os.environ.get("MRIDC_B200_DISABLE_TC", "0") != "1"
 
 
-_CONV5_G8 = os.environ.get("MRIDC_B200_CONV5_GEN1", "0") != "1"  # =1: first conv on the gen-1 loader-warp kernel (conv_tc.cu)
-_FINAL_TC = os.environ.get("MRIDC_B200_FINAL_FP32", "0") != "1"  # =1: exact-fp32 CUDA-core final conv (conv.cu)
 _ZERO_STATE = {}
 _YH_STATIC = {}      # (B, C, H, W, device) -> [static hybrid k-space buffer, version of the tensor last copied into it]
 _GRAPH_POOL = {}     # device -> CUDA-graph memory pool shared by all cascades (they replay one after the other)
@@ -69,30 +67,22 @@ class RimTcEngine:
             if i == 0:
                 if not (c.input_size == 4 and c.kernel_size == 5 and c.dilation == 1):
                     return False
-            else:
-                if c.input_size != 64 or c.kernel_size % 2 != 1 or c.kernel_size**2 > 25:
+            else:  # the receptive field of the second conv stays inside the 2-pixel BH border
+                if c.input_size != 64 or c.kernel_size % 2 != 1 or c.dilation * (c.kernel_size - 1) // 2 > 2:
                     return False
         f = block.final_layer[0]
         if not isinstance(f, ConvNonlinear) or f.features != 2 or f.input_size != 64 or f._act != _ops.ACT_NONE:
             return False
-        if f.kernel_size % 2 != 1 or f.kernel_size * f.dilation > 9:
-            return False
-        return True
+        return f.kernel_size == 3 and f.dilation == 1
 
-    # ---------------------------------------------------------------------------------------------
-    def use_bh(self, W) -> bool:
-        """BH-layout engine (ConvGRU and IndRNN cells): second conv with a receptive field inside the 2-pixel border, final
-        conv 3x3, and rows of at least 32 positions (W + 4 >= 32)."""
-        b = self.block
-        c1, f = b.layers[1].convs, b.final_layer[0]
-        return (os.environ.get("MRIDC_B200_TC_GEN1", "0") != "1" and W >= 28
-                and c1.dilation * (c1.kernel_size - 1) // 2 <= 2 and f.kernel_size == 3 and f.dilation == 1)
+    def covers(self, W) -> bool:
+        """The engine runs this block on images W pixels wide: rows of at least 32 positions (W + 4 >= 32), the tile width of
+        the BH kernels' loaders and TMA boxes."""
+        return self.supported(self.block) and W >= 28
 
     @staticmethod
     def _g8(lib, B, H, W, dev):
-        """Zero-initialised G8 buffer (conv_tc2.cu) for the bulk-copy-fed first conv, or None for the gen-1 kernel."""
-        if not _CONV5_G8:
-            return None
+        """Zero-initialised G8 buffer (conv_tc2.cu): the input of the bulk-copy-fed first conv."""
         return torch.zeros(lib.mrb_g8_bytes(B, H, W), dtype=torch.uint8, device=dev)
 
     def _params(self):
@@ -102,12 +92,12 @@ class RimTcEngine:
             ps += [st.convs.conv_layer.weight, st.rnn.ih.weight, st.rnn.hh if self._indrnn else st.rnn.hh.weight]
         return ps
 
-    def packs(self, bh=False):
-        """Packed (hi/lo split, UMMA-swizzled) weights, rebuilt only when a parameter changes."""
+    def packs(self):
+        """Packed (hi/lo split, UMMA-swizzled) weights, rebuilt only when a parameter changes: per layer (conv, cell), the
+        first conv has none (mrb_tc2_conv5x5x4 splits its fp32 weights itself)."""
         key = tuple((p.data_ptr(), p._version, str(p.device)) for p in self._params())
-        hit = self._packs.get(bh)
-        if hit is not None and hit[0] == key:
-            return hit[1]
+        if self._packs.get("key") == key:
+            return self._packs["packs"]
         lib = _lib.load()
         st = _lib.stream_ptr()
         b = self.block
@@ -116,39 +106,25 @@ class RimTcEngine:
         for i, stack in enumerate(b.layers):
             c, r = stack.convs, stack.rnn
             w = c.conv_layer.weight.detach().contiguous()
-            if i == 0:
-                pc = torch.empty(lib.mrb_tc_packed_floats(2, 64, 4, 5), dtype=torch.float32, device=dev)
-                _lib.check(lib.mrb_tc_pack_conv5x5x4(_lib.ptr(w), _lib.ptr(pc), 64, st))
-            else:
+            pc = None
+            if i == 1:
                 pc = torch.empty(lib.mrb_tc_packed_floats(0, 64, 64, c.kernel_size), dtype=torch.float32, device=dev)
                 _lib.check(lib.mrb_tc_pack_conv(_lib.ptr(w), _lib.ptr(pc), 64, 64, c.kernel_size, st))
             wih = r.ih.weight.detach().contiguous()
             if self._indrnn:  # the 1x1 ih conv; the per-channel recurrent weight goes to the kernel's epilogue
                 pg = torch.empty(lib.mrb_tc_packed_floats(0, 64, 64, 1), dtype=torch.float32, device=dev)
                 _lib.check(lib.mrb_tc_pack_conv(_lib.ptr(wih), _lib.ptr(pg), 64, 64, 1, st))
-            elif bh:  # all 192 gate rows in one CTA (conv_tc2.cu)
+            else:  # all 192 gate rows in one CTA (conv_tc2.cu)
                 pg = torch.empty(lib.mrb_tc2_gru_packed_bytes(), dtype=torch.uint8, device=dev)
                 whh = r.hh.weight.detach().contiguous()
                 _lib.check(lib.mrb_tc2_pack_gru(_lib.ptr(wih), _lib.ptr(whh), _lib.ptr(pg), 64, 64, st))
-            else:
-                pg = torch.empty(lib.mrb_tc_packed_floats(1, 64, 64, 1), dtype=torch.float32, device=dev)
-                whh = r.hh.weight.detach().contiguous()
-                _lib.check(lib.mrb_tc_pack_gru(_lib.ptr(wih), _lib.ptr(whh), _lib.ptr(pg), 64, 64, st))
             out.append((pc, pg))
-        self._packs[bh] = (key, out)
+        self._packs.update(key=key, packs=out)
         return out
 
-    def _cell(self, lib, x, h, pack, rnn, h_out, B, H, W, st):
-        """ConvGRUCell (rnn_cells.py:93-127) or IndRNNCell (:367-391) with kernel size 1 on channels-last buffers."""
-        if self._indrnn:
-            _lib.check(lib.mrb_tc_indrnn_nhwc(_lib.ptr(x), _lib.ptr(h), _lib.ptr(pack), _lib.ptr(rnn.ih.bias),
-                                              _lib.ptr(rnn.hh.detach().reshape(-1)), _lib.ptr(h_out), B, H, W, 64, st))
-        else:
-            _lib.check(lib.mrb_tc_gru_nhwc(_lib.ptr(x), _lib.ptr(h), _lib.ptr(pack), _lib.ptr(rnn.ih.bias),
-                                           _lib.ptr(h_out), B, H, W, 64, st))
-
     def _cell_bh(self, lib, x, h, pack, rnn, h_out, B, H, W, st):
-        """The same cells on BH buffers (conv_tc2.cu: gru2_kernel / ind2_kernel)."""
+        """ConvGRUCell (rnn_cells.py:93-127) or IndRNNCell (:367-391) with kernel size 1 on BH buffers (conv_tc2.cu:
+        gru2_kernel / ind2_kernel)."""
         if self._indrnn:
             _lib.check(lib.mrb_tc2_indrnn(_lib.ptr(x), _lib.ptr(h), _lib.ptr(pack), _lib.ptr(rnn.ih.bias),
                                           _lib.ptr(rnn.hh.detach().reshape(-1)), _lib.ptr(h_out), B, H, W, st))
@@ -157,33 +133,7 @@ class RimTcEngine:
                                        B, H, W, st))
 
     # ---------------------------------------------------------------------------------------------
-    def conv_stack(self, g4, h, h_alt, xbuf, eta, packs=None):
-        """One time step of the regulariser (rim_block.py:233-248) on channels-last buffers: conv5x5 -> GRU ->
-        conv3x3(dil) -> GRU -> final conv + eta update.  h / h_alt are ping-pong lists, swapped in place."""
-        lib = _lib.load()
-        st = _lib.stream_ptr()
-        b = self.block
-        packs = self.packs() if packs is None else packs
-        B, H, W, _ = g4.shape
-        c0, c1 = b.layers[0].convs, b.layers[1].convs
-        r0, r1 = b.layers[0].rnn, b.layers[1].rnn
-        fin = b.final_layer[0]
-        _lib.check(lib.mrb_tc_conv5x5x4_nhwc(_lib.ptr(g4), _lib.ptr(packs[0][0]), _lib.ptr(c0.conv_layer.bias),
-                                             _lib.ptr(xbuf), B, H, W, 64, 1, st))
-        self._cell(lib, xbuf, h[0], packs[0][1], r0, h_alt[0], B, H, W, st)
-        h[0], h_alt[0] = h_alt[0], h[0]
-        _lib.check(lib.mrb_tc_conv_nhwc(_lib.ptr(h[0]), _lib.ptr(packs[1][0]), _lib.ptr(c1.conv_layer.bias),
-                                        _lib.ptr(xbuf), B, H, W, 64, c1.kernel_size, c1.dilation, 1, st))
-        self._cell(lib, xbuf, h[1], packs[1][1], r1, h_alt[1], B, H, W, st)
-        h[1], h_alt[1] = h_alt[1], h[1]
-        new_eta = torch.empty_like(eta)
-        _lib.check(lib.mrb_conv_c2_nhwc_residual(_lib.ptr(h[1]), _lib.ptr(fin.conv_layer.weight),
-                                                 _lib.ptr(fin.conv_layer.bias), _lib.ptr(eta), _lib.ptr(new_eta),
-                                                 B, H, W, 64, fin.kernel_size, fin.dilation, st))
-        return new_eta
-
-    # ---------------------------------------------------------------------------------------------
-    def conv_stack_bh(self, g4, h, h_alt, xbuf, eta, packs, B, H, W, g8=None):
+    def conv_stack_bh(self, g4, h, h_alt, xbuf, eta, packs, B, H, W, g8):
         """One time step of the regulariser (rim_block.py:233-248) on BH buffers (conv_tc2.cu): conv5x5 -> ConvGRU -> border
         -> conv3x3(dil) -> ConvGRU -> final conv (tap GEMM) + eta update.  h / h_alt are ping-pong lists, swapped in place."""
         lib = _lib.load()
@@ -192,15 +142,11 @@ class RimTcEngine:
         c0, c1 = b.layers[0].convs, b.layers[1].convs
         r0, r1 = b.layers[0].rnn, b.layers[1].rnn
         fin = b.final_layer[0]
-        if g8 is not None:
-            # bulk-copy-fed 5x5: the fp32 gradient is split once into the 16-byte G8 positions, taps are address offsets
-            if g4 is not None:  # else: the DC kernel has written g8 itself
-                _lib.check(lib.mrb_g8_from_nhwc4(_lib.ptr(g4), _lib.ptr(g8), B, H, W, st))
-            _lib.check(lib.mrb_tc2_conv5x5x4(_lib.ptr(g8), _lib.ptr(c0.conv_layer.weight), _lib.ptr(c0.conv_layer.bias),
-                                             _lib.ptr(xbuf), B, H, W, 1, st))
-        else:
-            _lib.check(lib.mrb_tc_conv5x5x4_bh(_lib.ptr(g4), _lib.ptr(packs[0][0]), _lib.ptr(c0.conv_layer.bias),
-                                               _lib.ptr(xbuf), B, H, W, 64, 1, st))
+        # bulk-copy-fed 5x5: the fp32 gradient is split once into the 16-byte G8 positions, taps are address offsets
+        if g4 is not None:  # else: the DC kernel has written g8 itself
+            _lib.check(lib.mrb_g8_from_nhwc4(_lib.ptr(g4), _lib.ptr(g8), B, H, W, st))
+        _lib.check(lib.mrb_tc2_conv5x5x4(_lib.ptr(g8), _lib.ptr(c0.conv_layer.weight), _lib.ptr(c0.conv_layer.bias),
+                                         _lib.ptr(xbuf), B, H, W, 1, st))
         self._cell_bh(lib, xbuf, h[0], packs[0][1], r0, h_alt[0], B, H, W, st)
         h[0], h_alt[0] = h_alt[0], h[0]
         _lib.check(lib.mrb_bh_fix_border(_lib.ptr(h[0]), B, H, W, st))  # the dilated 3x3 reads it spatially
@@ -209,7 +155,7 @@ class RimTcEngine:
         self._cell_bh(lib, xbuf, h[1], packs[1][1], r1, h_alt[1], B, H, W, st)
         h[1], h_alt[1] = h_alt[1], h[1]
         new_eta = torch.empty_like(eta)
-        if _FINAL_TC and B * (H + 4) >= 16:  # the 3-D TMA box of the tap GEMM spans 16 rows of the [B (H+4)] x (W+4) grid
+        if B * (H + 4) >= 16:  # the 3-D TMA box of the tap GEMM spans 16 rows of the [B (H+4)] x (W+4) grid
             # tap GEMM on the tensor core + clamped gather: reads the interior of h[1] only, no border fix-up
             _lib.check(lib.mrb_tc2_final_conv(_lib.ptr(h[1]), _lib.ptr(fin.conv_layer.weight), _lib.ptr(fin.conv_layer.bias),
                                               _lib.ptr(eta), _lib.ptr(new_eta), B, H, W, st))
@@ -220,35 +166,30 @@ class RimTcEngine:
         return new_eta
 
     def bench_step(self, B, H, W, dev):
-        """-> (callable running the conv stack of ONE time step on random buffers in this engine's layout, description)."""
+        """-> (callable running the conv stack of ONE time step on random BH buffers, description)."""
+        if not self.covers(W):
+            raise ValueError("RimTcEngine.bench_step: the engine does not cover W = %d" % W)
         g4 = torch.randn((B, H, W, 4), device=dev)
         eta = torch.randn((B, H, W, 2), device=dev)
-        if self.use_bh(W):
-            lib = _lib.load()
-            nb = lib.mrb_bh_bytes(B, H, W)
-            h, h_alt = [], [torch.empty(nb, dtype=torch.uint8, device=dev) for _ in range(2)]
-            for _ in range(2):
-                t = torch.randn((B, H, W, 64), device=dev) * 0.1
-                buf = torch.empty(nb, dtype=torch.uint8, device=dev)
-                _lib.check(lib.mrb_bh_from_nhwc(_lib.ptr(t), _lib.ptr(buf), B, H, W, _lib.stream_ptr()))
-                h.append(buf)
-            xbuf = torch.empty(nb, dtype=torch.uint8, device=dev)
-            packs = self.packs(bh=True)
-            g8 = self._g8(lib, B, H, W, dev)
-            if g8 is not None and W == 320:
-                # production feed at the fastMRI width: the DC kernel writes the G8 conv input itself, so the step starts
-                # from a filled G8 buffer (no converter launch)
-                _lib.check(lib.mrb_g8_from_nhwc4(_lib.ptr(g4), _lib.ptr(g8), B, H, W, _lib.stream_ptr()))
-                g4 = None
-            return (lambda: self.conv_stack_bh(g4, h, h_alt, xbuf, eta, packs, B, H, W, g8),
-                    "split-bf16 tcgen05 ConvGRU stack of one time step on BH activations (bulk-copy-fed conv5x5x4, TMA-fed "
-                    "ConvGRU, border, conv3x3d2, TMA-fed ConvGRU, tap-GEMM conv3x3->2 + eta)")
-        h = [torch.randn((B, H, W, 64), device=dev) * 0.1 for _ in range(2)]
-        h_alt = [torch.empty_like(t) for t in h]
-        xbuf = torch.empty((B, H, W, 64), device=dev)
-        return (lambda: self.conv_stack(g4, h, h_alt, xbuf, eta),
-                "split-bf16 tcgen05 stack of one time step on fp32 channels-last activations (conv5x5x4, cell 1x1, conv3x3d2, "
-                "cell 1x1, conv3x3->2 + eta)")
+        lib = _lib.load()
+        nb = lib.mrb_bh_bytes(B, H, W)
+        h, h_alt = [], [torch.empty(nb, dtype=torch.uint8, device=dev) for _ in range(2)]
+        for _ in range(2):
+            t = torch.randn((B, H, W, 64), device=dev) * 0.1
+            buf = torch.empty(nb, dtype=torch.uint8, device=dev)
+            _lib.check(lib.mrb_bh_from_nhwc(_lib.ptr(t), _lib.ptr(buf), B, H, W, _lib.stream_ptr()))
+            h.append(buf)
+        xbuf = torch.empty(nb, dtype=torch.uint8, device=dev)
+        packs = self.packs()
+        g8 = self._g8(lib, B, H, W, dev)
+        if W == 320:
+            # production feed at the fastMRI width: the DC kernel writes the G8 conv input itself, so the step starts
+            # from a filled G8 buffer (no converter launch)
+            _lib.check(lib.mrb_g8_from_nhwc4(_lib.ptr(g4), _lib.ptr(g8), B, H, W, _lib.stream_ptr()))
+            g4 = None
+        return (lambda: self.conv_stack_bh(g4, h, h_alt, xbuf, eta, packs, B, H, W, g8),
+                "split-bf16 tcgen05 ConvGRU stack of one time step on BH activations (bulk-copy-fed conv5x5x4, TMA-fed "
+                "ConvGRU, border, conv3x3d2, TMA-fed ConvGRU, tap-GEMM conv3x3->2 + eta)")
 
     def _steps_bh(self, eta, masked_kspace, sense, mask_can, sigma, h, y_hybrid, ws, fresh_state):
         """The time loop on BH buffers.  h: two BH state buffers (never written); returns (etas, final states)."""
@@ -256,14 +197,14 @@ class RimTcEngine:
         b = self.block
         B, C, H, W, _ = masked_kspace.shape
         dev = masked_kspace.device
-        packs = self.packs(bh=True)
+        packs = self.packs()
         nb = lib.mrb_bh_bytes(B, H, W)
         h = list(h)
         h_alt = [torch.empty(nb, dtype=torch.uint8, device=dev) for _ in range(2)]
         xbuf = torch.empty(nb, dtype=torch.uint8, device=dev)
         g8 = self._g8(lib, B, H, W, dev)
         # W = 320 row-form DC kernel writes the G8 conv input (split + replicate border) itself: no fp32 gradient tensor
-        direct = g8 is not None and y_hybrid is not None and W == 320 and C <= 16
+        direct = y_hybrid is not None and W == 320 and C <= 16
         g4 = None if direct else torch.empty((B, H, W, 4), dtype=torch.float32, device=dev)
         etas = []
         for step in range(b.time_steps):
@@ -276,7 +217,11 @@ class RimTcEngine:
             etas.append(eta)
         return etas, h
 
-    def _run_bh(self, eta, masked_kspace, sense, mask_can, sigma, hx, ws, y_hybrid, want_hx):
+    # ---------------------------------------------------------------------------------------------
+    def run(self, eta, masked_kspace, sense, mask_can, sigma, hx, ws, y_hybrid=None, want_hx=True):
+        """The time loop of rim_block.py:217-249 on images the engine covers.  eta [B,H,W,2]; hx: list of 2 NCHW-shaped
+        tensors or None.  Returns (list of etas, [h0, h1]) with the hidden states NCHW-shaped (channels-last strides);
+        ``want_hx=False`` (CIRIM.forward, which drops them, cirim.py:156-163) skips the export of the hidden states."""
         lib = _lib.load()
         b = self.block
         B, C, H, W, _ = masked_kspace.shape
@@ -352,42 +297,3 @@ class RimTcEngine:
             out.append(t.permute(0, 3, 1, 2))
         return etas, out
 
-    # ---------------------------------------------------------------------------------------------
-    def run(self, eta, masked_kspace, sense, mask_can, sigma, hx, ws, y_hybrid=None, want_hx=True):
-        """The time loop of rim_block.py:217-249.  eta [B,H,W,2]; hx: list of 2 NCHW-shaped tensors or None.
-        Returns (list of etas, [h0, h1]) with the hidden states NCHW-shaped (channels-last strides); ``want_hx=False``
-        (CIRIM.forward, which drops them, cirim.py:156-163) skips the export of the hidden states."""
-        if self.use_bh(masked_kspace.shape[3]):
-            return self._run_bh(eta, masked_kspace, sense, mask_can, sigma, hx, ws, y_hybrid, want_hx)
-        lib = _lib.load()
-        b = self.block
-        B, C, H, W, _ = masked_kspace.shape
-        dev = masked_kspace.device
-        packs = self.packs()
-        st = _lib.stream_ptr()
-
-        if hx is None:
-            # zero initial state (rim_block.py:188-193): one cached, read-only zero buffer feeds the first time step of
-            # every cascade instead of a fresh 26 MB-per-slice fill per layer and cascade
-            key = (B, H, W, str(dev))
-            if _ZERO_STATE.get("key") != key:  # one buffer shared by all cascades / engines (latest geometry only)
-                _ZERO_STATE.update(key=key, buf=torch.zeros((B, H, W, 64), dtype=torch.float32, device=dev))
-            h = [_ZERO_STATE["buf"], _ZERO_STATE["buf"]]
-        else:
-            # never write the caller's tensors: .contiguous() is a no-op for channels-last inputs, so clone explicitly
-            h = [hx[0].permute(0, 2, 3, 1).clone(memory_format=torch.contiguous_format),
-                 hx[1].permute(0, 2, 3, 1).clone(memory_format=torch.contiguous_format)]
-        h_alt = [torch.empty((B, H, W, 64), dtype=torch.float32, device=dev) for _ in range(2)]
-        xbuf = torch.empty((B, H, W, 64), dtype=torch.float32, device=dev)
-        g4 = torch.empty((B, H, W, 4), dtype=torch.float32, device=dev)
-        etas = []
-        eta = eta.contiguous()
-        for step in range(b.time_steps):
-            _ops.dc_rim_grad(eta, masked_kspace, sense, mask_can, sigma, b.fft_centered, b.fft_normalization, out=g4,
-                             ws=ws, nhwc=True, y_hybrid=y_hybrid)
-            eta = self.conv_stack(g4, h, h_alt, xbuf, eta, packs)
-            if step == 0 and hx is None:
-                # the ping-pong swap left the shared zero buffer in h_alt: it must never be written
-                h_alt = [torch.empty_like(h[0]), torch.empty_like(h[1])]
-            etas.append(eta)
-        return etas, [h[0].permute(0, 3, 1, 2), h[1].permute(0, 3, 1, 2)]

@@ -27,86 +27,14 @@ def _diag(out_nchw, ref, tol, what):
         raise AssertionError(msg)
 
 
-def _pack(kind, w, w2=None, k=1):
+def _pack(w, k):
     from mridc_b200 import _lib
 
     lib = _lib.load()
-    st = _lib.stream_ptr()
     w = w.contiguous()
-    if kind == 2:
-        p = torch.empty(lib.mrb_tc_packed_floats(2, w.shape[0], 4, 5), device="cuda")
-        _lib.check(lib.mrb_tc_pack_conv5x5x4(_lib.ptr(w), _lib.ptr(p), w.shape[0], st))
-    elif kind == 0:
-        p = torch.empty(lib.mrb_tc_packed_floats(0, w.shape[0], 64, k), device="cuda")
-        _lib.check(lib.mrb_tc_pack_conv(_lib.ptr(w), _lib.ptr(p), w.shape[0], 64, k, st))
-    else:
-        p = torch.empty(lib.mrb_tc_packed_floats(1, 64, 64, 1), device="cuda")
-        _lib.check(lib.mrb_tc_pack_gru(_lib.ptr(w), _lib.ptr(w2), _lib.ptr(p), 64, 64, st))
+    p = torch.empty(lib.mrb_tc_packed_floats(0, w.shape[0], 64, k), device="cuda")
+    _lib.check(lib.mrb_tc_pack_conv(_lib.ptr(w), _lib.ptr(p), w.shape[0], 64, k, _lib.stream_ptr()))
     return p
-
-
-@pytest.mark.parametrize("B,H,W", [(1, 16, 8), (2, 37, 45), (3, 33, 32), (2, 5, 100), (1, 320, 320)])
-def test_tc_ops_vs_oracle(B, H, W):
-    from mridc_b200 import _lib
-    from oracle import nets as onets
-
-    lib = _lib.load()
-    st = _lib.stream_ptr()
-    g = torch.Generator().manual_seed(H)
-
-    def nhwc(t):
-        return t.permute(0, 2, 3, 1).contiguous().cuda()
-
-    # NB: every device tensor is bound to a name before its pointer is taken (a temporary would be returned to
-    # the caching allocator -- and possibly reused -- before the kernel is even launched).
-    # conv 5x5 over the 4-channel gradient
-    x4 = torch.randn(B, 4, H, W, generator=g)
-    w1 = torch.randn(64, 4, 5, 5, generator=g) * 0.2
-    b1 = torch.randn(64, generator=g)
-    ref = onets.conv_nonlinear(x4, w1, b1, 5, 1, "relu")
-    out = torch.empty(B, H, W, 64, device="cuda")
-    x4d, p1, b1d = nhwc(x4), _pack(2, w1.cuda()), b1.cuda()
-    _lib.check(lib.mrb_tc_conv5x5x4_nhwc(_lib.ptr(x4d), _lib.ptr(p1), _lib.ptr(b1d), _lib.ptr(out), B, H, W, 64, 1, st))
-    _diag(out.permute(0, 3, 1, 2), ref, 1e-5, "conv5x5x4")
-    # conv 3x3 dilation 2 (and dilation 1), 64 -> 64
-    x = torch.randn(B, 64, H, W, generator=g)
-    xd = nhwc(x)
-    for dil, relu in ((2, 1), (1, 0)):
-        w2 = torch.randn(64, 64, 3, 3, generator=g) * 0.05
-        b2 = torch.randn(64, generator=g)
-        ref = onets.conv_nonlinear(x, w2, b2, 3, dil, "relu" if relu else None)
-        p2, b2d = _pack(0, w2.cuda(), k=3), b2.cuda()
-        _lib.check(lib.mrb_tc_conv_nhwc(_lib.ptr(xd), _lib.ptr(p2), _lib.ptr(b2d), _lib.ptr(out), B, H, W, 64, 3, dil,
-                                        relu, st))
-        _diag(out.permute(0, 3, 1, 2), ref, 1e-5, "conv3x3 dil %d" % dil)
-    # ConvGRU cell, kernel size 1
-    h = torch.randn(B, 64, H, W, generator=g)
-    wih = torch.randn(192, 64, 1, 1, generator=g) * 0.1
-    whh = torch.randn(192, 64, 1, 1, generator=g) * 0.1
-    bih = torch.randn(192, generator=g)
-    ref = onets.conv_gru_cell(x, h, wih, bih, whh, 1, 1)
-    hd, pg, bihd = nhwc(h), _pack(1, wih.cuda(), whh.cuda()), bih.cuda()
-    _lib.check(lib.mrb_tc_gru_nhwc(_lib.ptr(xd), _lib.ptr(hd), _lib.ptr(pg), _lib.ptr(bihd), _lib.ptr(out), B, H, W, 64,
-                                   st))
-    _diag(out.permute(0, 3, 1, 2), ref, 1e-5, "gru")
-    # IndRNN cell, kernel size 1: ReLU(ih(x) + hh * h) (rnn_cells.py:391) = 1x1 tensor-core conv + recurrent epilogue
-    wi = torch.randn(64, 64, 1, 1, generator=g) * 0.1
-    bi = torch.randn(64, generator=g)
-    hhw = torch.randn(1, 64, 1, 1, generator=g)
-    ref = onets.indrnn_cell(x, h, wi, bi, hhw, 1, 1)
-    pi, bid, hhd = _pack(0, wi.cuda(), k=1), bi.cuda(), hhw.reshape(-1).cuda()
-    _lib.check(lib.mrb_tc_indrnn_nhwc(_lib.ptr(xd), _lib.ptr(hd), _lib.ptr(pi), _lib.ptr(bid), _lib.ptr(hhd), _lib.ptr(out),
-                                      B, H, W, 64, st))
-    _diag(out.permute(0, 3, 1, 2), ref, 1e-5, "indrnn")
-    # final conv 64 -> 2 with the eta update
-    w3 = torch.randn(2, 64, 3, 3, generator=g) * 0.05
-    eta = torch.randn(B, H, W, 2, generator=g)
-    ref = eta + onets.conv_nonlinear(x, w3, None, 3, 1, None).permute(0, 2, 3, 1)
-    o2 = torch.empty(B, H, W, 2, device="cuda")
-    w3d, etad = w3.cuda(), eta.cuda()
-    _lib.check(lib.mrb_conv_c2_nhwc_residual(_lib.ptr(xd), _lib.ptr(w3d), None, _lib.ptr(etad), _lib.ptr(o2), B, H, W,
-                                             64, 3, 1, st))
-    assert rel_l2(o2, ref) < 2e-6
 
 
 def test_dc_nhwc_layout_matches_nchw():
@@ -167,37 +95,6 @@ def test_rim_block_tc_vs_fp32_and_oracle(monkeypatch, layer):
     with torch.no_grad():
         r2, _ = onets.rim_block(sd, dict(cfg), ref, y, S, m, None, [t.clone() for t in ref_h], 1.0, True)
     assert rel_l2(e2[-1], r2[-1]) < 5e-5
-
-
-def test_tc_kernels_are_deterministic():
-    """Race detector: the warp-specialised pipeline must give bit-identical results run to run."""
-    from mridc_b200 import _lib
-
-    lib = _lib.load()
-    st = _lib.stream_ptr()
-    g = torch.Generator(device="cuda").manual_seed(7)
-    B, H, W = 2, 96, 112
-    x = torch.randn(B, H, W, 64, device="cuda", generator=g)
-    h = torch.randn(B, H, W, 64, device="cuda", generator=g)
-    g4 = torch.randn(B, H, W, 4, device="cuda", generator=g)
-    w1 = torch.randn(64, 4, 5, 5, device="cuda", generator=g) * 0.2
-    w2 = torch.randn(64, 64, 3, 3, device="cuda", generator=g) * 0.05
-    wih = torch.randn(192, 64, device="cuda", generator=g) * 0.1
-    whh = torch.randn(192, 64, device="cuda", generator=g) * 0.1
-    b = torch.randn(192, device="cuda", generator=g)
-    p1, p2, pg = _pack(2, w1), _pack(0, w2, k=3), _pack(1, wih, whh)
-    outs = [[], [], []]
-    for _ in range(12):
-        o1, o2, o3 = (torch.empty(B, H, W, 64, device="cuda") for _ in range(3))
-        _lib.check(lib.mrb_tc_conv5x5x4_nhwc(_lib.ptr(g4), _lib.ptr(p1), _lib.ptr(b), _lib.ptr(o1), B, H, W, 64, 1, st))
-        _lib.check(lib.mrb_tc_conv_nhwc(_lib.ptr(x), _lib.ptr(p2), _lib.ptr(b), _lib.ptr(o2), B, H, W, 64, 3, 2, 1, st))
-        _lib.check(lib.mrb_tc_gru_nhwc(_lib.ptr(x), _lib.ptr(h), _lib.ptr(pg), _lib.ptr(b), _lib.ptr(o3), B, H, W, 64, st))
-        for lst, o in zip(outs, (o1, o2, o3)):
-            lst.append(o)
-    torch.cuda.synchronize()
-    for lst in outs:
-        for o in lst[1:]:
-            assert torch.equal(o, lst[0])
 
 
 def _bh_roundtrip(x_nhwc):
@@ -276,7 +173,7 @@ def test_tc2_indrnn_vs_oracle(B, H, W):
     hh = torch.randn(1, 64, 1, 1, generator=g) * 0.5
     xb, _ = _bh_roundtrip(x.permute(0, 2, 3, 1).contiguous().cuda())
     hb, _ = _bh_roundtrip(h.permute(0, 2, 3, 1).contiguous().cuda())
-    pk = _pack(0, wih.cuda().contiguous(), k=1)
+    pk = _pack(wih.cuda(), 1)
     hhd = hh.reshape(-1).cuda()
     for bias in (bih, None):
         ref = onets.indrnn_cell(x, h, wih, bias, hh, 1, 1)
@@ -297,8 +194,8 @@ def test_tc2_indrnn_vs_oracle(B, H, W):
 
 
 @pytest.mark.parametrize("B,H,W", [(2, 37, 45), (1, 64, 32), (2, 33, 28), (1, 320, 320), (1, 12, 30)])
-def test_tc2_conv_ops_vs_oracle(B, H, W):
-    """The convolutions of the time step on BH activations: conv5x5 (fp32 gradient -> BH), conv3x3 (BH -> BH, replicate
+def test_tc2_bh_conv_ops_vs_oracle(B, H, W):
+    """The convolutions of the time step on BH activations: conv5x5 (fp32 gradient -> G8 -> BH), conv3x3 (BH -> BH, replicate
     padding = the BH border), final conv (BH -> eta)."""
     from mridc_b200 import _lib
     from oracle import nets as onets
@@ -316,12 +213,8 @@ def test_tc2_conv_ops_vs_oracle(B, H, W):
     x4 = torch.randn(B, 4, H, W, generator=g)
     w1 = torch.randn(64, 4, 5, 5, generator=g) * 0.2
     b1 = torch.randn(64, generator=g)
-    ref = onets.conv_nonlinear(x4, w1, b1, 5, 1, "relu")
-    x4d, p1, b1d = x4.permute(0, 2, 3, 1).contiguous().cuda(), _pack(2, w1.cuda()), b1.cuda()
-    ob = torch.full((nb,), 0x7f, dtype=torch.uint8, device="cuda")
-    _lib.check(lib.mrb_tc_conv5x5x4_bh(_lib.ptr(x4d), _lib.ptr(p1), _lib.ptr(b1d), _lib.ptr(ob), B, H, W, 64, 1, st))
-    _diag(from_bh(ob), ref, 1e-5, "conv5x5x4 (bh)")
-    # bulk-copy-fed variant: fp32 gradient -> G8 -> BH, weights split on the fly, with and without bias / ReLU
+    x4d, b1d = x4.permute(0, 2, 3, 1).contiguous().cuda(), b1.cuda()
+    # bulk-copy-fed: fp32 gradient -> G8 -> BH, weights split on the fly, with and without bias / ReLU
     g8 = torch.zeros(lib.mrb_g8_bytes(B, H, W), dtype=torch.uint8, device="cuda")
     _lib.check(lib.mrb_g8_from_nhwc4(_lib.ptr(x4d), _lib.ptr(g8), B, H, W, st))
     w1d = w1.cuda()
@@ -341,7 +234,7 @@ def test_tc2_conv_ops_vs_oracle(B, H, W):
         w2 = torch.randn(64, 64, 3, 3, generator=g) * 0.05
         b2 = torch.randn(64, generator=g)
         ref = onets.conv_nonlinear(x, w2, b2, 3, dil, "relu" if relu else None)
-        p2, b2d = _pack(0, w2.cuda(), k=3), b2.cuda()
+        p2, b2d = _pack(w2.cuda(), 3), b2.cuda()
         ob = torch.full((nb,), 0x7f, dtype=torch.uint8, device="cuda")
         _lib.check(lib.mrb_tc_conv_bh(_lib.ptr(xb), _lib.ptr(p2), _lib.ptr(b2d), _lib.ptr(ob), B, H, W, 64, 3, dil, relu, st))
         _diag(from_bh(ob), ref, 1e-5, "conv3x3 dil %d (bh)" % dil)
@@ -430,12 +323,18 @@ def test_unet_conv3x3_tc_vs_oracle(N, Cin, Cout, H, W):
     assert torch.equal(o2, ov)
 
 
-@pytest.mark.parametrize("B,H,W", [(1, 8, 32), (1, 12, 28), (3, 5, 40)])
-def test_cirim_tiny_images_on_the_bh_engine(B, H, W):
-    """Images smaller than a tile / a TMA box (the final tap GEMM falls back to the CUDA-core kernel below 16 padded rows)."""
+@pytest.mark.parametrize("B,H,W", [(1, 8, 32), (1, 12, 28), (3, 5, 40), (1, 12, 20)])
+def test_cirim_tiny_images_on_the_bh_engine_or_the_fp32_loop(monkeypatch, B, H, W):
+    """Images smaller than a tile / a TMA box (the final tap GEMM falls back to the CUDA-core kernel below 16 padded rows);
+    below the engine's width of 28 the block runs the exact-fp32 loop."""
     import mridc_b200 as mb
     from mridc_b200 import synth
+    from mridc_b200.rim_tc import RimTcEngine
     from oracle import models as omodels
+
+    runs = []
+    tc_run = RimTcEngine.run
+    monkeypatch.setattr(RimTcEngine, "run", lambda self, *a, **k: runs.append(W) or tc_run(self, *a, **k))
 
     cfg = synth.cirim_cfg("GRU", num_cascades=1, centered=True, normalization="ortho")
     batch = synth.make_batch(B, 3, H, W, centered=True, normalization="ortho")
@@ -449,6 +348,8 @@ def test_cirim_tiny_images_on_the_bh_engine(B, H, W):
     e = rel_l2(out[-1][-1], ref[-1][-1])
     print("[tc parity] tiny CIRIM %dx%dx%d rel-L2 %.2e" % (B, H, W, e))
     assert e < 3e-5
+    assert model.cirim[0]._tc_engine  # the block geometry is the engine's; only the width decides
+    assert bool(runs) == (W >= 28)
 
 
 def test_cirim_graph_replay_equals_eager(monkeypatch):

@@ -11,9 +11,8 @@ def load():
     if not os.path.exists(_build.TOOLS_LIB_PATH):
         _build.build_tools()
     lib = ctypes.CDLL(os.path.abspath(_build.TOOLS_LIB_PATH))
-    for name in ("mrb_tc_packed_floats", "mrb_tc_pack_conv", "mrb_tc_pack_gru", "mrb_tc_pack_conv5x5x4", "mrb_tc_conv_nhwc",
-                 "mrb_tc_conv5x5x4_nhwc", "mrb_tc_gru_nhwc", "mrb_tc_indrnn_nhwc", "mrb_conv_c2_nhwc_residual", "mrb_last_error",
-                 "mrb_tc_conv5x5x4_bh", "mrb_tc_conv_bh", "mrb_conv_c2_bh_residual", "mrb_bh_fix_border",
+    for name in ("mrb_tc_packed_floats", "mrb_tc_pack_conv", "mrb_last_error", "mrb_tc_conv_bh", "mrb_conv_c2_bh_residual",
+                 "mrb_bh_fix_border",
                  "mrb_bh_bytes", "mrb_bh_from_nhwc", "mrb_bh_to_nhwc", "mrb_tc2_gru_packed_bytes", "mrb_tc2_pack_gru", "mrb_tc2_gru", "mrb_tc2_unet_conv3x3"):
         res, args = _lib.SIGNATURES[name]
         fn = getattr(lib, name)

@@ -1,4 +1,4 @@
-"""Attribute tc_kernel time to its roles by switching them off (results are garbage, timing only)."""
+"""Per-role cycle counters of tc_kernel (the BH k x k conv of conv_tc.cu) at the dilated 3x3 of the CIRIM time step."""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -10,10 +10,9 @@ lib = _toolslib.load(); st = _lib.stream_ptr()   # profiling build of the same k
 B, H, W = int(sys.argv[1]) if len(sys.argv) > 1 else 1, 320, 320
 dev = torch.device("cuda")
 model = mb.CIRIM(synth.cirim_cfg("GRU")).cuda().eval()
-blk = model.cirim[0]; eng = RimTcEngine(blk); packs = eng.packs(bh=False)
-g4 = torch.randn(B, H, W, 4, device=dev); x = torch.randn(B, H, W, 64, device=dev); h = torch.randn(B, H, W, 64, device=dev)
-out = torch.empty(B, H, W, 64, device=dev)
-c0, c1, r0 = blk.layers[0].convs, blk.layers[1].convs, blk.layers[0].rnn
+blk = model.cirim[0]; eng = RimTcEngine(blk); packs = eng.packs()
+x = torch.randn(B, H, W, 64, device=dev)
+c1 = blk.layers[1].convs
 def t(fn, n=20):
     for _ in range(3): fn()
     torch.cuda.synchronize()
@@ -26,11 +25,7 @@ nb = lib.mrb_bh_bytes(B, H, W)
 xb = torch.empty(nb, dtype=torch.uint8, device=dev); ob = torch.empty(nb, dtype=torch.uint8, device=dev)
 lib.mrb_bh_from_nhwc(_lib.ptr(x), _lib.ptr(xb), B, H, W, st)
 ops = {
- "conv5x5x4_bh": lambda: lib.mrb_tc_conv5x5x4_bh(_lib.ptr(g4), _lib.ptr(packs[0][0]), _lib.ptr(c0.conv_layer.bias), _lib.ptr(ob), B, H, W, 64, 1, st),
  "conv3x3d2_bh": lambda: lib.mrb_tc_conv_bh(_lib.ptr(xb), _lib.ptr(packs[1][0]), _lib.ptr(c1.conv_layer.bias), _lib.ptr(ob), B, H, W, 64, 3, 2, 1, st),
- "conv5x5x4": lambda: lib.mrb_tc_conv5x5x4_nhwc(_lib.ptr(g4), _lib.ptr(packs[0][0]), _lib.ptr(c0.conv_layer.bias), _lib.ptr(out), B, H, W, 64, 1, st),
- "gru": lambda: lib.mrb_tc_gru_nhwc(_lib.ptr(x), _lib.ptr(h), _lib.ptr(packs[0][1]), _lib.ptr(r0.ih.bias), _lib.ptr(out), B, H, W, 64, st),
- "conv3x3d2": lambda: lib.mrb_tc_conv_nhwc(_lib.ptr(x), _lib.ptr(packs[1][0]), _lib.ptr(c1.conv_layer.bias), _lib.ptr(out), B, H, W, 64, 3, 2, 1, st),
 }
 for flags, name in ((0, "full"),):
     lib.mrb_tc_set_debug(flags)
@@ -47,9 +42,6 @@ for dbg in (0,):
     print("%-12s loader: total %7.0f wait_empty %7.0f store %7.0f (st-wait+arrive %7.0f) issue %7.0f | mma: total %7.0f wait_full %7.0f wait_acc %7.0f issue %7.0f commit %7.0f wait_b %7.0f seg-top..issue %7.0f | epi: total %7.0f wait %7.0f (cycles, mean over CTAs)" % (
         k, p[0], p[1], p[2], p[13], p[3], p[4], p[5], p[6], p[7], p[10], p[11], p[12], p[8], p[9]))
 lib.mrb_tc_set_debug(0); lib.mrb_tc_set_prof(None)
-w3 = blk.final_layer[0].conv_layer.weight
-eta = torch.randn(B, H, W, 2, device=dev); o2 = torch.empty_like(eta)
-print("conv_c2 %.1f us" % t(lambda: lib.mrb_conv_c2_nhwc_residual(_lib.ptr(x), _lib.ptr(w3), None, _lib.ptr(eta), _lib.ptr(o2), B, H, W, 64, 3, 1, st)))
 lib.mrb_tc_set_prof(_lib.ptr(prof))
 for k, f in ops.items():
     prof.zero_(); f(); torch.cuda.synchronize()

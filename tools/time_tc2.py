@@ -45,19 +45,18 @@ new = lambda: _lib.check(lib.mrb_tc2_final_conv(_lib.ptr(ob), _lib.ptr(w3), None
 u0, u1 = after_gru(old), after_gru(new)
 print("final conv B=%d: fp32 CUDA-core + border fix %.1f us, tensor-core tap GEMM %.1f us (%.0f GB/s at 272 B/px)" %
       (B, u0, u1, px * 272 / u1 / 1e3))
-# first conv: gen-1 loader-warp kernel vs the bulk-copy-fed G8 kernel (incl. its fp32 -> G8 converter)
+# first conv: the bulk-copy-fed G8 kernel and its fp32 -> G8 converter
 from mridc_b200.rim_tc import RimTcEngine
 import mridc_b200 as mb
 from mridc_b200 import synth
 blk = mb.CIRIM(synth.cirim_cfg("GRU")).cuda().eval().cirim[0]
-eng = RimTcEngine(blk); packs = eng.packs(bh=True)
+eng = RimTcEngine(blk); packs = eng.packs()
 c0 = blk.layers[0].convs; c1 = blk.layers[1].convs
 g4 = torch.randn(B, H, W, 4, device=dev)
 g8 = torch.zeros(lib.mrb_g8_bytes(B, H, W), dtype=torch.uint8, device=dev)
-u_old = t(lambda: _lib.check(lib.mrb_tc_conv5x5x4_bh(_lib.ptr(g4), _lib.ptr(packs[0][0]), _lib.ptr(c0.conv_layer.bias), _lib.ptr(ob), B, H, W, 64, 1, st)))
 u_cv = t(lambda: _lib.check(lib.mrb_g8_from_nhwc4(_lib.ptr(g4), _lib.ptr(g8), B, H, W, st)))
 u_new = t(lambda: _lib.check(lib.mrb_tc2_conv5x5x4(_lib.ptr(g8), _lib.ptr(c0.conv_layer.weight), _lib.ptr(c0.conv_layer.bias), _lib.ptr(ob), B, H, W, 1, st)))
-print("conv5x5 B=%d: gen-1 %.1f us; G8 converter %.1f us + bulk-copy kernel %.1f us (%.0f GB/s at 272 B/px)" % (B, u_old, u_cv, u_new, px * 272 / u_new / 1e3))
+print("conv5x5 B=%d: G8 converter %.1f us + bulk-copy kernel %.1f us (%.0f GB/s at 272 B/px)" % (B, u_cv, u_new, px * 272 / u_new / 1e3))
 u3 = t(lambda: _lib.check(lib.mrb_tc_conv_bh(_lib.ptr(hb), _lib.ptr(packs[1][0]), _lib.ptr(c1.conv_layer.bias), _lib.ptr(ob), B, H, W, 64, 3, 2, 1, st)))
 print("conv3x3 d2 B=%d: %.1f us (%.1f TFLOP/s algorithmic)" % (B, u3, px * 2 * 64 * 64 * 9 / u3 / 1e6))
 # IndRNN cell on BH activations
