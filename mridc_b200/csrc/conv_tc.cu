@@ -502,9 +502,15 @@ static int launch(Params& P, void* out, cudaStream_t st) {
 #endif
     const size_t max_smem = device_max_smem_optin();
     P.tmem_cols = 512;
+    // The two loader groups take turns by kernel row: a group's next unit starts k segments after the end of its last one,
+    // so without at least k + 1 TMEM stages a loader can reach a stage two rounds ahead of the issuer, where the parity
+    // wait of mbarrier cannot tell the round it needs from the one before (the 5x5 conv on 4 stages hung).  A kernel size
+    // whose ring would be shorter gives up the second accumulator buffer.
+    if ((512 - P.acc_bufs * P.acc_cols) / A_STAGE_COLS < P.ksz + 1) P.acc_bufs = 1;
     P.stages = (512 - P.acc_bufs * P.acc_cols) / A_STAGE_COLS;
     if (P.stages > MAX_STAGES) P.stages = MAX_STAGES;
-    MRB_REQUIRE(P.stages >= 2, MRB_EUNSUPPORTED, "tensor-core conv: accumulator leaves no room for the TMEM A ring");
+    MRB_REQUIRE(P.stages >= 2 && P.stages >= P.ksz + 1, MRB_EUNSUPPORTED,
+                "tensor-core conv: the TMEM A ring needs %d stages for k = %d", P.ksz + 1, P.ksz);
     MRB_REQUIRE(P.P < 2147483647LL, MRB_EUNSUPPORTED, "tensor-core conv: too many pixels");
     MRB_REQUIRE(P.nseg >= 1 && P.nseg <= MAX_SEGS, MRB_EUNSUPPORTED, "tensor-core conv: bad segment count");
     CUtensorMap tm_out;

@@ -18,19 +18,34 @@ __device__ __forceinline__ double warp_sum(double v) {
     return v;
 }
 
-// stats[2*plane + {0,1}] += (sum, sumsq) of plane `blockIdx.y` ; planes are x + n*bs + c*HW
-__global__ void plane_stats_kernel(const float* __restrict__ x, long long bs, int C, long long HW,
-                                   double* __restrict__ stats) {
-    const int plane = blockIdx.y;
+// stats[2*plane + {0,1}] = (sum, sumsq) of one plane (planes are x + n*bs + c*HW).  A cluster of PS_CLUSTER CTAs owns a
+// plane: element i is summed by thread i mod (PS_CLUSTER * PS_THREADS), four loads in flight per thread, and the CTA
+// partials are combined through distributed shared memory in rank order.  The order of every addition is fixed by HW
+// alone, so the statistics are the same bits run to run and whatever the number of planes in the launch (the atomics of a
+// plane-count-dependent grid were neither).  The price: a launch of few planes reads them with 8 CTAs each.
+constexpr int PS_CLUSTER = 8, PS_THREADS = 1024, PS_UNROLL = 4;
+__global__ void __launch_bounds__(PS_THREADS) plane_stats_kernel(const float* __restrict__ x, long long bs, int C,
+                                                                 long long HW, double* __restrict__ stats) {
+    cg::cluster_group cluster = cg::this_cluster();
+    const int cs = (int)cluster.num_blocks(), rank = (int)cluster.block_rank();
+    const int plane = blockIdx.x / cs;
     const int n = plane / C, c = plane - n * C;
     const float* p = x + (long long)n * bs + (long long)c * HW;
     double s = 0.0, ss = 0.0;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < HW; i += (long long)gridDim.x * blockDim.x) {
-        double v = (double)p[i];
-        s += v;
-        ss += v * v;
+    const long long T = (long long)cs * PS_THREADS;
+    for (long long i = (long long)rank * PS_THREADS + threadIdx.x; i < HW; i += PS_UNROLL * T) {
+        float v[PS_UNROLL];
+#pragma unroll
+        for (int u = 0; u < PS_UNROLL; ++u) v[u] = i + u * T < HW ? __ldg(p + i + u * T) : 0.f;
+#pragma unroll
+        for (int u = 0; u < PS_UNROLL; ++u) {
+            const double d = (double)v[u];
+            s += d;
+            ss += d * d;
+        }
     }
     __shared__ double sh[2][32];
+    __shared__ double part[2];
     s = warp_sum(s);
     ss = warp_sum(ss);
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -42,11 +57,20 @@ __global__ void plane_stats_kernel(const float* __restrict__ x, long long bs, in
         ss = lane < nw ? sh[1][lane] : 0.0;
         s = warp_sum(s);
         ss = warp_sum(ss);
-        if (lane == 0) {
-            atomicAdd(&stats[2 * plane], s);
-            atomicAdd(&stats[2 * plane + 1], ss);
-        }
+        if (lane == 0) { part[0] = s; part[1] = ss; }
     }
+    cluster.sync();  // every CTA's partial sums are published
+    if (rank == 0 && threadIdx.x == 0) {
+        double ts = 0.0, tss = 0.0;
+        for (int r = 0; r < cs; ++r) {
+            const double* rp = cluster.map_shared_rank(part, r);
+            ts += rp[0];
+            tss += rp[1];
+        }
+        stats[2 * plane] = ts;
+        stats[2 * plane + 1] = tss;
+    }
+    cluster.sync();  // remote reads done before any CTA of the cluster may exit
 }
 
 __global__ void instnorm_apply_kernel(const float* __restrict__ x, long long xbs, float* __restrict__ out,
@@ -69,10 +93,9 @@ __global__ void instnorm_apply_kernel(const float* __restrict__ x, long long xbs
 
 // InstanceNorm2d + LeakyReLU in ONE pass over global memory: a thread-block cluster owns one (n, c) plane, every CTA keeps
 // its share of the plane in shared memory while it accumulates the fp64 sums, the per-CTA sums are exchanged through
-// distributed shared memory (fixed rank order: the statistics do not depend on scheduling, unlike the atomics of the
-// two-kernel form), and the normalised values are written from shared memory.  1 read + 1 write per element instead of
-// 2 reads + 1 write and three launches (memset, statistics, apply).  In-place use (out == x) is safe: an element is
-// read before its own CTA writes it.
+// distributed shared memory (fixed rank order: the statistics do not depend on scheduling), and the normalised values are
+// written from shared memory.  1 read + 1 write per element instead of the 2 reads + 1 write and two launches (statistics,
+// apply) of the two-kernel form.  In-place use (out == x) is safe: an element is read before its own CTA writes it.
 constexpr int IN_THREADS = 512;
 __global__ void __launch_bounds__(IN_THREADS) instnorm_cluster_kernel(const float* __restrict__ x, long long xbs, float* out,
                                                                       long long obs, int C, int HW, int chunk, float eps,
@@ -400,10 +423,22 @@ extern "C" int mrb_instnorm_lrelu(const void* x, long long x_bstride, void* out,
             return MRB_OK;
         }
     }
-    MRB_CUDA(cudaMemsetAsync(stats, 0, sizeof(double) * 2 * planes, st));
+    {
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3((unsigned)(planes * PS_CLUSTER));
+        cfg.blockDim = dim3(PS_THREADS);
+        cfg.stream = st;
+        cudaLaunchAttribute at[1];
+        at[0].id = cudaLaunchAttributeClusterDimension;
+        at[0].val.clusterDim.x = (unsigned)PS_CLUSTER;
+        at[0].val.clusterDim.y = 1;
+        at[0].val.clusterDim.z = 1;
+        cfg.attrs = at;
+        cfg.numAttrs = 1;
+        MRB_CUDA(cudaLaunchKernelEx(&cfg, plane_stats_kernel, (const float*)x, x_bstride, C, HW, (double*)stats));
+        MRB_LAUNCHED();
+    }
     dim3 grid(split_grid(HW, planes), planes);
-    plane_stats_kernel<<<grid, 256, 0, st>>>((const float*)x, x_bstride, C, HW, (double*)stats);
-    MRB_LAUNCHED();
     instnorm_apply_kernel<<<grid, 256, 0, st>>>((const float*)x, x_bstride, (float*)out, out_bstride, C, HW,
                                                 (const double*)stats, eps, slope);
     MRB_LAUNCHED();
