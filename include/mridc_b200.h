@@ -9,6 +9,8 @@
  * Conventions
  *   - plain pointers and sizes only; every pointer is DEVICE memory owned by the caller (PyTorch),
  *     contiguous, fp32 unless stated; complex tensors are interleaved (re,im) = "complex-last-2".
+ *   - every pointer is 16-byte aligned (the tensor-core kernels read and write through TMA and bulk copies, which
+ *     require it; PyTorch's allocator hands out 512-byte aligned blocks).
  *   - all work is enqueued on `stream` (a cudaStream_t passed as void*); no hidden synchronisation,
  *     graph-capturable after one eager warm-up call (twiddle tables are created on first use per device
  *     and FFT length, owned by the library, immutable afterwards).

@@ -39,9 +39,19 @@ __global__ void abs_normalize_kernel(const float* __restrict__ x, long long n, i
         out[i] = __fdiv_rn(magnitude(x, i, is_complex), mx);
 }
 
-// sums[0] = sum (gt - pred)^2, sums[1] = sum gt^2 (fp64); ext[0..3] = ordered-int max gt, min gt, max pred, min pred
+// unsigned order key of a float: fkey(a) < fkey(b) iff a < b for non-NaN a, b, and key 0 lies below every such key (it is
+// the key of the all-ones NaN pattern), so a ZEROED word is a valid start for atomicMax.  A minimum is kept as the maximum
+// of ~fkey (whose zero start stands for +inf).  Zero starts let the caller initialise the workspace with one memset.
+__device__ __forceinline__ unsigned fkey(float f) {
+    const unsigned u = __float_as_uint(f);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float key2f(unsigned k) { return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k); }
+
+// sums[0] = sum (gt - pred)^2, sums[1] = sum gt^2 (fp64); ext[0..3] = fkey(max gt), ~fkey(min gt), fkey(max pred),
+// ~fkey(min pred); sums and ext zeroed by the host wrapper
 __global__ void metric_sums_kernel(const float* __restrict__ gt, const float* __restrict__ pred, long long n,
-                                   double* __restrict__ sums, int* __restrict__ ext) {
+                                   double* __restrict__ sums, unsigned* __restrict__ ext) {
     double se = 0.0, sg = 0.0;
     float gmax = -INFINITY, gmin = INFINITY, pmax = -INFINITY, pmin = INFINITY;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
@@ -61,8 +71,8 @@ __global__ void metric_sums_kernel(const float* __restrict__ gt, const float* __
     if ((threadIdx.x & 31) == 0) {
         atomicAdd(&sums[0], se);
         atomicAdd(&sums[1], sg);
-        atomicMax(&ext[0], f2ord(gmax)); atomicMin(&ext[1], f2ord(gmin));
-        atomicMax(&ext[2], f2ord(pmax)); atomicMin(&ext[3], f2ord(pmin));
+        atomicMax(&ext[0], fkey(gmax)); atomicMax(&ext[1], ~fkey(gmin));
+        atomicMax(&ext[2], fkey(pmax)); atomicMax(&ext[3], ~fkey(pmin));
     }
 }
 
@@ -109,17 +119,19 @@ __global__ void ssim_sum_kernel(const float* __restrict__ gt, const float* __res
 }
 
 // Everything test_step derives from the sums, on the device (no host round trip between the reductions):
-// res[0] = mse, [1] = nmse, [2] = psnr, [3] = ssim, [4] = data range used.  maxval_mode 0: max(gt)
-// (reconstruction_metrics.py:23,35), 1: max(pred) - min(pred) (base.py:431,434), 2: res[4] preset by the caller.
-__global__ void metrics_finish_kernel(const double* __restrict__ sums, const int* __restrict__ ext, double n, int maxval_mode,
-                                      double* __restrict__ res) {
+// res[0] = mse, [1] = nmse, [2] = psnr, [3] = NaN when SSIM is skipped (ssim_finish_kernel writes it otherwise),
+// [4] = data range used.  maxval_mode 0: max(gt) (reconstruction_metrics.py:23,35), 1: max(pred) - min(pred)
+// (base.py:431,434), 2: `maxval`.  Host values arrive as kernel arguments, which a captured CUDA graph holds by value.
+__global__ void metrics_finish_kernel(const double* __restrict__ sums, const unsigned* __restrict__ ext, double n, int maxval_mode,
+                                      double maxval, int want_ssim, double* __restrict__ res) {
     const double mse = sums[0] / n;
-    double R = res[4];
-    if (maxval_mode == 0) R = (double)ord2f(ext[0]);
-    if (maxval_mode == 1) R = (double)(ord2f(ext[2]) - ord2f(ext[3]));  // float32 subtraction, like numpy on float32
+    double R = maxval;
+    if (maxval_mode == 0) R = (double)key2f(ext[0]);
+    if (maxval_mode == 1) R = (double)(key2f(ext[2]) - key2f(~ext[3]));  // float32 subtraction, like numpy on float32
     res[0] = mse;
     res[1] = sums[0] / sums[1];
     res[2] = 10.0 * log10(R * R / mse);
+    if (!want_ssim) res[3] = __longlong_as_double(0x7ff8000000000000LL);
     res[4] = R;
 }
 __global__ void ssim_finish_kernel(const double* __restrict__ per_slice, int B, double windows, double* __restrict__ res) {
@@ -161,27 +173,18 @@ extern "C" int mrb_recon_metrics(const void* gt, const void* pred, int B, int H,
                 "mrb_recon_metrics: win_size exceeds image extent (need H, W >= 7; got %d x %d)", H, W);
     MRB_REQUIRE(maxval_mode >= 0 && maxval_mode <= 2, MRB_EINVAL, "mrb_recon_metrics: maxval_mode must be 0, 1 or 2 (+ 4)");
     cudaStream_t st = (cudaStream_t)stream;
-    // workspace: doubles [0,1] sums | ints at double slot 2..3: ext[4] | doubles [8 .. 8+B) per-slice SSIM sums
-    struct Init { double sums[2]; int ext[4]; } init;
-    init.sums[0] = init.sums[1] = 0.0;
-    const int lo = (int)0x80000000, hi = 0x7fffffff;  // ordered-int -inf-ish / +inf-ish sentinels
-    init.ext[0] = lo; init.ext[1] = hi; init.ext[2] = lo; init.ext[3] = hi;
+    // workspace: doubles [0,1] sums | unsigned at double slot 2..3: ext[4] | doubles [8 .. 8+B) per-slice SSIM sums; every
+    // start value is zero (see fkey), so one memset initialises it
     double* wsd = (double*)ws;
-    // cudaMemcpyAsync from pageable host memory stages the source before returning, so the stack struct is safe
-    MRB_CUDA(cudaMemcpyAsync(wsd, &init, sizeof(init), cudaMemcpyHostToDevice, st));
-    MRB_CUDA(cudaMemsetAsync(wsd + 8, 0, sizeof(double) * B, st));
     double* resd = (double*)res;
-    if (maxval_mode == 2) MRB_CUDA(cudaMemcpyAsync(resd + 4, &maxval, sizeof(double), cudaMemcpyHostToDevice, st));
+    MRB_CUDA(cudaMemsetAsync(wsd, 0, sizeof(double) * (8 + (size_t)B), st));
     const long long n = (long long)B * H * W;
-    metric_sums_kernel<<<mgrid(n), 256, 0, st>>>((const float*)gt, (const float*)pred, n, wsd, (int*)(wsd + 2));
+    metric_sums_kernel<<<mgrid(n), 256, 0, st>>>((const float*)gt, (const float*)pred, n, wsd, (unsigned*)(wsd + 2));
     MRB_LAUNCHED();
-    metrics_finish_kernel<<<1, 1, 0, st>>>(wsd, (const int*)(wsd + 2), (double)n, maxval_mode, resd);
+    metrics_finish_kernel<<<1, 1, 0, st>>>(wsd, (const unsigned*)(wsd + 2), (double)n, maxval_mode, maxval, want_ssim ? 1 : 0,
+                                           resd);
     MRB_LAUNCHED();
-    if (!want_ssim) {
-        const double qnan = __builtin_nan("");
-        MRB_CUDA(cudaMemcpyAsync(resd + 3, &qnan, sizeof(double), cudaMemcpyHostToDevice, st));
-        return MRB_OK;
-    }
+    if (!want_ssim) return MRB_OK;
     const int vw = W - SSIM_WIN + 1, vh = H - SSIM_WIN + 1;
     dim3 grid((vw + SSIM_TX - 1) / SSIM_TX, (vh + SSIM_TY - 1) / SSIM_TY, B);
     ssim_sum_kernel<<<grid, dim3(SSIM_TX, SSIM_TY), 0, st>>>((const float*)gt, (const float*)pred, H, W, resd + 4, wsd + 8);
