@@ -1,4 +1,5 @@
-"""Build recipe for libmridc_b200.so (hand-written CUDA for sm_100a, C-ABI in include/mridc_b200.h).
+"""Build recipe for libmridc_b200.so (hand-written CUDA for sm_100a, C-ABI in include/mridc_b200.h) and
+libmridc_b200_espirit.so (coil-sensitivity estimation, C-ABI in include/mridc_b200_espirit.h).
 
 The library is built IN-TREE (mridc_b200/libmridc_b200.so) with nvcc so that it travels with the source
 snapshot to the GPU box; nvcc cross-compiles without a GPU.  `python -m mridc_b200.build` or
@@ -15,6 +16,11 @@ CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libmridc_b200.so")
 STAMP = os.path.join(PKG_DIR, "csrc", ".build_stamp")
 SOURCES = ["core.cu", "fft.cu", "dc.cu", "conv.cu", "unet.cu", "conv_tc.cu", "conv_tc2.cu", "qmri.cu", "metrics.cu"]
+# ESPIRiT library: a library of its own (no core.cu); its transforms come from libmridc_b200.so through Python
+ESPIRIT_SOURCES = ["espirit.cu"]
+ESPIRIT_HEADER = os.path.join(PKG_DIR, "..", "include", "mridc_b200_espirit.h")
+ESPIRIT_LIB_PATH = os.path.join(PKG_DIR, "libmridc_b200_espirit.so")
+ESPIRIT_STAMP = os.path.join(PKG_DIR, "csrc", ".build_stamp_espirit")
 # tools-only library (tools/libmridc_b200_tools.so): the tensor-core kernels with their per-role cycle counters and role
 # switches compiled in (-DMRB_TC_PROF) plus the tcgen05 issue micro-benchmark; never loaded by the package
 TOOLS_SOURCES = ["core.cu", "conv_tc.cu", "conv_tc2.cu", "conv.cu", "tc_microbench.cu"]
@@ -38,7 +44,7 @@ def _digest():
     h = hashlib.sha256()
     for root, _, files in sorted(os.walk(CSRC)):
         for f in sorted(files):
-            if f.endswith((".cu", ".cuh", ".h")):
+            if f.endswith((".cu", ".cuh", ".h")) and f not in ESPIRIT_SOURCES:
                 with open(os.path.join(root, f), "rb") as fh:
                     h.update(f.encode() + b"\0" + fh.read())
     with open(os.path.join(PKG_DIR, "..", "include", "mridc_b200.h"), "rb") as fh:
@@ -47,19 +53,46 @@ def _digest():
     return h.hexdigest()
 
 
+def _espirit_digest():
+    h = hashlib.sha256()
+    for f in ESPIRIT_SOURCES:
+        with open(os.path.join(CSRC, f), "rb") as fh:
+            h.update(f.encode() + b"\0" + fh.read())
+    with open(ESPIRIT_HEADER, "rb") as fh:
+        h.update(fh.read())
+    h.update(" ".join(NVCC_FLAGS).encode())
+    return h.hexdigest()
+
+
+def _fresh(path, stamp, digest):
+    if os.path.exists(path) and os.path.exists(stamp):
+        with open(stamp) as fh:
+            return fh.read().strip() == digest
+    return False
+
+
 def build(force=False, verbose=False):
-    """Compile every CUDA source for sm_100a into one shared library. Returns the library path."""
+    """Compile every CUDA source for sm_100a: libmridc_b200.so and libmridc_b200_espirit.so. Returns the path of the
+    first."""
     digest = _digest()
-    if not force and os.path.exists(LIB_PATH) and os.path.exists(STAMP):
-        with open(STAMP) as fh:
-            if fh.read().strip() == digest:
-                return LIB_PATH
+    if force or not _fresh(LIB_PATH, STAMP, digest):
+        _compile(SOURCES, LIB_PATH, os.path.join(PKG_DIR, "csrc", "build"), verbose)
+        with open(STAMP, "w") as fh:
+            fh.write(digest)
+    digest = _espirit_digest()
+    if force or not _fresh(ESPIRIT_LIB_PATH, ESPIRIT_STAMP, digest):
+        _compile(ESPIRIT_SOURCES, ESPIRIT_LIB_PATH, os.path.join(PKG_DIR, "csrc", "build", "espirit"), verbose)
+        with open(ESPIRIT_STAMP, "w") as fh:
+            fh.write(digest)
+    return LIB_PATH
+
+
+def _compile(sources, lib_path, objdir, verbose):
     nvcc = _nvcc()
-    objdir = os.path.join(PKG_DIR, "csrc", "build")
     os.makedirs(objdir, exist_ok=True)
     procs = []
     objs = []
-    for src in SOURCES:
+    for src in sources:
         obj = os.path.join(objdir, src.replace(".cu", ".o"))
         objs.append(obj)
         cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", os.path.join(CSRC, src), "-o", obj]
@@ -74,11 +107,8 @@ def build(force=False, verbose=False):
             sys.stderr.write(out)
     if failed:
         raise RuntimeError("nvcc compilation failed")
-    cmd = [nvcc, "-shared", "-Wno-deprecated-gpu-targets", "-o", LIB_PATH] + objs + ["-lcudart"]
+    cmd = [nvcc, "-shared", "-Wno-deprecated-gpu-targets", "-o", lib_path] + objs + ["-lcudart"]
     subprocess.check_call(cmd)
-    with open(STAMP, "w") as fh:
-        fh.write(digest)
-    return LIB_PATH
 
 
 def build_tools():
