@@ -11,26 +11,45 @@
 // on tcgen05.mma.kind::f16 (bf16 operands, fp32 accumulation in TMEM).  hi + lo carries 16-17 significant bits
 // (|x - hi - lo| <= 2^-18 |x|), the dropped a_lo*b_lo term is <= 2^-18 relative: ~3e-6 rms per operator, 2.5e-5
 // end to end over the 40 time steps of CIRIM 5x8 (measured with a CPU emulation of this arithmetic against the fp32
-// oracle; the budget is 1e-4).  Round 1 used 3xTF32 (22 bits, 2.6e-6 end to end): same three MMAs per product but
-// at half the tensor-pipe rate and twice the instruction count (K = 8 instead of 16 per MMA) -- the kernels were
-// bound by exactly those two.
+// oracle; the budget is 1e-4).
 //
-// Structure: one persistent CTA per SM.  Work item = one 128-position tile, all 64 output channels.  Segment = one tap
-// (64 input channels = one K chunk of 64 bf16).
-//   * B operand = the weights of one tap (hi rows | lo rows, pre-packed in the UMMA K-major SWIZZLE_128B layout by
-//     mrb_tc_pack_conv), streamed from L2 through a small ring of shared-memory slots by the weight-streaming lane.
-//   * A operand = activations, held in TENSOR MEMORY (tcgen05.mma with A from TMEM): a ring of TMEM stages of
-//     64 columns (32 hi + 32 lo columns of packed bf16 pairs = one 64-channel K chunk for the 128 positions/lanes).
-//     Shared memory therefore carries no activation traffic for the MMAs.
-//   loader warps (2 groups x 4, alternating (tile, kernel row) units): cp.async gather of the warp's 32 positions plus
-//                     the halo of one kernel row into a swizzled staging tile (current + next in flight); tap kx of that
-//                     row is staging row lane + kx*dil, copied to the TMEM stage with tcgen05.st (thread = position = TMEM
-//                     lane);
-//   MMA warp (1 lane) 4 k-steps (K = 16) x 2 stacked tcgen05.mma.kind::f16 per segment (A from TMEM, B descriptor in smem)
-//                     and tcgen05.commit of the stage back to the loaders / of the accumulator to the epilogue;
-//   epilogue warps (8) tcgen05.ld the accumulator (one position per thread, 2 warps per lane quadrant), apply bias and
-//                     optional ReLU, split into hi / lo bf16 and stage the tile in the TMA box layout;
-//   TMA store lane    the two box stores of each tile.
+// Structure: one persistent CTA per SM, A and B operands from shared memory, TMEM holds accumulators only.
+//   Work item = one or two consecutive 128-position tiles of the flat [B(H+4)(W+4)] grid (a pair may straddle two
+//   slices), all 64 output channels.  Unit = (item, kernel row ky): for each tile of the item one 2-D TMA box per half
+//   (hi, lo) of 136 positions x 128 B in SWIZZLE_128B (17 x 1024 B), starting `pad` positions before the tile's first
+//   position of that kernel row.  Tap (ky, kx) of a tile is the same box read kx*dil rows further on: only the A
+//   descriptor's start moves, by kx*dil*128 B (desc_rows).  Box rows outside the tensor are zero-filled by TMA; they only
+//   feed border outputs.
+//   TMA producer (1 lane)  per unit: the item's A boxes, then the unit's k weight chunks ([b_hi; b_lo], 16 KB, one bulk
+//                 copy each, packed by mrb_tc_pack_conv);
+//   MMA issuer (1 warp, elected lane)  per tap: the 8 MMAs of tile 0 then the 8 of tile 1 from the same weight chunk
+//                 (each streamed chunk feeds both tiles), in the order of umma_segment_ss_stacked: taps row-major, k-steps
+//                 0..3, a_hi x [b_hi; b_lo] (N = 128) into [main | cross] then a_lo x b_hi (N = 64) into cross.  A tile's
+//                 accumulation order does not depend on whether it runs in a pair, so every output is bit-identical
+//                 whatever the batch or the grid;
+//   epilogue warps (8)  tcgen05.ld the accumulator (one position per thread, 2 warps per lane quadrant), RN add of main +
+//                 cross, bias, optional ReLU, split into hi / lo bf16 and stage the tile in the TMA box layout;
+//   TMA store lane  the two box stores of each tile.
+//
+// Rings (each mbarrier parity wait must be within one phase of the barrier: a ring is deeper than the distance its
+// producer can run ahead of its slowest consumer, since the parity cannot tell phase it from phase it - 2):
+//   A units     2 slots (4 boxes = 68 KB each).  One producer and one consumer walk the same unit sequence; the producer
+//               refills a slot after the issuer's commit of the unit two before (a_empty), the issuer waits a_full: the
+//               producer is 0..2 units ahead, never 3.
+//   weights     3 slots of 16 KB, same protocol per tap (b_full / b_empty).  The producer's order A(u), W(u, 0..k-1),
+//               A(u+1) cannot deadlock: the A(u+2) wait needs only unit u's MMAs, whose chunks were issued before A(u+1).
+//   accumulators 4 TMEM buffers of 128 columns [main 64 | cross 64] (all 512 columns); tile s of the CTA uses buffer
+//               s % 4.  The issuer waits acc_empty (8 epilogue arrivals) of tile s - 4 before the first MMA of tile s,
+//               an item takes at most 2 buffers, and every epilogue warp walks the tiles in order.
+//   output tile 1 slot (hi box | lo box).  An epilogue warp writes tile s after out_free of tile s - 1 (store lane) and
+//               cannot pass tile s + 1 before all 8 warps have arrived on out_ready for tile s.
+// Nothing reads a TMA-landed slot through the generic proxy (the MMAs release A and B slots with tcgen05.commit), so no
+// proxy fence is needed there; the epilogue's generic writes of the output tile are fenced before out_ready.
+//
+// Shared memory: 2 x 68 KB A + 3 x 16 KB weights + 32 KB output tile + barriers and bias = 216.5 KB (+ 1 KB alignment).
+//
+// Work dealing: all CTAs take pairs for as many rounds as every CTA completes, then the rem < 2 * grid remaining tiles
+// are dealt so that no CTA runs a pair while another idles: rem - grid CTAs take a pair, the others one tile each.
 #include <cuda.h>
 
 #include "tc_ptx.cuh"
@@ -40,23 +59,24 @@ namespace tc {
 
 constexpr int TILE_M = 128;
 constexpr int COUT = 64;                      // output channels (all of them in one CTA)
-constexpr int KC = 32;                        // TMEM columns of one K chunk half (hi or lo): 64 bf16 channels, packed in pairs
 constexpr int KCH = 64;                       // channels per K chunk (one 128-byte row of bf16 in the B operand)
-constexpr int A_STAGE_COLS = 2 * KC;          // hi + lo
 constexpr int EPI_WARPS = 8;                  // 2 warps per TMEM lane quadrant (each takes half of the channels)
-constexpr int LOAD_GROUPS = 2, LOAD_WARPS = 4 * LOAD_GROUPS;  // loader groups alternate (tile, kernel row) units
-constexpr int MMA_WARPS = 2;                  // MMA issuer + TMA store lane
-constexpr int THREADS = (EPI_WARPS + LOAD_WARPS + MMA_WARPS + 1) * 32;  // + weight-streaming warp
-constexpr int B_STAGES = 6;                   // max depth of the streamed-weights ring (Params::b_stages)
+constexpr int PRODUCER_WARP = EPI_WARPS, MMA_WARP = EPI_WARPS + 1, STORE_WARP = EPI_WARPS + 2;
+constexpr int THREADS = (EPI_WARPS + 3) * 32;
 constexpr int MAX_SEGS = 25;
-constexpr int MAX_STAGES = 6;
 constexpr int W_CHUNK_BYTES = COUT * 128;     // hi (or lo) rows of one weight chunk
-
+constexpr int B_STAGES = 3;                   // streamed-weights ring
+constexpr int A_UNITS = 2;                    // A ring: (item, kernel row) units
+constexpr int A_BOX_ROWS = 136;               // 128 + 2 * pad, rounded up to whole 8-row swizzle atoms
+constexpr int A_BOX_BYTES = A_BOX_ROWS * 128; // 17 x 1024: every box stays 1024-aligned
+constexpr int A_UNIT_BYTES = 4 * A_BOX_BYTES; // [tile 0 hi | tile 0 lo | tile 1 hi | tile 1 lo]
+constexpr int ACC_BUFS = 4;
+constexpr int ACC_COLS = 2 * COUT;            // [main | cross]
 constexpr int BH_PAD = 2;                     // replicate border of the BH activation layout (conv_tc2.cu)
-constexpr int BH_PX_BYTES = 256;              // 64 hi + 64 lo bf16 per position
 constexpr int OUT_BOX_BYTES = TILE_M * 128;   // one [128 positions x 64 bf16] TMA box
-constexpr int HALO_ROWS = 32 + 2 * BH_PAD;    // staging rows of one loader unit at most: 32 positions + pad on each side
-constexpr int BIAS_FLOATS = COUT;
+constexpr int BAR_BYTES = 256;
+constexpr size_t SMEM_BYTES = 1024 + (size_t)A_UNITS * A_UNIT_BYTES + (size_t)B_STAGES * 2 * W_CHUNK_BYTES +
+                              2 * OUT_BOX_BYTES + BAR_BYTES + COUT * sizeof(float);
 
 // Profiling hooks (per-role cycle counters, role switches) exist only in the tools build (-DMRB_TC_PROF,
 // tools/libmridc_b200_tools.so); the product kernel carries none of them.
@@ -69,290 +89,216 @@ constexpr int BIAS_FLOATS = COUT;
 #endif
 
 struct Params {
-    const uint8_t* src;      // BH input (replicate border valid)
     const void* wpack;       // packed bf16 weights: [tap][hi|lo][64 rows x 128 B swizzled]
     const float* bias;       // [64] (may be null)
-    int B, H, W;             // image size
-    long long P;             // flat positions of the BH layout, B (H+4)(W+4): the tiles run over them
-    int n_tiles;
-    int nseg;                // segments (taps) per tile; the global segment stream s = item * nseg + sgi is dealt to
-                             // the TMEM stages and the weight ring
-    int acc_cols;            // TMEM columns of one accumulator buffer: [hi*hi chain | cross-term chain]
-    int acc_bufs;            // accumulator buffers
-    int tmem_cols;           // allocation: 512
-    int relu;
-    int b_stages;            // depth of the streamed-weights ring (<= B_STAGES)
-    int tb_depth;            // cp.async staging tiles per loader warp
-    int tb_half;             // bytes of one staging half (32 + 2*pad rows x 128 B)
-    int tb_bytes;            // bytes of one staging tile (2 halves)
+    int n_tiles;             // 128-position tiles over the B (H+4)(W+4) flat positions
+    int pitch;               // W + 4
     int ksz, dil;            // conv geometry
-    int stages;              // A stages in TMEM (columns acc_bufs*acc_cols + 64*s)
+    int relu;
 #ifdef MRB_TC_PROF
     unsigned long long* prof; // optional [gridDim.x][16] cycle counters (tools/tc_roles.py)
-    int debug;                // role switches: 1 skip MMAs, 2 skip global loads, 4 skip epilogue math, 8 skip tcgen05.st
+    int debug;                // role switches: 1 skip MMAs, 2 skip TMA / bulk loads, 4 skip epilogue math
 #endif
 };
 
-__global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ CUtensorMap tm_out, const Params P) {
+// The items of this CTA (see the header): item i covers tiles [t0, t0 + count); count 0 past the last one.
+struct Deal {
+    int rounds, base, n2, n_tiles;
+    __device__ explicit Deal(int nt) : n_tiles(nt) {
+        rounds = nt / (2 * (int)gridDim.x);
+        base = 2 * (int)gridDim.x * rounds;
+        n2 = max(0, nt - base - (int)gridDim.x);
+    }
+    __device__ int item(int i, int& t0) const {
+        const int c = blockIdx.x;
+        if (i < rounds) { t0 = 2 * (c + (int)gridDim.x * i); return 2; }
+        if (i > rounds) return 0;
+        if (c < n2) { t0 = base + 2 * c; return 2; }
+        t0 = base + n2 + c;  // base + 2 n2 + (c - n2)
+        return t0 < n_tiles ? 1 : 0;
+    }
+};
+
+__global__ void __launch_bounds__(THREADS, 1)
+tc_kernel(const __grid_constant__ CUtensorMap tm_in, const __grid_constant__ CUtensorMap tm_out, const Params P) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
-    // layout: [output tile][streamed-weights ring][loader staging tiles][barriers][bias]
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    uint8_t* out_s = smem;                                            // [hi box | lo box] output tile (1024-aligned)
-    uint8_t* bst_s = smem + 2 * OUT_BOX_BYTES;                        // [b_stages][2*W_CHUNK_BYTES]
-    uint8_t* tb_s = bst_s + (size_t)P.b_stages * 2 * W_CHUNK_BYTES;   // [LOAD_WARPS][depth][tb_bytes]
-    uint64_t* bars = (uint64_t*)(tb_s + (size_t)LOAD_WARPS * P.tb_depth * P.tb_bytes);
-    uint64_t* full = bars;                          // [MAX_STAGES]
-    uint64_t* empty = bars + MAX_STAGES;            // [MAX_STAGES]
-    uint64_t* acc_full = bars + 2 * MAX_STAGES;     // [2]
-    uint64_t* acc_empty = acc_full + 2;             // [2]
-    uint32_t* tmem_slot = (uint32_t*)(acc_empty + 2);
-    uint64_t* b_full = acc_empty + 4;               // [B_STAGES]
-    uint64_t* b_empty = b_full + B_STAGES;          // [B_STAGES]
-    uint64_t* out_free = acc_empty + 3;             // [1] the TMA stores of the previous tile have read out_s
-    uint64_t* out_ready = b_empty + B_STAGES;       // [1] every epilogue warp has written its part of the output tile
-    float* bias_s = (float*)(out_ready + 2);        // [BIAS_FLOATS] (16-byte aligned): bias staged once per CTA
+    uint8_t* a_s = smem;                                             // [A_UNITS][A_UNIT_BYTES]
+    uint8_t* w_s = a_s + (size_t)A_UNITS * A_UNIT_BYTES;             // [B_STAGES][hi rows | lo rows]
+    uint8_t* out_s = w_s + (size_t)B_STAGES * 2 * W_CHUNK_BYTES;     // [hi box | lo box] output tile
+    uint64_t* a_full = (uint64_t*)(out_s + 2 * OUT_BOX_BYTES);       // [A_UNITS]
+    uint64_t* a_empty = a_full + A_UNITS;                            // [A_UNITS] tcgen05.commit of the unit's MMAs
+    uint64_t* b_full = a_empty + A_UNITS;                            // [B_STAGES]
+    uint64_t* b_empty = b_full + B_STAGES;                           // [B_STAGES] tcgen05.commit of the tap's MMAs
+    uint64_t* acc_full = b_empty + B_STAGES;                         // [ACC_BUFS]
+    uint64_t* acc_empty = acc_full + ACC_BUFS;                       // [ACC_BUFS] one arrival per epilogue warp
+    uint64_t* out_ready = acc_empty + ACC_BUFS;                      // every epilogue warp has written its part of the tile
+    uint64_t* out_free = out_ready + 1;                              // the TMA stores of the previous tile have read out_s
+    uint32_t* tmem_slot = (uint32_t*)(out_free + 1);
+    float* bias_s = (float*)(out_s + 2 * OUT_BOX_BYTES + BAR_BYTES); // [COUT] (16-byte aligned): bias staged once per CTA
 
     // warp index through a shuffle: provably warp-uniform for the compiler (role branches and the MMA issuer's operands
     // then live in uniform registers)
     const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
-    const int first_tile = blockIdx.x;
-    const int tile_stride = gridDim.x;
+    const Deal deal(P.n_tiles);
 
     if (threadIdx.x == 0) {
-        for (int s = 0; s < P.stages; ++s) {
-            mbar_init(&full[s], 4);    // one loader group fills a stage: one arrival per warp (lane 0, after __syncwarp)
-            mbar_init(&empty[s], 1);
+        for (int i = 0; i < A_UNITS; ++i) {
+            mbar_init(&a_full[i], 1);   // the producer's arrive.expect_tx; the TMA boxes complete the transaction bytes
+            mbar_init(&a_empty[i], 1);
         }
-        for (int b = 0; b < 2; ++b) {
-            mbar_init(&acc_full[b], 1);
-            mbar_init(&acc_empty[b], EPI_WARPS);  // one arrival per epilogue warp
+        for (int i = 0; i < B_STAGES; ++i) {
+            mbar_init(&b_full[i], 1);
+            mbar_init(&b_empty[i], 1);
         }
-        for (int b = 0; b < B_STAGES; ++b) {
-            mbar_init(&b_full[b], 1);   // the producer's arrive.expect_tx; the bulk copy completes the transaction bytes
-            mbar_init(&b_empty[b], 1);  // tcgen05.commit of the MMAs that read the slot
+        for (int i = 0; i < ACC_BUFS; ++i) {
+            mbar_init(&acc_full[i], 1);
+            mbar_init(&acc_empty[i], EPI_WARPS);
         }
-        mbar_init(out_free, 1);
         mbar_init(out_ready, EPI_WARPS);
+        mbar_init(out_free, 1);
         fence_barrier_init();
     }
     for (int i = threadIdx.x; i < COUT; i += THREADS) bias_s[i] = P.bias ? P.bias[i] : 0.f;
-    if (warp == EPI_WARPS + LOAD_WARPS) tmem_alloc(tmem_slot, (uint32_t)P.tmem_cols);
+    if (warp == MMA_WARP) tmem_alloc(tmem_slot, 512);
     fence_proxy_async();
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    const uint32_t a_col0 = (uint32_t)(P.acc_bufs * P.acc_cols);  // first TMEM column of the A ring
-    int n_items = 0;
-    for (int t = first_tile; t < P.n_tiles; t += tile_stride) ++n_items;
-    if (warp >= EPI_WARPS && warp < EPI_WARPS + LOAD_WARPS) {
-        // ============================== LOADERS ==============================
-        // The global segment stream s = item * nseg + sgi is dealt to the two loader groups in (tile, kernel row) units
-        // of k segments; segment s goes to TMEM stage s % stages.
-        const int lw = warp - EPI_WARPS;
-        const int grp = lw >> 2;                     // loader group
-        const int quad = lw & 3;                     // == warp % 4: the TMEM lane quadrant this warp may write
-        const int c16 = lane & 7;                    // 16-byte chunk within a 128-byte half row (coalesced view)
-        const int rl0 = lane >> 3;                   // rows rl0 + 4*i of the staging tile (coalesced view)
-        const uint32_t tb_u32 = smem_u32(tb_s + (size_t)lw * P.tb_depth * P.tb_bytes);  // tb_depth staging tiles of this warp
-        const uint32_t HB = (uint32_t)P.tb_half;     // the lo half of a staging row lives HB bytes after the hi half
-        const bool ld_on = !TC_DBG(P, 2);
-        TCP(long long t_start = clock64(), t_wait = 0, t_st = 0, t_issue = 0, t_stw = 0, c0;)
+    const int k = P.ksz, dil = P.dil, pad = dil * (k - 1) / 2;
 
-        int stage = 0;
-        uint32_t phase = 0;
-        auto stage_set = [&](long long s) { stage = (int)(s % P.stages); phase = (uint32_t)(s / P.stages) & 1u; };
-        auto stage_adv = [&](int n) {
-            stage += n;
-            while (stage >= P.stages) { stage -= P.stages; phase ^= 1u; }
-        };
-        // staging row `row` of tile tb (64 hi bf16 in half 0, 64 lo bf16 in half 1) -> TMEM stage (thread = position =
-        // TMEM lane quad*32 + lane): columns [0,32) = hi pairs, [32,64) = lo pairs -- a straight copy
-        auto store_stage = [&](uint32_t tb, int row, int stg) {
-            const uint32_t ta = tmem_base + ((uint32_t)(quad * 32) << 16) + a_col0 + (uint32_t)(stg * A_STAGE_COLS);
-#pragma unroll
-            for (int hf = 0; hf < 2; ++hf) {
-                uint32_t v[32];
-#pragma unroll
-                for (int c = 0; c < 8; ++c) {
-                    const float4 a = lds128(tb + hf * HB + swz(row, c));
-                    v[4 * c] = __float_as_uint(a.x); v[4 * c + 1] = __float_as_uint(a.y);
-                    v[4 * c + 2] = __float_as_uint(a.z); v[4 * c + 3] = __float_as_uint(a.w);
+    if (warp == PRODUCER_WARP) {
+        // ============================== TMA PRODUCER ==============================
+        if (lane == 0) {
+            TCP(long long t_start = clock64(), t_wa = 0, t_wb = 0, c0;)
+            const bool ld_on = !TC_DBG(P, 2);
+            const uint8_t* wpack = reinterpret_cast<const uint8_t*>(P.wpack);
+            int u = 0, bs = 0;
+            uint32_t uph = 0, bph = 0;
+            int t0;
+            for (int i = 0, cnt; (cnt = deal.item(i, t0)) > 0; ++i) {
+                for (int ky = 0; ky < k; ++ky) {
+                    TCP(c0 = clock64();)
+                    mbar_wait_sleep(&a_empty[u], uph ^ 1, 64);
+                    TCP(t_wa += clock64() - c0;)
+                    // first position of the box: kernel row ky of the tile's first position, pad positions to the left
+                    const int q_off = (ky * dil - pad) * P.pitch - pad;
+                    const uint32_t dst = smem_u32(a_s + (size_t)u * A_UNIT_BYTES), bar = smem_u32(&a_full[u]);
+                    if (ld_on) {
+                        mbar_expect_tx(&a_full[u], (uint32_t)(cnt * 2 * A_BOX_BYTES));
+                        for (int j = 0; j < cnt; ++j) {
+                            const int q0 = (t0 + j) * TILE_M + q_off;
+                            tma_load_2d(dst + (uint32_t)(2 * j * A_BOX_BYTES), &tm_in, 0, q0, bar);
+                            tma_load_2d(dst + (uint32_t)((2 * j + 1) * A_BOX_BYTES), &tm_in, 64, q0, bar);
+                        }
+                    } else {
+                        mbar_arrive(&a_full[u]);
+                    }
+                    if (++u == A_UNITS) { u = 0; uph ^= 1; }
+                    for (int kx = 0; kx < k; ++kx) {
+                        TCP(c0 = clock64();)
+                        mbar_wait_sleep(&b_empty[bs], bph ^ 1, 64);
+                        TCP(t_wb += clock64() - c0;)
+                        if (ld_on) {
+                            mbar_expect_tx(&b_full[bs], (uint32_t)(2 * W_CHUNK_BYTES));
+                            bulk_load_1d(smem_u32(w_s + (size_t)bs * 2 * W_CHUNK_BYTES),
+                                         wpack + (size_t)(ky * k + kx) * 2 * W_CHUNK_BYTES, (uint32_t)(2 * W_CHUNK_BYTES),
+                                         smem_u32(&b_full[bs]));
+                        } else {
+                            mbar_arrive(&b_full[bs]);
+                        }
+                        if (++bs == B_STAGES) { bs = 0; bph ^= 1; }
+                    }
                 }
-                if (!TC_DBG(P, 8)) {
-                    tmem_st16(ta + hf * KC, v);
-                    tmem_st16(ta + hf * KC + 16, v + 16);
-                }
             }
-        };
-        // wait for the stage, copy one staging row per lane, hand the stage to the issuer
-        auto fill_stage = [&](uint32_t tb, int row) {
-            TCP(c0 = clock64();)
-            mbar_wait_sleep(&empty[stage], phase ^ 1, 40);
-            TCP(t_wait += clock64() - c0;)
-            tc_fence_after();
-            TCP(c0 = clock64();)
-            store_stage(tb, row, stage);
-            TCP(const long long c2 = clock64();)
-            tmem_st_wait();
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&full[stage]);
-            TCP(t_st += clock64() - c0; t_stw += clock64() - c2;)
-        };
-
-        // unit = (tile, kernel row ky): the warp's 32 positions plus pad on each side of flat row offset
-        // (ky*dil - pad) * pitch; tap kx reads staging row lane + kx*dil.  Positions outside the tensor are zero-filled
-        // (they only feed border positions, whose results are not used).
-        const int k = P.ksz, dil = P.dil, pad = dil * (k - 1) / 2;
-        const long long pitch = P.W + 2 * BH_PAD;
-        const int n_units = n_items * k;
-        const int nrows = 32 + 2 * pad;
-        auto issue_halo = [&](int tile, int ky, int slot) {
-            const long long q0 = (long long)tile * TILE_M + quad * 32 - pad + (long long)(ky * dil - pad) * pitch;
-            const uint32_t sbase = tb_u32 + (uint32_t)(slot * P.tb_bytes);
-#pragma unroll
-            for (int i = 0; i < HALO_ROWS / 4; ++i) {
-                const int sr = rl0 + 4 * i;
-                if (sr >= nrows) break;  // the staging tile has exactly nrows rows (a zero-fill would land in the lo half)
-                const long long q = q0 + sr;
-                const bool ok = q >= 0 && q < P.P;
-                const uint8_t* g = P.src + q * BH_PX_BYTES + c16 * 16;
-                const uint32_t nb = (ok && ld_on) ? 16u : 0u;
-                cp_async16(sbase + swz(sr, c16), ok ? (const void*)g : (const void*)P.src, nb, true);
-                cp_async16(sbase + HB + swz(sr, c16), ok ? (const void*)(g + 128) : (const void*)P.src, nb, true);
-            }
-        };
-        int pf_u = grp, pf_tile = first_tile, pf_ky = grp, pf_slot = 0;
-        while (pf_ky >= k) { pf_ky -= k; pf_tile += tile_stride; }
-        auto prefetch_unit = [&]() {
-            if (pf_u < n_units) issue_halo(pf_tile, pf_ky, pf_slot);
-            asm volatile("cp.async.commit_group;" ::: "memory");
-            pf_u += LOAD_GROUPS;
-            pf_ky += LOAD_GROUPS;
-            while (pf_ky >= k) { pf_ky -= k; pf_tile += tile_stride; }
-            pf_slot ^= 1;
-        };
-        prefetch_unit();
-        int slot = 0;
-        stage_set((long long)grp * k);
-        for (int u = grp; u < n_units; u += LOAD_GROUPS) {
-            TCP(c0 = clock64();)
-            prefetch_unit();
-            TCP(t_issue += clock64() - c0;)
-            asm volatile("cp.async.wait_group 1;" ::: "memory");
-            __syncwarp();
-            const uint32_t tb = tb_u32 + (uint32_t)(slot * P.tb_bytes);
-            for (int kx = 0; kx < k; ++kx) {
-                fill_stage(tb, lane + kx * dil);
-                stage_adv(1);
-            }
-            __syncwarp();  // every lane has read its rows before the slot is refilled
-            stage_adv(k * (LOAD_GROUPS - 1));  // the other group's unit
-            slot ^= 1;
-        }
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
 #ifdef MRB_TC_PROF
-        if (P.prof && lane == 0 && lw == 0) {
-            unsigned long long* o = P.prof + (size_t)blockIdx.x * 16;
-            o[0] = clock64() - t_start; o[1] = t_wait; o[2] = t_st; o[3] = t_issue; o[13] = t_stw;
-        }
+            if (P.prof) {
+                unsigned long long* o = P.prof + (size_t)blockIdx.x * 16;
+                o[0] = clock64() - t_start; o[1] = t_wa; o[2] = t_wb;
+            }
 #endif
-    } else if (warp == EPI_WARPS + LOAD_WARPS) {
+        }
+    } else if (warp == MMA_WARP) {
         // ============================== MMA ISSUER ==============================
-        // Segments are issued in order into one accumulator buffer per tile, so a position's result is bit-identical run
-        // to run and whatever the batch it is part of.  Whole warp, warp-uniform control flow (see umma_commit).
+        // Whole warp, warp-uniform control flow, one elected lane per tcgen05 instruction (see umma_commit).
         TCP(const bool prof = P.prof != nullptr;)
-        int stage = 0;
-        uint32_t phase = 0;
-        int bs = 0;
-        uint32_t bphase = 0;
-        TCP(long long t_start = clock64(), t_wfull = 0, t_wacc = 0, t_mma = 0, t_commit = 0, t_wb = 0, t_prep = 0, c0 = 0, c1 = 0;)
-        int buf = 0;
-        uint32_t acc_phase = 0;
+        TCP(long long t_start = clock64(), t_wa = 0, t_wb = 0, t_wacc = 0, t_mma = 0, t_commit = 0, c0 = 0;)
         const uint32_t tmem_u = uni(tmem_base);
-        const uint32_t bst_u32 = smem_u32(bst_s);
-        // loop-invariant operands: every segment has N = 64 and the same accumulator columns; only the weight slot moves
-        const uint64_t desc0 = make_desc(bst_u32);
+        // loop-invariant operands: only the unit slot, the tap row and the weight slot move
+        const uint64_t adesc0 = make_desc(smem_u32(a_s)), bdesc0 = make_desc(smem_u32(w_s));
         constexpr uint32_t idesc_n = make_idesc(TILE_M, COUT), idesc_2n = make_idesc(TILE_M, 2 * COUT);
-        for (int tile = first_tile; tile < P.n_tiles; tile += tile_stride) {
+        constexpr uint32_t BOX16 = A_BOX_BYTES >> 4;  // descriptor units
+        int u = 0, bs = 0, seq = 0;  // seq: tiles of this CTA so far (accumulator buffer seq % 4)
+        uint32_t uph = 0, bph = 0;
+        int t0;
+        for (int i = 0, cnt; (cnt = deal.item(i, t0)) > 0; ++i) {
             TCP(if (prof) c0 = clock64();)
-            mbar_wait(&acc_empty[buf], acc_phase ^ 1);
+            for (int j = 0; j < cnt; ++j) mbar_wait(&acc_empty[(seq + j) & 3], (((uint32_t)(seq + j) >> 2) & 1u) ^ 1u);
             TCP(if (prof) t_wacc += clock64() - c0;)
             tc_fence_after();
-            const uint32_t d = tmem_u + (uint32_t)(buf * P.acc_cols);
-            for (int sgi = 0; sgi < P.nseg; ++sgi) {
-                TCP(if (prof) c1 = clock64();)
-                // every MMA operand is derived from kernel parameters and uniform loop state (no shared-memory table, no
-                // shuffles): it stays in uniform registers, and it is ready before the waits return
-                const uint64_t dbh = desc0 + (uint64_t)((bs * 2 * W_CHUNK_BYTES) >> 4);
-                const uint32_t a_hi = tmem_u + a_col0 + (uint32_t)(stage * A_STAGE_COLS);
+            const uint32_t d0 = tmem_u + (uint32_t)((seq & 3) * ACC_COLS), d1 = tmem_u + (uint32_t)(((seq + 1) & 3) * ACC_COLS);
+            for (int ky = 0; ky < k; ++ky) {
+                const uint64_t au = adesc0 + (uint64_t)((u * A_UNIT_BYTES) >> 4);
                 TCP(if (prof) c0 = clock64();)
-                mbar_wait(&b_full[bs], bphase);
-                TCP(if (prof) t_wb += clock64() - c0;)
-                TCP(if (prof) c0 = clock64();)
-                mbar_wait(&full[stage], phase);
-                TCP(if (prof) t_wfull += clock64() - c0;)
-                tc_fence_after();
-                TCP(if (prof) { c0 = clock64(); t_prep += c0 - c1; })
-                if (!TC_DBG(P, 1)) {
-                    // the N = 2n MMA of k-step 0 of the first segment overwrites [main | cross]; everything after it
-                    // accumulates (MMAs of one thread execute in order)
-                    umma_segment_ts_stacked(d, d + (uint32_t)COUT, a_hi, a_hi + KC, dbh, idesc_2n, idesc_n, sgi == 0 ? 0u : 1u);
+                mbar_wait(&a_full[u], uph);
+                TCP(if (prof) t_wa += clock64() - c0;)
+                for (int kx = 0; kx < k; ++kx) {
+                    const uint64_t a = desc_rows(au, (uint32_t)(kx * dil));
+                    const uint64_t b = bdesc0 + (uint64_t)((bs * 2 * W_CHUNK_BYTES) >> 4);
+                    const uint32_t acc = (ky | kx) != 0;  // the first MMA of a tile overwrites [main | cross]
+                    TCP(if (prof) c0 = clock64();)
+                    mbar_wait(&b_full[bs], bph);
+                    TCP(if (prof) { t_wb += clock64() - c0; c0 = clock64(); })
+                    tc_fence_after();
+                    if (!TC_DBG(P, 1)) {
+                        umma_segment_ss_stacked(d0, d0 + COUT, a, a + BOX16, b, idesc_2n, idesc_n, acc);
+                        if (cnt == 2) umma_segment_ss_stacked(d1, d1 + COUT, a + 2 * BOX16, a + 3 * BOX16, b, idesc_2n, idesc_n, acc);
+                    }
+                    TCP(if (prof) { t_mma += clock64() - c0; c0 = clock64(); })
+                    umma_commit(&b_empty[bs]);  // the chunk is reusable once both tiles' MMAs have read it
+                    TCP(if (prof) t_commit += clock64() - c0;)
+                    if (++bs == B_STAGES) { bs = 0; bph ^= 1u; }
                 }
-                TCP(if (prof) { t_mma += clock64() - c0; c0 = clock64(); })
-                umma_commit(&empty[stage]);  // stage reusable once these MMAs have read it
-                umma_commit(&b_empty[bs]);
-                if (++bs == P.b_stages) { bs = 0; bphase ^= 1u; }
-                TCP(if (prof) t_commit += clock64() - c0;)
-                if (++stage == P.stages) { stage = 0; phase ^= 1u; }
+                umma_commit(&a_empty[u]);
+                if (++u == A_UNITS) { u = 0; uph ^= 1u; }
             }
-            umma_commit(&acc_full[buf]);
-            if (++buf == P.acc_bufs) { buf = 0; acc_phase ^= 1u; }
+            for (int j = 0; j < cnt; ++j) umma_commit(&acc_full[(seq + j) & 3]);
+            seq += cnt;
         }
 #ifdef MRB_TC_PROF
         if (prof && lane == 0) {
             unsigned long long* o = P.prof + (size_t)blockIdx.x * 16;
-            o[4] = clock64() - t_start; o[5] = t_wfull; o[6] = t_wacc; o[7] = t_mma; o[10] = t_commit; o[11] = t_wb; o[12] = t_prep;
+            o[4] = clock64() - t_start; o[5] = t_wa; o[6] = t_wacc; o[7] = t_mma; o[10] = t_commit; o[11] = t_wb;
         }
 #endif
-    } else if (warp == EPI_WARPS + LOAD_WARPS + 1) {
+    } else if (warp == STORE_WARP) {
         // ============================== TMA STORE LANE ==============================
         if (lane == 0) {
+            TCP(long long t_start = clock64(), t_w = 0, c0;)
             const uint32_t out_u32 = smem_u32(out_s);
             uint32_t oph = 0;
-            for (int tile = first_tile; tile < P.n_tiles; tile += tile_stride) {
-                mbar_wait_sleep(out_ready, oph, 64);
-                tma_store_2d(&tm_out, out_u32, 0, tile * TILE_M);
-                tma_store_2d(&tm_out, out_u32 + OUT_BOX_BYTES, 64, tile * TILE_M);
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-                mbar_arrive(out_free);
-                oph ^= 1;
-            }
-            asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");  // stores complete before the CTA exits
-        }
-    } else if (warp == EPI_WARPS + LOAD_WARPS + MMA_WARPS) {
-        // ============================== WEIGHT STREAMER ==============================
-        // one lane, one bulk copy (cp.async.bulk, 2*W_CHUNK_BYTES contiguous bytes: hi rows | lo rows) per segment
-        if (lane == 0) {
-            int bs = 0;
-            uint32_t bphase = 0;
-            const uint32_t bytes = (uint32_t)(2 * W_CHUNK_BYTES);
-            for (int it = 0; it < n_items; ++it) {
-                for (int sgi = 0; sgi < P.nseg; ++sgi) {
-                    mbar_wait_sleep(&b_empty[bs], bphase ^ 1, 64);
-                    const uint8_t* gsrc = reinterpret_cast<const uint8_t*>(P.wpack) + (size_t)sgi * bytes;
-                    const uint32_t bar = smem_u32(&b_full[bs]);
-                    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-                    asm volatile(
-                        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                            smem_u32(bst_s + (size_t)bs * bytes)),
-                        "l"(gsrc), "r"(bytes), "r"(bar)
-                        : "memory");
-                    if (++bs == P.b_stages) { bs = 0; bphase ^= 1; }
+            int t0;
+            for (int i = 0, cnt; (cnt = deal.item(i, t0)) > 0; ++i) {
+                for (int j = 0; j < cnt; ++j) {
+                    TCP(c0 = clock64();)
+                    mbar_wait_sleep(out_ready, oph, 64);
+                    TCP(t_w += clock64() - c0;)
+                    tma_store_2d(&tm_out, out_u32, 0, (t0 + j) * TILE_M);
+                    tma_store_2d(&tm_out, out_u32 + OUT_BOX_BYTES, 64, (t0 + j) * TILE_M);
+                    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                    asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+                    mbar_arrive(out_free);
+                    oph ^= 1;
                 }
             }
+            asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");  // stores complete before the CTA exits
+#ifdef MRB_TC_PROF
+            if (P.prof) {
+                unsigned long long* o = P.prof + (size_t)blockIdx.x * 16;
+                o[12] = clock64() - t_start; o[13] = t_w;
+            }
+#endif
         }
     } else {
         // ============================== EPILOGUE ==============================
@@ -372,10 +318,12 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
             sts128u(out_u32 + OUT_BOX_BYTES + swz(m, c8), make_uint4(lo[0], lo[1], lo[2], lo[3]));
         };
         TCP(long long e_start = clock64(), e_wait = 0;)
-        int buf = 0;
-        uint32_t acc_phase = 0;
-        for (int tile = first_tile; tile < P.n_tiles; tile += tile_stride) {
-            const uint32_t t0 = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(buf * P.acc_cols);
+        int n_mine = 0, t0;
+        for (int i = 0, cnt; (cnt = deal.item(i, t0)) > 0; ++i) n_mine += cnt;
+        for (int seq = 0; seq < n_mine; ++seq) {
+            const int buf = seq & 3;
+            const uint32_t acc_phase = ((uint32_t)seq >> 2) & 1u;
+            const uint32_t t0m = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(buf * ACC_COLS);
             bool released = false;
             TCP(long long c0 = clock64();)
             mbar_wait_sleep(&acc_full[buf], acc_phase, 64);
@@ -389,7 +337,7 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
                 for (int jb = 0; jb < 2; ++jb) {
                     const int j = j_lo + jb * 16;
                     float a[8], a2[8], b1[8], b2[8];
-                    tmem_ld8x4(t0 + j, t0 + 64 + j, t0 + j + 8, t0 + 64 + j + 8, a, a2, b1, b2);
+                    tmem_ld8x4(t0m + j, t0m + 64 + j, t0m + j + 8, t0m + 64 + j + 8, a, a2, b1, b2);
 #pragma unroll
                     for (int q = 0; q < 8; ++q) {
                         o[jb * 16 + q] = a[q] + a2[q];
@@ -418,6 +366,7 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
                 tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&acc_empty[buf]);
+                mbar_wait_sleep(out_free, oph ^ 1, 32);
             }
             // the tile's [128 positions x (64 hi | 64 lo)] boxes are complete once all eight epilogue warps have
             // arrived; the TMA store lane takes it from there
@@ -425,7 +374,6 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
             __syncwarp();
             if (lane == 0) mbar_arrive(out_ready);
             oph ^= 1;
-            if (++buf == P.acc_bufs) { buf = 0; acc_phase ^= 1u; }
         }
 #ifdef MRB_TC_PROF
         if (P.prof && threadIdx.x == 0) {
@@ -436,9 +384,9 @@ __global__ void __launch_bounds__(THREADS, 1) tc_kernel(const __grid_constant__ 
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == EPI_WARPS + LOAD_WARPS) {
+    if (warp == MMA_WARP) {
         tc_fence_after();
-        tmem_dealloc(tmem_base, (uint32_t)P.tmem_cols);
+        tmem_dealloc(tmem_base, 512);
     }
 }
 
@@ -485,45 +433,31 @@ int pack_launch(const PackDesc& D, void* dst, cudaStream_t st) {
     return MRB_OK;
 }
 
-static size_t smem_needed(const Params& P) {
-    return 1024 + (size_t)2 * OUT_BOX_BYTES + (size_t)P.b_stages * 2 * W_CHUNK_BYTES +
-           (size_t)LOAD_WARPS * P.tb_depth * P.tb_bytes + 256 + 2 * B_STAGES * 8 + BIAS_FLOATS * sizeof(float);
-}
-
 #ifdef MRB_TC_PROF
 static int g_debug = 0;
 static unsigned long long* g_prof = nullptr;
 #endif
 
-static int launch(Params& P, void* out, cudaStream_t st) {
+static int launch(Params& P, const void* src, void* out, long long n_pos, cudaStream_t st) {
 #ifdef MRB_TC_PROF
     P.debug = g_debug;
     P.prof = g_prof;
 #endif
     const size_t max_smem = device_max_smem_optin();
-    P.tmem_cols = 512;
-    // The two loader groups take turns by kernel row: a group's next unit starts k segments after the end of its last one,
-    // so without at least k + 1 TMEM stages a loader can reach a stage two rounds ahead of the issuer, where the parity
-    // wait of mbarrier cannot tell the round it needs from the one before (the 5x5 conv on 4 stages hung).  A kernel size
-    // whose ring would be shorter gives up the second accumulator buffer.
-    if ((512 - P.acc_bufs * P.acc_cols) / A_STAGE_COLS < P.ksz + 1) P.acc_bufs = 1;
-    P.stages = (512 - P.acc_bufs * P.acc_cols) / A_STAGE_COLS;
-    if (P.stages > MAX_STAGES) P.stages = MAX_STAGES;
-    MRB_REQUIRE(P.stages >= 2 && P.stages >= P.ksz + 1, MRB_EUNSUPPORTED,
-                "tensor-core conv: the TMEM A ring needs %d stages for k = %d", P.ksz + 1, P.ksz);
-    MRB_REQUIRE(P.P < 2147483647LL, MRB_EUNSUPPORTED, "tensor-core conv: too many pixels");
-    MRB_REQUIRE(P.nseg >= 1 && P.nseg <= MAX_SEGS, MRB_EUNSUPPORTED, "tensor-core conv: bad segment count");
-    CUtensorMap tm_out;
+    MRB_REQUIRE(SMEM_BYTES <= max_smem, MRB_EUNSUPPORTED, "tensor-core conv: %zu bytes of shared memory needed, %zu available",
+                SMEM_BYTES, max_smem);
+    // every TMA coordinate (a box starts up to pad rows and pad positions before its tile) must fit an int
+    MRB_REQUIRE(n_pos + (long long)BH_PAD * (P.pitch + 1) + 2 * TILE_M < 2147483647LL, MRB_EUNSUPPORTED,
+                "tensor-core conv: too many pixels");
+    MRB_REQUIRE(P.ksz * P.ksz <= MAX_SEGS && P.dil * (P.ksz - 1) / 2 <= BH_PAD, MRB_EUNSUPPORTED,
+                "tensor-core conv: bad geometry");
+    CUtensorMap tm_in, tm_out;
+    memset(&tm_in, 0, sizeof(tm_in));
     memset(&tm_out, 0, sizeof(tm_out));
-    int rc = tc2::make_bh_tmap(&tm_out, out, P.P, TILE_M);
+    int rc = tc2::make_bh_tmap(&tm_in, src, n_pos, A_BOX_ROWS);
     if (rc) return rc;
-    // 32 + 2*pad flat positions per unit
-    P.tb_half = (32 + P.dil * (P.ksz - 1)) * 128;
-    P.tb_bytes = 2 * P.tb_half;
-    P.tb_depth = 2;  // one staging tile feeds k segments: current + next is enough
-    P.b_stages = B_STAGES;
-    while (P.b_stages > 2 && smem_needed(P) > max_smem) --P.b_stages;
-    MRB_REQUIRE(smem_needed(P) <= max_smem, MRB_EUNSUPPORTED, "tensor-core conv: staging does not fit shared memory");
+    rc = tc2::make_bh_tmap(&tm_out, out, n_pos, TILE_M);
+    if (rc) return rc;
     static bool attr_set = false;  // per-process, not per launch (the attribute calls are not free)
     if (!attr_set) {
         MRB_CUDA(cudaFuncSetAttribute(tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_smem));
@@ -535,7 +469,7 @@ static int launch(Params& P, void* out, cudaStream_t st) {
     // step then run with the same shared-memory carve-out.  Alternating this kernel between a ~195 KB and a ~227 KB
     // configuration (two different carve-outs) produced sporadic "Warp Illegal Instruction" traps in the weight streamer
     // and hangs on the B200; same-size sequences never failed.
-    tc_kernel<<<grid, THREADS, max_smem, st>>>(tm_out, P);
+    tc_kernel<<<grid, THREADS, max_smem, st>>>(tm_in, tm_out, P);
     MRB_LAUNCHED();
     return MRB_OK;
 }
@@ -578,26 +512,18 @@ extern "C" int mrb_tc_conv_bh(const void* x_bh, const void* wpack, const void* b
     MRB_REQUIRE((k % 2) == 1 && k * k <= tc::MAX_SEGS && dil >= 1, MRB_EUNSUPPORTED, "mrb_tc_conv_bh: unsupported geometry");
     MRB_REQUIRE(dil * (k - 1) / 2 <= tc::BH_PAD, MRB_EUNSUPPORTED, "mrb_tc_conv_bh: the receptive field exceeds the BH border");
     MRB_REQUIRE(B >= 1 && H >= 1 && W >= 1, MRB_EINVAL, "tensor-core conv: bad shape");
+    const long long n_pos = (long long)B * (H + 2 * tc::BH_PAD) * (W + 2 * tc::BH_PAD);
+    long long nt = (n_pos + tc::TILE_M - 1) / tc::TILE_M;
+    MRB_REQUIRE(nt <= 2147483647LL, MRB_EUNSUPPORTED, "tensor-core conv: too many pixels");
     tc::Params P;
     memset(&P, 0, sizeof(P));
-    P.B = B; P.H = H; P.W = W;
-    P.P = (long long)B * (H + 2 * tc::BH_PAD) * (W + 2 * tc::BH_PAD);
-    long long nt = (P.P + tc::TILE_M - 1) / tc::TILE_M;
-    MRB_REQUIRE(nt <= 2147483647LL, MRB_EUNSUPPORTED, "tensor-core conv: too many pixels");
     P.n_tiles = (int)nt;
-    P.src = (const uint8_t*)x_bh;
-    P.wpack = wpack; P.bias = (const float*)bias;
+    P.pitch = W + 2 * tc::BH_PAD;
     // One segment per tap (64 input channels = one 128-byte bf16 row of B), stacked MMAs of N = 128 and 64 (half the MMA
     // instructions of a channel split).  The k*k weight chunks (2*64*128 B each: hi rows | lo rows) are streamed from L2
-    // through a small ring -- resident they would leave no room for the halo staging tiles.
-    P.nseg = k * k;
-    // One accumulator group per buffer (hi*hi chain | cross-term chain, summed in the epilogue), two buffers.  Measured
-    // and removed: two MMA issuers on alternating segments with plain st.global from the epilogue -- 443 vs 371 us at
-    // B = 16: the thread-per-position stores (32 cache lines per instruction) compete with the loaders' cp.async for L1
-    // wavefronts.
-    P.acc_cols = 2 * cout;
-    P.acc_bufs = 2;
+    // through a small ring -- resident they would leave no room for the A boxes; each streamed chunk feeds two tiles.
+    P.wpack = wpack; P.bias = (const float*)bias;
     P.relu = relu;
     P.ksz = k; P.dil = dil;
-    return tc::launch(P, out_bh, (cudaStream_t)stream);
+    return tc::launch(P, x_bh, out_bh, n_pos, (cudaStream_t)stream);
 }

@@ -82,14 +82,6 @@ int make_bh_tmap(void* mp, const void* base, long long Q, int box_rows) {
     MRB_REQUIRE(r == CUDA_SUCCESS, MRB_ECUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
     return MRB_OK;
 }
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* m, int c0, int c1, uint32_t bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(dst),
-                 "l"(m), "r"(c0), "r"(c1), "r"(bar)
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
 #ifdef MRB_TC_PROF
 __device__ int g_skip_mma = 0;
 #endif
@@ -977,11 +969,6 @@ __device__ __forceinline__ uint64_t make_desc_ns(uint32_t saddr, uint32_t lbo, u
     d |= (uint64_t)((sbo >> 4) & 0x3FFF) << 32;  // byte distance between 8-row core matrices
     d |= (uint64_t)1 << 46;                      // descriptor version (Blackwell); layout type 0 = no swizzle
     return d;
-}
-__device__ __forceinline__ void bulk_load_1d(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
-                 "r"(bytes), "r"(bar)
-                 : "memory");
 }
 
 __global__ void __launch_bounds__(C5_THREADS, 1)

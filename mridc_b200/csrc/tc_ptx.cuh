@@ -1,4 +1,4 @@
-// PTX wrappers shared by the tcgen05 / TMEM kernels (conv_tc.cu: TMEM-A engine; conv_tc2.cu: TMA + smem-A engine).
+// PTX wrappers shared by the tcgen05 / TMEM kernels (conv_tc.cu: the BH k x k conv; conv_tc2.cu: the other BH kernels).
 #pragma once
 #include "common.cuh"
 
@@ -103,47 +103,37 @@ __device__ __forceinline__ void umma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, u
         "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
-// Stacked-B variant (2 MMAs per k-step instead of 3): the packed weight chunk holds the hi rows immediately followed
-// by the lo rows, so ONE descriptor with N = 2n multiplies a_hi by [b_hi ; b_lo] -> columns [d, d+n) = a_hi*b_hi and
-// [d+n, d+2n) = a_hi*b_lo; the second MMA adds a_lo*b_hi (N = n) onto the cross-term columns [d+n, d+2n).
-__device__ __forceinline__ void umma_segment_ts_stacked(uint32_t d, uint32_t dsm, uint32_t a_hi, uint32_t a_lo, uint64_t dbh,
+// Stacked-B segment (2 MMAs per k-step instead of 3), A and B from shared memory: the packed weight chunk holds the hi
+// rows immediately followed by the lo rows, so ONE descriptor with N = 2n multiplies a_hi by [b_hi ; b_lo] -> columns
+// [d, d+n) = a_hi*b_hi and [d+n, d+2n) = a_hi*b_lo; the second MMA adds a_lo*b_hi (N = n) onto the cross-term columns
+// [d+n, d+2n).  Four k-steps of K = 16 advance every SWIZZLE_128B K-major descriptor by 32 bytes.
+__device__ __forceinline__ void umma_segment_ss_stacked(uint32_t d, uint32_t dsm, uint64_t a_hi, uint64_t a_lo, uint64_t dbh,
                                                         uint32_t idesc2n, uint32_t idescn, uint32_t acc0) {
     asm volatile(
         "{\n\t"
         ".reg .pred pa, pt, pe;\n\t"
         "elect.sync _|pe, 0xffffffff;\n\t"
-        ".reg .b32 ah1, ah2, ah3, al1, al2, al3;\n\t"
-        ".reg .b64 bh1, bh2, bh3;\n\t"
+        ".reg .b64 ah1, ah2, ah3, al1, al2, al3, bh1, bh2, bh3;\n\t"
         "setp.ne.b32 pa, %7, 0;\n\t"
         "setp.eq.b32 pt, 0, 0;\n\t"
-        "add.u32 ah1, %2, 8;\n\t add.u32 ah2, %2, 16;\n\t add.u32 ah3, %2, 24;\n\t"
-        "add.u32 al1, %3, 8;\n\t add.u32 al2, %3, 16;\n\t add.u32 al3, %3, 24;\n\t"
+        "add.u64 ah1, %2, 2;\n\t add.u64 ah2, %2, 4;\n\t add.u64 ah3, %2, 6;\n\t"
+        "add.u64 al1, %3, 2;\n\t add.u64 al2, %3, 4;\n\t add.u64 al3, %3, 6;\n\t"
         "add.u64 bh1, %4, 2;\n\t add.u64 bh2, %4, 4;\n\t add.u64 bh3, %4, 6;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], [%2], %4, %5, pa;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], [%3], %4, %6, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], [ah1], bh1, %5, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], [al1], bh1, %6, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], [ah2], bh2, %5, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], [al2], bh2, %6, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], [ah3], bh3, %5, pt;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], [al3], bh3, %6, pt;\n\t"
+        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], %2, %4, %5, pa;\n\t"
+        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], %3, %4, %6, pt;\n\t"
+        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], ah1, bh1, %5, pt;\n\t"
+        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], al1, bh1, %6, pt;\n\t"
+        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], ah2, bh2, %5, pt;\n\t"
+        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], al2, bh2, %6, pt;\n\t"
+        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], ah3, bh3, %5, pt;\n\t"
+        "@pe tcgen05.mma.cta_group::1.kind::f16 [%1], al3, bh3, %6, pt;\n\t"
         "}\n" ::"r"(d),
-        "r"(dsm), "r"(a_hi), "r"(a_lo), "l"(dbh), "r"(idesc2n), "r"(idescn), "r"(acc0)
+        "r"(dsm), "l"(a_hi), "l"(a_lo), "l"(dbh), "r"(idesc2n), "r"(idescn), "r"(acc0)
         : "memory");
 }
 // lane-0 broadcast: tells the compiler that a value is warp-uniform (see umma_commit)
 __device__ __forceinline__ uint32_t uni(uint32_t v) { return __shfl_sync(0xffffffffu, v, 0); }
 __device__ __forceinline__ uint64_t uni64(uint64_t v) { return ((uint64_t)uni((uint32_t)(v >> 32)) << 32) | uni((uint32_t)v); }
-// registers -> TMEM: 16 consecutive columns of this thread's lane
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t* v) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr),
-        "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]),
-        "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
-        : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-
 // four 8-column loads with a single wait (GRU epilogue: hh_n, r, z, ih_n blocks)
 __device__ __forceinline__ void tmem_ld8x4(uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, float* v0, float* v1, float* v2,
                                            float* v3) {
@@ -180,6 +170,10 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t saddr) {
     d |= (uint64_t)2 << 61;                  // SWIZZLE_128B
     return d;
 }
+// The same matrix `rows` 128-byte rows further on, for a descriptor of a 1024-byte aligned SWIZZLE_128B tile: only the
+// start address moves (rows * 128 B).  The tensor core takes the swizzle phase of a row from the address bits, as TMA
+// writes it, so a start inside the 8-row pattern needs no matrix base offset (bits 49-51 stay 0).
+__device__ __forceinline__ uint64_t desc_rows(uint64_t d, uint32_t rows) { return d + (uint64_t)(rows * (128 >> 4)); }
 __host__ __device__ constexpr uint32_t make_idesc(int M, int N) {
     // c_format F32 (1) @4, a_format BF16 (1) @7, b_format BF16 (1) @10, K-major A and B, N>>3 @17, M>>4 @24
     return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
@@ -298,6 +292,22 @@ __device__ __forceinline__ uint4 lds128u(uint32_t saddr) {
 }
 __device__ __forceinline__ void sts128u(uint32_t saddr, uint4 v) {
     asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(saddr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
+}
+// 2-D TMA box load global -> shared memory, completing the box's bytes on the mbarrier's transaction count; m = address
+// of a CUtensorMap.  Box rows outside the tensor (negative coordinates too) are zero-filled.
+__device__ __forceinline__ void tma_load_2d(uint32_t dst, const void* m, int c0, int c1, uint32_t bar) {
+    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(dst),
+                 "l"(m), "r"(c0), "r"(c1), "r"(bar)
+                 : "memory");
+}
+// contiguous bulk copy global -> shared memory, completing the mbarrier's transaction count
+__device__ __forceinline__ void bulk_load_1d(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
+                 "r"(bytes), "r"(bar)
+                 : "memory");
+}
+__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
 // 2-D TMA box store shared memory -> global (bulk async group of the issuing thread); m = address of a CUtensorMap
 __device__ __forceinline__ void tma_store_2d(const void* m, uint32_t src, int c0, int c1) {
