@@ -75,10 +75,23 @@ class RimTcEngine:
             return False
         return f.kernel_size == 3 and f.dilation == 1
 
+    @staticmethod
+    def covers_width(W) -> bool:
+        """Images at least 28 pixels wide run on the engine, narrower ones on the exact-fp32 loop.  The entry points serve
+        every width (tests/test_gpu_tc_geometry.py, DESIGN 4.3): moving narrower images to the engine would change their
+        numerics, which is a decision of its own."""
+        return W >= 28
+
     def covers(self, W) -> bool:
-        """The engine runs this block on images W pixels wide: rows of at least 32 positions (W + 4 >= 32), the tile width of
-        the BH kernels' loaders and TMA boxes."""
-        return self.supported(self.block) and W >= 28
+        """The engine runs this block on images W pixels wide (covers_width)."""
+        return self.supported(self.block) and self.covers_width(W)
+
+    @staticmethod
+    def final_conv_symbol(B, H) -> str:
+        """Entry point of the final conv: the tensor-core tap GEMM from 16 rows of the [B (H+4)] x (W+4) grid (the height
+        of its 3-D TMA box) up, the CUDA-core kernel (after a border fix-up) below.  Both entry points serve every B, H, W
+        (tests/test_gpu_tc_geometry.py); the split only keeps the smallest batches on exact-fp32 arithmetic."""
+        return "mrb_tc2_final_conv" if B * (H + 4) >= 16 else "mrb_conv_c2_bh_residual"
 
     @staticmethod
     def _g8(lib, B, H, W, dev):
@@ -155,7 +168,7 @@ class RimTcEngine:
         self._cell_bh(lib, xbuf, h[1], packs[1][1], r1, h_alt[1], B, H, W, st)
         h[1], h_alt[1] = h_alt[1], h[1]
         new_eta = torch.empty_like(eta)
-        if B * (H + 4) >= 16:  # the 3-D TMA box of the tap GEMM spans 16 rows of the [B (H+4)] x (W+4) grid
+        if self.final_conv_symbol(B, H) == "mrb_tc2_final_conv":
             # tap GEMM on the tensor core + clamped gather: reads the interior of h[1] only, no border fix-up
             _lib.check(lib.mrb_tc2_final_conv(_lib.ptr(h[1]), _lib.ptr(fin.conv_layer.weight), _lib.ptr(fin.conv_layer.bias),
                                               _lib.ptr(eta), _lib.ptr(new_eta), B, H, W, st))

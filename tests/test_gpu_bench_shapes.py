@@ -61,26 +61,40 @@ def _real64(t):
     return (torch.view_as_real(t) if t.is_complex() else t).double()
 
 
-def slice_errors(out, ref):
-    """-> (rel-L2, max-abs error / max |ref|) of every slice (dim 0) of out against ref, float64 on the CPU."""
+# Below this many values a slice's own norm is no scale for its rounding error: a few sums can cancel to any smallness
+# while the error of each stays the size of its terms (see check_slices' ``scale``)
+SMALL_SLICE = 64
+
+
+def slice_errors(out, ref, scale=None):
+    """-> (rel-L2, max-abs error / max |ref|) of every slice (dim 0) of out against ref, float64 on the CPU.  With
+    ``scale`` (see check_slices) and slices of fewer than SMALL_SLICE values, both are taken relative to the scale."""
     ref = _real64(ref)
     out = _real64(out).to(ref.device)
     assert out.shape == ref.shape, (tuple(out.shape), tuple(ref.shape))
     d = (out - ref).reshape(ref.shape[0], -1)
     r = ref.reshape(ref.shape[0], -1)
+    if scale is not None and r.shape[1] < SMALL_SLICE:
+        r = _real64(scale).to(ref.device).reshape(r.shape)
+        assert bool((r >= ref.reshape(r.shape).abs() * (1 - 1e-12)).all()), "the scale must bound |ref|"
     rel = d.norm(dim=1) / r.norm(dim=1).clamp_min(1e-300)
     mx = d.abs().amax(1) / r.abs().amax(1).clamp_min(1e-300)
     return rel.cpu(), mx.cpu()
 
 
-def check_slices(name, out, ref, tol, slices=None):
+def check_slices(name, out, ref, tol, slices=None, scale=None):
     """Every slice's rel-L2 <= tol (NaN fails).  Prints the worst slice, its max-abs error relative to its max |ref| and
-    the margin to the tolerance.  ``slices``: the batch indices of the compared slices (default 0 .. n-1)."""
-    rel, mx = slice_errors(out, ref)
+    the margin to the tolerance.  ``slices``: the batch indices of the compared slices (default 0 .. n-1).
+    ``scale``: shaped like ref, the sum of the magnitudes of the terms each value adds up (|eta| + |b| + sum |w| |x| for
+    a conv), which bounds its rounding error.  Slices of fewer than SMALL_SLICE values are then held to tol relative to
+    the norm of their scale instead of their own: one or two outputs can cancel to any smallness, their error cannot."""
+    rel, mx = slice_errors(out, ref, scale)
     ids = list(range(len(rel))) if slices is None else [int(i) for i in slices]
     w = int(torch.nan_to_num(rel, nan=float("inf")).argmax())
-    print("[bench shapes] %-50s %2d slices, worst %2d: rel-L2 %.2e  max-abs/max|ref| %.2e  tol %.0e  margin %6.1fx" % (
-        name, len(ids), ids[w], rel[w], mx[w], tol, tol / float(rel[w]) if rel[w] != 0 else float("inf")))
+    small = scale is not None and _real64(ref).reshape(len(rel), -1).shape[1] < SMALL_SLICE
+    print("[bench shapes] %-50s %2d slices, worst %2d: rel-L2 %.2e  max-abs/max|ref| %.2e  tol %.0e  margin %6.1fx%s" % (
+        name, len(ids), ids[w], rel[w], mx[w], tol, tol / float(rel[w]) if rel[w] != 0 else float("inf"),
+        "  (relative to the term magnitudes)" if small else ""))
     bad = [(ids[i], float(rel[i])) for i in range(len(ids)) if not rel[i] <= tol]
     assert not bad, "%s: slices over the rel-L2 tolerance %.0e: %s" % (name, tol, bad)
     return rel
