@@ -26,10 +26,11 @@ from .cascadenet import CascadeNetBlock  # noqa: F401
 from .recurrentvarnet import Conv2dGRU, RecurrentInit, RecurrentVarNetBlock  # noqa: F401
 from .qvarnet import qVarNetBlock  # noqa: F401
 from .jrscirim import JRSCIRIMBlock  # noqa: F401
-from .models import CIRIM, VarNet, UNet, ZF, qCIRIM  # noqa: F401
+from .models import CIRIM, VarNet, UNet, ZF, PICS, qCIRIM  # noqa: F401
 from .pipeline import HostPrefetcher  # noqa: F401
 from .transforms import MRIDataTransforms, assemble_reconstructions, save_reconstructions  # noqa: F401
 from .espirit import espirit_maps  # noqa: F401
+from .pics import l1_wavelet_recon  # noqa: F401
 from . import metrics  # noqa: F401
 
 __version__ = "0.1.0"

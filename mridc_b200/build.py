@@ -1,5 +1,6 @@
-"""Build recipe for libmridc_b200.so (hand-written CUDA for sm_100a, C-ABI in include/mridc_b200.h) and
-libmridc_b200_espirit.so (coil-sensitivity estimation, C-ABI in include/mridc_b200_espirit.h).
+"""Build recipe for libmridc_b200.so (hand-written CUDA for sm_100a, C-ABI in include/mridc_b200.h),
+libmridc_b200_espirit.so (coil-sensitivity estimation, C-ABI in include/mridc_b200_espirit.h) and
+libmridc_b200_pics.so (l1-wavelet SENSE reconstruction, C-ABI in include/mridc_b200_pics.h).
 
 The library is built IN-TREE (mridc_b200/libmridc_b200.so) with nvcc so that it travels with the source
 snapshot to the GPU box; nvcc cross-compiles without a GPU.  `python -m mridc_b200.build` or
@@ -21,6 +22,11 @@ ESPIRIT_SOURCES = ["espirit.cu"]
 ESPIRIT_HEADER = os.path.join(PKG_DIR, "..", "include", "mridc_b200_espirit.h")
 ESPIRIT_LIB_PATH = os.path.join(PKG_DIR, "libmridc_b200_espirit.so")
 ESPIRIT_STAMP = os.path.join(PKG_DIR, "csrc", ".build_stamp_espirit")
+# PICS library: a library of its own as well; its data-term gradient comes from libmridc_b200.so through Python
+PICS_SOURCES = ["pics.cu"]
+PICS_HEADER = os.path.join(PKG_DIR, "..", "include", "mridc_b200_pics.h")
+PICS_LIB_PATH = os.path.join(PKG_DIR, "libmridc_b200_pics.so")
+PICS_STAMP = os.path.join(PKG_DIR, "csrc", ".build_stamp_pics")
 # tools-only library (tools/libmridc_b200_tools.so): the tensor-core kernels with their per-role cycle counters and role
 # switches compiled in (-DMRB_TC_PROF) plus the tcgen05 issue micro-benchmark; never loaded by the package
 TOOLS_SOURCES = ["core.cu", "conv_tc.cu", "conv_tc2.cu", "conv.cu", "tc_microbench.cu"]
@@ -44,7 +50,7 @@ def _digest():
     h = hashlib.sha256()
     for root, _, files in sorted(os.walk(CSRC)):
         for f in sorted(files):
-            if f.endswith((".cu", ".cuh", ".h")) and f not in ESPIRIT_SOURCES:
+            if f.endswith((".cu", ".cuh", ".h")) and f not in ESPIRIT_SOURCES + PICS_SOURCES:
                 with open(os.path.join(root, f), "rb") as fh:
                     h.update(f.encode() + b"\0" + fh.read())
     with open(os.path.join(PKG_DIR, "..", "include", "mridc_b200.h"), "rb") as fh:
@@ -53,12 +59,12 @@ def _digest():
     return h.hexdigest()
 
 
-def _espirit_digest():
+def _side_digest(sources, header):
     h = hashlib.sha256()
-    for f in ESPIRIT_SOURCES:
+    for f in sources:
         with open(os.path.join(CSRC, f), "rb") as fh:
             h.update(f.encode() + b"\0" + fh.read())
-    with open(ESPIRIT_HEADER, "rb") as fh:
+    with open(header, "rb") as fh:
         h.update(fh.read())
     h.update(" ".join(NVCC_FLAGS).encode())
     return h.hexdigest()
@@ -72,18 +78,21 @@ def _fresh(path, stamp, digest):
 
 
 def build(force=False, verbose=False):
-    """Compile every CUDA source for sm_100a: libmridc_b200.so and libmridc_b200_espirit.so. Returns the path of the
-    first."""
+    """Compile every CUDA source for sm_100a: libmridc_b200.so, libmridc_b200_espirit.so and libmridc_b200_pics.so.
+    Returns the path of the first."""
     digest = _digest()
     if force or not _fresh(LIB_PATH, STAMP, digest):
         _compile(SOURCES, LIB_PATH, os.path.join(PKG_DIR, "csrc", "build"), verbose)
         with open(STAMP, "w") as fh:
             fh.write(digest)
-    digest = _espirit_digest()
-    if force or not _fresh(ESPIRIT_LIB_PATH, ESPIRIT_STAMP, digest):
-        _compile(ESPIRIT_SOURCES, ESPIRIT_LIB_PATH, os.path.join(PKG_DIR, "csrc", "build", "espirit"), verbose)
-        with open(ESPIRIT_STAMP, "w") as fh:
-            fh.write(digest)
+    for sources, header, lib, stamp, sub in (
+            (ESPIRIT_SOURCES, ESPIRIT_HEADER, ESPIRIT_LIB_PATH, ESPIRIT_STAMP, "espirit"),
+            (PICS_SOURCES, PICS_HEADER, PICS_LIB_PATH, PICS_STAMP, "pics")):
+        digest = _side_digest(sources, header)
+        if force or not _fresh(lib, stamp, digest):
+            _compile(sources, lib, os.path.join(PKG_DIR, "csrc", "build", sub), verbose)
+            with open(stamp, "w") as fh:
+                fh.write(digest)
     return LIB_PATH
 
 

@@ -9,6 +9,7 @@ of scope (SURVEY.md section 2, rows 9/17) -- ``trainer`` is accepted and ignored
   VarNet  mridc/collections/reconstruction/models/vn.py:22-142
   UNet    mridc/collections/reconstruction/models/unet.py:21-121
   ZF      mridc/collections/reconstruction/models/zf.py:20-100
+  PICS    mridc/collections/reconstruction/models/pics.py (BART `pics`; here FISTA on the GPU, mridc_b200.pics)
   qCIRIM  mridc/collections/quantitative/models/qcirim.py:21-341 (quantitative module; BASELINE.json configs[4])
 """
 import math
@@ -17,14 +18,14 @@ from typing import Any, Generator, List, Mapping, Union
 import torch
 import torch.nn as nn
 
-from . import _lib, _ops, utils
+from . import _lib, _ops, pics, utils
 from .qrim import RescaleByMax, SignalForwardModel, qRIMBlock
 from .rim import RIMBlock
 from .sensitivity import BaseSensitivityModel
 from .unet import NormUnet
 from .varnet import VarNetBlock
 
-__all__ = ["CIRIM", "VarNet", "UNet", "ZF", "qCIRIM"]
+__all__ = ["CIRIM", "VarNet", "UNet", "ZF", "PICS", "qCIRIM"]
 
 
 def _cfg_dict(cfg) -> dict:
@@ -239,6 +240,37 @@ class ZF(_BaseModel):
                              self.fft_normalization, self.spatial_dims, self.coil_dim)
         pred = utils.check_stacked_complex(pred)
         _, pred = utils.center_crop_to_smallest(target, pred)
+        return pred
+
+
+class PICS(_BaseModel):
+    """l1-wavelet compressed-sensing SENSE reconstruction, the classical baseline of upstream ``PICS`` (which calls BART
+    ``pics``).  Solved here by ``mridc_b200.pics.l1_wavelet_recon`` with the contract of DESIGN.md section 4.8: cfg
+    ``reg_wt`` is lamda, ``num_iters`` the number of FISTA iterations."""
+
+    def __init__(self, cfg, trainer=None):
+        super().__init__(cfg, trainer)
+        c = self._cfg
+        self.reg_wt = c.get("reg_wt")
+        self.num_iters = c.get("num_iters")
+        self.fft_centered = c.get("fft_centered")
+        self.fft_normalization = c.get("fft_normalization")
+        self.spatial_dims = _listify(c.get("spatial_dims"))
+        self.coil_dim = c.get("coil_dim")
+        _ops.check_spatial_dims(self.spatial_dims)
+        if self.coil_dim is not None and self.coil_dim != 1:
+            raise NotImplementedError("mridc_b200 PICS takes k-space as [B, C, H, W, 2] (coil_dim 1); got %s" % (
+                self.coil_dim,))
+
+    @torch.no_grad()
+    def forward(self, y: torch.Tensor, sensitivity_maps: torch.Tensor, mask: torch.Tensor,
+                init_pred: torch.Tensor = None, target: torch.Tensor = None) -> torch.Tensor:
+        """-> complex [B, H, W], cropped to ``target``.  ``init_pred`` is unused: FISTA starts from zero."""
+        pred = pics.l1_wavelet_recon(y, sensitivity_maps, mask, self.reg_wt, self.num_iters, self.fft_centered,
+                                     self.fft_normalization)
+        pred = torch.view_as_complex(pred)
+        if target is not None:
+            _, pred = utils.center_crop_to_smallest(target, pred)
         return pred
 
 
